@@ -30,6 +30,10 @@ models over the whole matrix.
 
 `--impl reference` times that restated reference alone (the real reference needs TensorFlow, which cannot
 be installed here), on the same config / metric / unit.
+
+`--dump-outputs DIR` writes the headline fit's state after its last timed step to DIR/<name>.npy (float32, about
+42 MB): what a caller of the timed steps receives, for comparing two builds output for output.  The inputs are drawn
+from fixed seeds, so two runs with the same arguments start from identical data.
 """
 import argparse
 import contextlib
@@ -168,7 +172,7 @@ def run_reference_arm(args):
     if rank != 0:
         return
     threads = os.cpu_count() or 1
-    K, W = max(args.steps, 1), max(args.warmup, 0)
+    K, W = args.steps, max(args.warmup, 0)
     val, ms, sample = cpu_reference_run(K, W, threads)
     out = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
            "steps": K, "warmup": W, "ms_per_step": ms, "higher_is_better": True,
@@ -267,6 +271,27 @@ def time_steps(ctx, eng, K, W, sampler=None):
     kms, kn = eng.kernel_time_ms()
     return dict(ms=ctx.max_over_ranks(ms_local), ms_local=ms_local, kernel_ms=kms / max(kn, 1), launches=eng.launch_count - l0,
                 t0=t0, t1=t1)
+
+
+def dump_outputs(ctx, eng, out_dir, n_cells=128, seed=0):
+    """The engine state after its last step, gathered over the ranks' event shards, as float32 .npy files in
+    out_dir: the per-event parameters (Wc, intercept, sigma_log: models x rows x events) whole, and the
+    variational parameters (Z_loc, Z_std_log: models x cells x events) for a fixed, seeded sample of n_cells
+    cells -- all of them would be 16 GB at the headline size."""
+    from brie_b200.sharding import gather_event_axis
+    torch = ctx.torch
+    Ng = eng.Ng
+    cells = np.sort(np.random.default_rng(seed).choice(eng.Nc, min(n_cells, eng.Nc), replace=False))
+    rows = torch.from_numpy(cells).to(eng.device)
+    arrays = {"Z_loc": eng.Z_loc.index_select(1, rows)[:, :, :Ng],
+              "Z_std_log": eng.Z_std_log.index_select(1, rows)[:, :, :Ng],
+              "Wc": eng.Wc[:, :max(len(mk) for mk in eng.masks), :Ng],
+              "intercept": eng.intercept[:, :Ng], "sigma_log": eng.sigma_log[:, :Ng]}
+    arrays = {k: gather_event_axis(v.cpu().numpy(), v.dim() - 1) for k, v in arrays.items()}
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in arrays.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def shape_leg(ctx, name, K, W, events=None, note=None):
@@ -471,13 +496,19 @@ def main():
                     help="run the end-to-end leg on the headline workload only if its predicted wall time is below this; "
                          "else on C2 (said in e2e.workload)")
     ap.add_argument("--out-root", default="/dev/shm" if os.path.isdir("/dev/shm") else "/tmp")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline fit's state after its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
         return run_reference_arm(args)
 
     ctx = Ctx()
     torch = ctx.torch
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     c = SHAPES[HEAD]
     M = len(c["masks"])
     (lo, hi), group, Ng = shard_of(ctx, HEAD)
@@ -495,6 +526,8 @@ def main():
         time.sleep(0.25)
     r = time_steps(ctx, eng, K, W)
     clocks = sampler.stop(r["t0"], r["t1"]) if ctx.rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(ctx, eng, args.dump_outputs)
     value = c["cells"] * Ng * S * M * K / (r["ms"] * 1e-3)
     peak, peak_src = hbm_peak()
     alg_bytes = c["cells"] * (hi - lo) * (4 * c["layers"] + 48 * M)        # this GPU's launch (SURVEY.md 8d)

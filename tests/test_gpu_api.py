@@ -414,3 +414,33 @@ def test_device_simulator_mirrors_reference_semantics():
     sim3 = simulator(ad, mode="prior", prior_sigma=1.5, seed=1)
     zs3 = np.log(ad.layers['Psi_sim'] / (1 - ad.layers['Psi_sim']))
     assert abs(np.std(np.clip(zs3 - z0, -20, 20)) - 1.5) < 0.1
+
+
+def test_bench_dump_outputs_hold_the_state_after_the_timed_steps(tmp_path, monkeypatch):
+    """bench.py --dump-outputs on a small shape with the headline's layout (M = 4, Kc = 3, gene intercept): the
+    files are the engine state after the warm-up and exactly --steps timed steps, and the same arguments give the
+    same inputs, so two runs dump the same arrays bit for bit."""
+    import bench
+    monkeypatch.setitem(bench.SHAPES, "T", dict(bench.SHAPES[bench.HEAD], cells=300, events=70))
+    ctx = bench.Ctx()
+    dumps = []
+    for run, K in enumerate((4, 4, 5)):
+        (lo, hi), group, Ng = bench.shard_of(ctx, "T")
+        eng, _ = bench.build_engine(ctx, "T", lo, hi, Ng, group)
+        bench.time_steps(ctx, eng, K, 3)
+        assert eng.step_counters()[0] == 3 + K
+        out = str(tmp_path / str(run))
+        bench.dump_outputs(ctx, eng, out, n_cells=16)
+        d = {f[:-len(".npy")]: np.load(os.path.join(out, f)) for f in os.listdir(out)}
+        assert set(d) == {"Z_loc", "Z_std_log", "Wc", "intercept", "sigma_log"}
+        assert all(v.dtype == np.float32 for v in d.values())
+        cells = np.sort(np.random.default_rng(0).choice(300, 16, replace=False))
+        assert d["Z_loc"].shape == (4, 16, 70) and d["Wc"].shape == (4, 3, 70) and d["sigma_log"].shape == (4, 70)
+        assert np.array_equal(d["Z_loc"], eng.Z_loc[:, cells, :70].cpu().numpy())
+        assert np.array_equal(d["Z_std_log"], eng.Z_std_log[:, cells, :70].cpu().numpy())
+        assert np.array_equal(d["intercept"], eng.intercept[:, :70].cpu().numpy())
+        dumps.append(d)
+        del eng
+    for k in dumps[0]:
+        assert np.array_equal(dumps[0][k], dumps[1][k]), k
+    assert not np.array_equal(dumps[0]["Z_loc"], dumps[2]["Z_loc"])

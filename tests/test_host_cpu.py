@@ -464,3 +464,13 @@ def test_bench_reference_arm_runs_and_mirrors_the_config():
     other = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                            capture_output=True, text=True, timeout=60, cwd=ROOT, env=dict(os.environ, RANK="1"))
     assert other.returncode == 0 and other.stdout.strip() == ""            # ranks other than 0 exit without work
+
+
+def test_bench_rejects_zero_steps_and_a_dump_of_the_reference_arm():
+    """--steps is the number of timed steps, so 0 is an error rather than a silent 1; --dump-outputs writes the GPU
+    arm's outputs and is refused with --impl reference.  Both are refused before any work."""
+    for extra, msg in ((["--steps", "0"], "--steps must be at least 1"),
+                       (["--impl", "reference", "--dump-outputs", "unused"], "--dump-outputs applies to the GPU arm")):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "" and msg in out.stderr, (extra, out.stderr[-2000:])
