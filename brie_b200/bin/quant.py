@@ -37,7 +37,7 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
           intercept=None, intercept_mode='gene', nproc=1, min_counts=50,
           min_counts_uniq=10, min_cells_uniq=30, min_MIF_uniq=0.001,
           min_iter=5000, max_iter=20000, MC_size=1, batch_size=500000,
-          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False):
+          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0):
     """CLI driver (quant.py:13-130).  `nproc` is accepted for compatibility (host threads are
     not on the hot path any more); `seed` keys the counter-based noise (new, default 0).
     `out_dir` (new): directory for `.npy` memory maps of the dense (cells, events) output layers
@@ -46,7 +46,8 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     1M x 20k; the output container then references the maps instead of embedding the arrays.  Under
     torchrun it defaults to `<out_file stem>.layers/`, so no (cells, events) array ever travels through a
     collective.  `resume` (new, needs out_dir): skip the event chunks a previous run of the same fit left
-    there (checkpoint / restart).
+    there (checkpoint / restart).  `n_perm` (new): permutation replicates per tested covariate; adds the
+    pooled permutation p-values and their FDR to the container (varm) and the table (fitBRIE).
 
     Multi-GPU: launch one process per GPU (`python -m torch.distributed.run --nproc-per-node N
     -m brie_b200.bin.quant ...`); every rank reads the input, fits its own event shard
@@ -106,7 +107,7 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     fitBRIE(adata, Xc=Xc, Xg=Xg, LRT_index=LRT_index, layer_keys=layer_keys,
             intercept=intercept, intercept_mode=intercept_mode,
             min_iter=min_iter, max_iter=max_iter, MC_size=MC_size, batch_size=batch_size,
-            pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed,
+            pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed, n_perm=n_perm,
             **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
 
     adata.uns['brie_version'] = brie_b200.__version__
@@ -178,9 +179,15 @@ def main():
              "chunk by chunk; the output file references them) [default: in RAM; <out_file>.layers under torchrun]")
     group3.add_option("--resume", action="store_true", dest="resume", default=False,
         help="With --outDir: skip the event chunks a previous run of the same fit has finished")
+    group4 = OptionGroup(parser, "Calibration (not in the reference)")
+    group4.add_option("--nPerm", type=int, dest="n_perm", default=0,
+        help="Permutation replicates per tested feature: refit the model with that feature's cells permuted "
+             "--nPerm times and add p-values against the permutation null pooled over all events, with their "
+             "FDR (columns <feature>_pval_perm, <feature>_FDR_perm) [default: %default]")
     parser.add_option_group(group1)
     parser.add_option_group(group2)
     parser.add_option_group(group3)
+    parser.add_option_group(group4)
 
     (options, args) = parser.parse_args()
     if len(sys.argv[1:]) == 0:
@@ -198,6 +205,12 @@ def main():
     else:
         LRT_index = np.array(options.LRT_index.split(","), float).astype(int)
     intercept = None if options.intercept_mode.upper() in ["GENE", 'CELL'] else 0   # quant.py:205
+    if options.n_perm < 0:
+        print("[BRIE2] Error: --nPerm needs to be 0 or more.")
+        sys.exit(1)
+    if options.n_perm > 0 and LRT_index is not None and len(LRT_index) == 0:
+        print("[BRIE2] Error: --nPerm needs tested features (--LRTindex).")
+        sys.exit(1)
 
     quant(options.in_file, options.cell_file, options.gene_file,
           options.out_file, LRT_index, options.layers.split(','),
@@ -205,7 +218,7 @@ def main():
           options.min_uniq_count, options.min_cell, options.min_MIF,
           options.min_iter, options.max_iter, options.MC_size,
           options.batch_size, options.pseudo_count, options.test_base, options.seed,
-          options.out_dir, options.resume)
+          options.out_dir, options.resume, options.n_perm)
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         if dist.is_initialized():

@@ -58,6 +58,60 @@ def fdr_by_group(pval, group_size=None, event_offset=0):
     return fdr
 
 
+MAX_MODEL_IDS = 4096                       # 12-bit model word of the Philox stream (csrc/brie_philox.h)
+
+
+def perm_indices(seed, t, b, Nc):
+    """Cell permutation of replicate b of test position t (index into LRT_index, not the covariate number).
+    It depends on (seed, t, b, Nc) alone, so every event chunk and every rank permutes the cells alike."""
+    return np.random.default_rng((int(seed), 1 + int(t), int(b))).permutation(int(Nc))
+
+
+def perm_model_id(t, b, n_tests, n_perm):
+    """RNG model word of permuted model (t, b): after the base model (0) and the LRT refits (1..T)."""
+    return 1 + n_tests + t * n_perm + b
+
+
+def check_n_perm(n_perm, n_tests):
+    """Validate `n_perm` for a fit with `n_tests` tested covariates (before any device work)."""
+    if isinstance(n_perm, bool) or int(n_perm) != n_perm:
+        raise ValueError("n_perm must be an integer, got %r" % (n_perm,))
+    n_perm = int(n_perm)
+    if n_perm < 0:
+        raise ValueError("n_perm must be >= 0, got %d" % n_perm)
+    if n_perm > 0 and n_tests == 0:
+        raise ValueError("n_perm > 0 needs at least one tested covariate (LRT_index)")
+    if 1 + n_tests * (1 + n_perm) > MAX_MODEL_IDS:
+        raise ValueError("n_perm = %d with %d tested covariates needs %d model ids; the noise stream has %d"
+                         % (n_perm, n_tests, 1 + n_tests * (1 + n_perm), MAX_MODEL_IDS))
+    return n_perm
+
+
+def perm_pvalue(gain, gain_perm):
+    """Pooled empirical p-values (Ng, T) of the observed gains `gain` (Ng, T) against the permutation null
+    `gain_perm` (Ng, T, B) of every event: (1 + #{(g', b) : gain_perm[g', t, b] >= gain[g, t]}) / (1 + Ng * B).
+    NaN compares False, as in the double loop."""
+    gain, gain_perm = np.asarray(gain), np.asarray(gain_perm)
+    Ng, T, B = gain_perm.shape
+    out = np.empty(gain.shape, np.float64)
+    for t in range(T):
+        null = np.sort(gain_perm[:, t, :].reshape(-1))
+        null = null[~np.isnan(null)]
+        n_ge = null.size - np.searchsorted(null, gain[:, t], side='left')
+        out[:, t] = (1.0 + n_ge) / (1.0 + Ng * B)
+    return out
+
+
+def _set_perm_outputs(res):
+    """pval_perm and fdr_perm of a result holding ELBO_gain and ELBO_gain_perm, over all of its events: one
+    pooled null and one BH scope per tested covariate.  This scope differs on purpose from the chi2 FDR's
+    (fdr_by_group, the reference's per-batch scope, degenerate at 1-event batches)."""
+    res.pval_perm = perm_pvalue(res.ELBO_gain, res.ELBO_gain_perm)
+    res.fdr_perm = np.zeros(res.pval_perm.shape)
+    for i in range(res.fdr_perm.shape[1]):
+        res.fdr_perm[:, i] = fdr_bh(res.pval_perm[:, i])
+
+
 class BRIE_RV():
     """Return value object for BRIE2 model (model_wrap.py:15-76)."""
 
@@ -109,6 +163,9 @@ class BRIE_RV():
             self.fdr = np.append(self.fdr, new_RV.fdr, axis=0)
             self.pval = np.append(self.pval, new_RV.pval, axis=0)
             self.ELBO_gain = np.append(self.ELBO_gain, new_RV.ELBO_gain, axis=0)
+        if hasattr(new_RV, 'ELBO_gain_perm'):           # pval_perm / fdr_perm: fitBRIE recomputes them over all events
+            for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
+                setattr(self, k, np.append(getattr(self, k), getattr(new_RV, k), axis=0))
         if hasattr(new_RV, 'n_iter'):
             self.n_iter = np.append(self.n_iter, new_RV.n_iter, axis=1)
         if getattr(self, 'timing', None) is not None and getattr(new_RV, 'timing', None) is not None:
@@ -193,11 +250,20 @@ def _host_pseudo_count_inplace(data, pseudo_count):
         np.add(data[i], pseudo_count, out=data[i], where=idx, casting='unsafe')
 
 
-def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=None):
+def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=None, n_perm=0, tested=(),
+                 n_cols=0, full=True):
     """[(column masks, model ids, intercept mode)] per FitEngine: the base model (id 0) with as many LRT refits
     (ids 1..T) as one launch batches, the remaining refits in further engines of at most `max_models` models; a
     cell-mode base model sits alone, because the reference's refits always use the per-event layout
-    (model_wrap.py:174-178)."""
+    (model_wrap.py:174-178).
+
+    With `n_perm` = B > 0 the permuted models (t, b) follow in additional engines, never in the observed ones:
+    an engine's model count sets the association of its float32 cell sums, so the observed outputs stay
+    bit-identical to the B = 0 fit, and no engine is larger than the largest observed one (the device budget
+    of fitBRIE holds).  Model (t, b) is the observed alternative of test t -- the full model (base_mode
+    'full', base layout) or test model t (base_mode 'null', per-event layout) -- with column tested[t] replaced
+    in place by column n_cols + j of the engine's design, j its position in the engine; its id is
+    perm_model_id(t, b, T, B)."""
     if max_models is None:
         from .._lib import BRIE_MAX_MODELS as max_models
     T = len(test_masks)
@@ -211,6 +277,14 @@ def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=No
     for t0 in range(first_tests, T, max_models):
         t1 = min(t0 + max_models, T)
         plan.append((test_masks[t0:t1], list(range(1 + t0, 1 + t1)), 'gene'))
+    if n_perm > 0:
+        size = min(max(len(ids) for _, ids, _ in plan), max_models)
+        perm = [(t, b) for t in range(T) for b in range(n_perm)]
+        for p0 in range(0, len(perm), size):
+            part = perm[p0:p0 + size]
+            masks = [[n_cols + j if k == tested[t] else k for k in (base_cols if full else test_masks[t])]
+                     for j, (t, b) in enumerate(part)]
+            plan.append((masks, [perm_model_id(t, b, T, n_perm) for t, b in part], intercept_mode if full else 'gene'))
     return plan
 
 
@@ -223,8 +297,17 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     init key, default 0), `group_size` / `event_offset` / `n_events_total` (reference
     batch geometry when called from fitBRIE), `device`, `init_objs` (per-model
     injected initial values: [base, refit_0, ...]), `n_eval` (loss_gene evaluations,
-    500 in the reference), `dist_group`.  All other **keyargs go to the fit schedule
-    as in the reference (`min_iter, max_iter, add_iter, epsilon_conv, MC_size`).
+    500 in the reference), `dist_group`, `n_perm` (permutation null, default 0: see below).
+    All other **keyargs go to the fit schedule as in the reference (`min_iter, max_iter,
+    add_iter, epsilon_conv, MC_size`).
+
+    `n_perm` = B > 0 also fits, for every test position t and replicate b < B, the observed
+    alternative of test t (the full model, or test model t with base_mode 'null') with the tested
+    column's cells permuted by `perm_indices(seed, t, b, Nc)`, and returns `ELBO_gain_perm`
+    (Ng, T, B), its null gains; `pval_perm` (Ng, T), the pooled empirical p-values of `ELBO_gain`
+    against the gains of every event and replicate (`perm_pvalue`); and `fdr_perm`, BH over all
+    events.  Permuted models only evaluate `loss_gene`; the observed outputs are bit-identical to
+    the n_perm = 0 fit.
     """
     from scipy.sparse import issparse
     seed = keyargs.pop('seed', 0)
@@ -239,6 +322,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     target = keyargs.pop('target', "ELBO")                          # reaches BRIE2.fit through **keyargs (:144)
     host_side_effect = keyargs.pop('host_side_effect', True)
     out_sink = keyargs.pop('out_sink', None)                        # _ChunkSink: fitBRIE's output arrays
+    n_tests = len(LRT_index) if LRT_index is not None else (0 if Xc is None else np.shape(Xc)[1])
+    n_perm = check_n_perm(keyargs.pop('n_perm', 0), n_tests)
     for k in ('optimizer', 'learn_rate', 'verbose'):                # accepted and ignored (:214-237)
         keyargs.pop(k, None)
 
@@ -320,20 +405,31 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     # that runs the remaining refits in further engines, one after the other, over the same device tiles.
     # NB the reference builds the refits WITHOUT intercept_mode (model_wrap.py:174-178), so they always use
     # the default per-event ('gene') intercept/sigma layout: a cell-mode base model gets an engine of its own.
-    plan = _engine_plan(base_cols, test_masks, cell_mode, intercept_mode)
+    plan = _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, n_perm=n_perm, tested=LRT_index,
+                        n_cols=Kc, full=full)
     t_ph = _tick("engine_setup", t_ph)
 
     brie_results = None
     n_iter_rows, lg_tests, wc_last, launches = [None] * (T + 1), [None] * T, [None] * T, 0
+    lg_perm = {}                                                    # (t, b) -> loss_gene of permuted model (t, b)
     for masks_e, ids_e, mode_e in plan:
-        eng = FitEngine(data, masks=masks_e, model_ids=ids_e, intercept_mode=mode_e, **common)
-        io = None if init_objs is None else [init_objs[i] for i in ids_e]
+        io, kw_e = None, common
+        if ids_e[0] > T:                                            # permuted models: their columns appended to Xc
+            tb = [divmod(mid - 1 - T, n_perm) for mid in ids_e]
+            cols = [Xc[perm_indices(seed, t, b, Nc), LRT_index[t]] for t, b in tb]
+            kw_e = dict(common, Xc=np.concatenate([Xc, np.stack(cols, axis=1)], axis=1))
+        elif init_objs is not None:
+            io = [init_objs[i] for i in ids_e]
+        eng = FitEngine(data, masks=masks_e, model_ids=ids_e, intercept_mode=mode_e, **kw_e)
         eng.fit(n_eval=n_eval, init_objs=io, **keyargs)             # :144, :180
         t_ph = _tick("fit", t_ph)
         if timing is not None:
             for k, v in eng.phase_s.items():
                 timing[k] = timing.get(k, 0.0) + v
         for j, mid in enumerate(ids_e):
+            if mid > T:
+                lg_perm[divmod(mid - 1 - T, n_perm)] = eng.loss_gene[j].cpu().numpy()
+                continue
             n_iter_rows[mid] = eng.n_iter[j]
             if mid == 0:
                 brie_results = _rv_from_engine(eng, j, Xc[:, base_cols], Xg, intercept_mode, out_sink)   # :146
@@ -362,6 +458,12 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     brie_results.pval = chi2.sf(2 * ELBO_gain, df=1)                # :190
     fdr = fdr_by_group(brie_results.pval, group_size, event_offset)
     brie_results.fdr = fdr
+    if n_perm > 0:
+        gain_perm = np.zeros((Ng, T, n_perm), dtype=np.float32)
+        for (t, b), lg in lg_perm.items():
+            gain_perm[:, t, b] = (lg_tests[t] if full else brie_results.loss_gene) - lg
+        brie_results.ELBO_gain_perm = gain_perm
+        _set_perm_outputs(brie_results)
     return brie_results
 
 
@@ -391,6 +493,9 @@ def _merge_shared(parts):
             out.intercept = np.append(out.intercept, r.intercept, axis=1)
         if hasattr(r, 'ELBO_gain'):
             for k in ('fdr', 'pval', 'ELBO_gain'):
+                setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
+        if hasattr(r, 'ELBO_gain_perm'):
+            for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
                 setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
     out.shape = (out.Nc, out.Ng)
     if hasattr(out, 'pval'):               # one fit => one multiple-testing scope over all events
@@ -445,6 +550,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     `resume` (not in the reference; needs `out_dir`): every finished event chunk is checkpointed
     under `out_dir`; with resume=True a re-run of the same fit (same data shape, design, seed and
     schedule) skips the chunks already there and returns what the uninterrupted fit would have.
+    `n_perm` (not in the reference, default 0): permutation replicates per tested covariate, see
+    fit_BRIE_matrix; `pval_perm` / `fdr_perm` are pooled over all events of the fit (every chunk and
+    rank) and stored as varm['ELBO_gain_perm', 'pval_perm', 'fdr_perm'] with uns['brie_param']['n_perm'].
 
     Returns the BRIE_RV result and adds to `adata` exactly the keys the reference adds
     (obsm['Xc'], varm['cell_coeff'], varm['Xg'], obsm['gene_coeff'], varm|obsm['intercept',
@@ -459,6 +567,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         LRT_index = np.arange(Xc.shape[1])
     Nc, Ng = adata.shape
     n_models = 1 + len(LRT_index)
+    n_perm = check_n_perm(keyargs.pop('n_perm', 0), len(LRT_index))
+    if n_perm > 0:                         # (absent at 0: the fit signature of a checkpoint stays as it was)
+        keyargs['n_perm'] = n_perm
     out_dir = keyargs.pop('out_dir', None)
     resume = keyargs.pop('resume', False)
     out_keys = tuple(keyargs.pop('out_keys', None) or BIG_KEYS)
@@ -558,6 +669,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             pseudo_count=pseudo_count, sigma=sigma, base_mode=base_mode,
             tau_prior=tau_prior, **keyargs)
 
+    if n_perm > 0:                         # one pooled null over every event of the fit, the same on every rank
+        _set_perm_outputs(ResVal)
+
     # update adata (:271-311)
     if Xc.shape[0] > 0:
         adata.obsm['Xc'] = Xc
@@ -585,6 +699,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         adata.varm['fdr'] = ResVal.fdr
         adata.varm['pval'] = ResVal.pval
         adata.varm['ELBO_gain'] = ResVal.ELBO_gain
+    if n_perm > 0:
+        for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
+            adata.varm[k] = getattr(ResVal, k)
 
     adata.uns['brie_param'] = {
         'LRT_index': LRT_index,
@@ -595,4 +712,6 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         'pseudo_count': pseudo_count,
         'layer_keys': layer_keys
     }
+    if n_perm > 0:
+        adata.uns['brie_param']['n_perm'] = n_perm
     return ResVal

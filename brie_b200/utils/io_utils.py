@@ -85,4 +85,9 @@ def dump_results(adata):
         for suffix, source in (('_ceoff', 'cell_coeff'), ('_ELBO_gain', 'ELBO_gain'),
                                ('_pval', 'pval'), ('_FDR', 'fdr')):
             table[label + suffix] = adata.varm[source][:, pos]
+    if 'pval_perm' in adata.varm:          # permutation null (brie-quant --nPerm): after all the reference's columns
+        for pos, feature in enumerate(tested):
+            label = names[feature] if names is not None else 'X%d' % pos
+            table[label + '_pval_perm'] = adata.varm['pval_perm'][:, pos]
+            table[label + '_FDR_perm'] = adata.varm['fdr_perm'][:, pos]
     return table
