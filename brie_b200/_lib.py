@@ -8,7 +8,7 @@ import ctypes as C
 import os
 
 BRIE_MAX_MODELS = 32
-ABI_VERSION = 7
+ABI_VERSION = 8
 TARGETS = {"ELBO": 0, "marginLik": 1}
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BRIE_LIB_PATH", os.path.join(_HERE, "libbrie_b200.so"))
@@ -63,6 +63,7 @@ SYMBOLS = {
     "brie_fit_get_step": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_uint32)]),
     "brie_fit_run_steps": (C.c_int, [_P, C.c_int32, C.c_int32, _P]),
     "brie_fit_set_active_blocks": (C.c_int, [_P, _P, C.c_int64, C.POINTER(C.c_int32)]),
+    "brie_fit_set_count_codes": (C.c_int, [_P, _P, C.c_int64, _P]),
     "brie_fit_step_phase": (C.c_int, [_P, C.c_int32, C.c_int32, _P]),
     "brie_fit_cell_grad": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int64)]),
     "brie_comm_nccl_version": (C.c_int, []),
@@ -93,6 +94,8 @@ SYMBOLS = {
     "brie_add_pseudo_count": (C.c_int, [C.c_int64, C.c_int64, C.c_float, _P, _P, _P]),
     "brie_gene_stats_scratch_bytes": (C.c_size_t, [C.c_int64, C.c_int64]),
     "brie_gene_stats": (C.c_int, [C.c_int64, C.c_int64, _P, _P, _P, _P, _P, _P]),
+    "brie_encode_counts_scratch_bytes": (C.c_size_t, []),
+    "brie_encode_counts": (C.c_int, [C.c_int64, C.c_int64, _P, _P, _P, _P, _P, _P, _P, _P]),
     "brie_gather_events": (C.c_int, [C.c_int64, C.c_int64, _P, _P, C.c_int64, C.c_int64, _P, _P]),
     "brie_scatter_events": (C.c_int, [C.c_int64, C.c_int64, _P, _P, C.c_int64, C.c_int64, _P, _P]),
 }

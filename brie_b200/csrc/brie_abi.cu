@@ -64,6 +64,10 @@ struct brie_fit {
   bool wide = false;
   size_t off_PM = 0, off_R = 0, off_gWc = 0;   // (M, Nc, ld), (M, Nc, ld), (M, Kc, ld) in scratch
   cublasHandle_t blas = nullptr;
+  // counts as packed dictionary codes (brie_fit_set_count_codes); null = the float32 tiles
+  const uint32_t* codes = nullptr;
+  int64_t code_mstride = 0;
+  const float* code_dict = nullptr;
 };
 
 using namespace brie;
@@ -75,7 +79,7 @@ constexpr int kMaxDevices = 64;
 bool kc_supported(int k) { return k == 0 || k == 1 || k == 2 || k == 4 || k == 8 || k == 16; }
 bool kg_supported(int k) { return k == 0 || k == 4 || k == 8; }
 
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false>
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool CODE8>
 cudaError_t launch_step(const StepArgs& a, dim3 grid, cudaStream_t s) {
   // per instantiation and per device: opt in to > 48 KB dynamic shared memory (the attribute is per device)
   static bool configured[kMaxDevices] = {false};
@@ -83,19 +87,25 @@ cudaError_t launch_step(const StepArgs& a, dim3 grid, cudaStream_t s) {
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
-    e = cudaFuncSetAttribute(elbo_step_kernel<KC, KG, CELL, LOSS, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             step_smem_bytes(KC, KG, CELL, LOSS, EXT));
+    e = cudaFuncSetAttribute(elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8));
     if (e != cudaSuccess) return e;
     if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
   }
-  elbo_step_kernel<KC, KG, CELL, LOSS, EXT><<<grid, kThreads, step_smem_bytes(KC, KG, CELL, LOSS, EXT), s>>>(a);
+  elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8><<<grid, kThreads, step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8), s>>>(a);
   return cudaGetLastError();
+}
+
+// the count form (f32 tiles or packed codes) is the innermost choice
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false>
+cudaError_t launch_step_fmt(const StepArgs& a, dim3 grid, cudaStream_t s) {
+  return a.codes ? launch_step<KC, KG, CELL, LOSS, EXT, true>(a, grid, s) : launch_step<KC, KG, CELL, LOSS, EXT, false>(a, grid, s);
 }
 
 cudaError_t dispatch_step_wide(const StepArgs& a, bool cell, bool loss, dim3 grid, cudaStream_t s) {
   if (cell)
-    return loss ? launch_step<0, 0, true, true, true>(a, grid, s) : launch_step<0, 0, true, false, true>(a, grid, s);
-  return loss ? launch_step<0, 0, false, true, true>(a, grid, s) : launch_step<0, 0, false, false, true>(a, grid, s);
+    return loss ? launch_step_fmt<0, 0, true, true, true>(a, grid, s) : launch_step_fmt<0, 0, true, false, true>(a, grid, s);
+  return loss ? launch_step_fmt<0, 0, false, true, true>(a, grid, s) : launch_step_fmt<0, 0, false, false, true>(a, grid, s);
 }
 
 const char* blas_status(cublasStatus_t st) {
@@ -168,8 +178,8 @@ int wide_gradients(brie_fit* f, cudaStream_t s) {
 template <int KC, int KG>
 cudaError_t dispatch_step2(const StepArgs& a, bool cell, bool loss, dim3 grid, cudaStream_t s) {
   if (cell)
-    return loss ? launch_step<KC, KG, true, true>(a, grid, s) : launch_step<KC, KG, true, false>(a, grid, s);
-  return loss ? launch_step<KC, KG, false, true>(a, grid, s) : launch_step<KC, KG, false, false>(a, grid, s);
+    return loss ? launch_step_fmt<KC, KG, true, true>(a, grid, s) : launch_step_fmt<KC, KG, true, false>(a, grid, s);
+  return loss ? launch_step_fmt<KC, KG, false, true>(a, grid, s) : launch_step_fmt<KC, KG, false, false>(a, grid, s);
 }
 
 template <int KC>
@@ -348,8 +358,10 @@ int brie_fit_get_sizes(const brie_fit* fit, brie_fit_sizes* out) {
 int brie_fit_bind(brie_fit* fit, const brie_fit_buffers* b) {
   if (!fit || !b) return fail(BRIE_ERR_ARG, "null argument");
   const brie_fit_desc& d = fit->d;
-  if (!b->counts[0] || !b->counts[1]) return fail(BRIE_ERR_ARG, "counts[0], counts[1] required");
-  if ((d.n_layers == 3) != (b->counts[2] != nullptr))
+  // a gathered sub-fit may step on packed codes alone (brie_fit_set_count_codes) and bind no count tiles
+  const bool no_counts = b->event_ids && !b->counts[0] && !b->counts[1] && !b->counts[2];
+  if (!no_counts && (!b->counts[0] || !b->counts[1])) return fail(BRIE_ERR_ARG, "counts[0], counts[1] required");
+  if (!no_counts && (d.n_layers == 3) != (b->counts[2] != nullptr))
     return fail(BRIE_ERR_ARG, "counts[2] must be given iff n_layers == 3");
   if ((d.has_efflen != 0) != (b->efflen3 != nullptr))
     return fail(BRIE_ERR_ARG, "efflen3 must be given iff has_efflen");
@@ -526,6 +538,7 @@ int brie_fit_step_phase(brie_fit* f, int32_t phase, int32_t trace_slot, void* st
       BRIE_CUDA(cudaGetLastError());
       f->launches += 1;
     } else {
+    if (!f->codes && !f->buf.counts[0]) return fail(BRIE_ERR_ARG, "neither count tiles nor count codes bound");
     StepArgs a;
     memset(&a, 0, sizeof a);
     a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.event_offset = d.event_offset; a.seed = d.seed;
@@ -545,6 +558,9 @@ int brie_fit_step_phase(brie_fit* f, int32_t phase, int32_t trace_slot, void* st
     a.ev_ids = f->buf.event_ids;
     a.c_mstride = f->buf.counts_model_stride;
     a.eff_mstride = f->buf.efflen_model_stride;
+    a.codes = f->codes;
+    a.code_mstride = f->code_mstride;
+    a.dict = f->code_dict;
     dim3 grid(M, f->sz.n_col_tiles, f->sz.n_row_chunks);
     if (f->blk_ids) {
       a.blk_ids = f->blk_ids;
@@ -691,6 +707,23 @@ int brie_fit_set_active_blocks(brie_fit* f, const int32_t* blk_ids, int64_t blk_
   f->blk_ids = blk_ids;
   f->blk_stride = blk_stride;
   f->blk_tiles = tiles;
+  return BRIE_OK;
+}
+
+int brie_fit_set_count_codes(brie_fit* f, const uint32_t* codes, int64_t codes_model_stride, const float* dict) {
+  if (!f) return fail(BRIE_ERR_ARG, "null argument");
+  if (f->step_open) return fail(BRIE_ERR_ARG, "a split step is still open");
+  if (codes) {
+    if (!dict) return fail(BRIE_ERR_ARG, "dict required with codes");
+    if ((((uintptr_t)codes) & 15u) != 0) return fail(BRIE_ERR_ARG, "codes must be 16-byte aligned");
+    if (codes_model_stride < 0 || codes_model_stride % 4 != 0)
+      return fail(BRIE_ERR_ARG, "codes_model_stride must be >= 0 and a multiple of 4");
+  } else if (f->bound && !f->buf.counts[0]) {
+    return fail(BRIE_ERR_ARG, "this fit has no count tiles to fall back to");
+  }
+  f->codes = codes;
+  f->code_mstride = codes ? codes_model_stride : 0;
+  f->code_dict = codes ? dict : nullptr;
   return BRIE_OK;
 }
 

@@ -121,6 +121,132 @@ __global__ void __launch_bounds__(256) scatter_columns_kernel(const float* __res
   }
 }
 
+// ---- dictionary coding of the count tiles (brie_encode_counts) -------------------------------------------------
+// Per layer, a 1024-slot open-addressing set of the non-zero values' bit patterns (0 = empty slot): a layer that
+// can be coded holds at most 255 of them, so the set stays at most a quarter full.  Probes are bounded by the
+// table size, so the passes end whatever the data.
+constexpr int kCodeHash = 1024;
+constexpr int kCodeMax = 255;                  // non-zero values per layer a code byte can index
+constexpr int32_t kCodeOverflow = 1 << 30;     // n_values[l] once layer l cannot be coded
+
+__device__ __forceinline__ uint32_t code_hash(uint32_t bits) { return (bits * 0x9E3779B1u) >> 22; }
+
+// Inserts `bits` into a set; returns 1 if it was new, 0 if present, -1 if the set is full.
+__device__ __forceinline__ int code_set_insert(uint32_t* keys, uint32_t bits) {
+  uint32_t h = code_hash(bits);
+  for (int i = 0; i < kCodeHash; ++i, h = (h + 1) & (kCodeHash - 1)) {
+    const uint32_t k = *(volatile uint32_t*)&keys[h];
+    if (k == bits) return 0;
+    if (k == 0u) {
+      const uint32_t old = atomicCAS(&keys[h], 0u, bits);
+      if (old == 0u) return 1;
+      if (old == bits) return 0;
+    }
+  }
+  return -1;
+}
+
+// Pass 1: every CTA collects the values of its part of the tiles in shared memory, then merges its sets into the
+// global ones (keys (3, kCodeHash)), counting the distinct values of each layer in n_values.
+__global__ void __launch_bounds__(256) code_collect_kernel(const float* __restrict__ c1, const float* __restrict__ c2,
+                                                           const float* __restrict__ c3, int64_t n4, uint32_t* keys,
+                                                           int32_t* n_values) {
+  __shared__ uint32_t s_keys[3][kCodeHash];
+  __shared__ int s_n[3];
+  for (int i = threadIdx.x; i < 3 * kCodeHash; i += blockDim.x) (&s_keys[0][0])[i] = 0u;
+  if (threadIdx.x < 3) s_n[threadIdx.x] = 0;
+  __syncthreads();
+  const float* cs[3] = {c1, c2, c3};
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+#pragma unroll
+    for (int l = 0; l < 3; ++l) {
+      if (!cs[l]) continue;
+      const uint4 v = reinterpret_cast<const uint4*>(cs[l])[i];
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        if ((w[j] & 0x7fffffffu) == 0u) continue;                      // +0 / -0: code 0
+        if ((w[j] >> 31) != 0u || (w[j] & 0x7fffffffu) > 0x7f800000u) {  // negative or NaN: not codable
+          atomicMax(&s_n[l], kCodeOverflow);
+          continue;
+        }
+        if (*(volatile int*)&s_n[l] > kCodeMax) continue;
+        const int r = code_set_insert(s_keys[l], w[j]);
+        if (r > 0) atomicAdd(&s_n[l], 1);
+        if (r < 0) atomicMax(&s_n[l], kCodeOverflow);
+      }
+    }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 3 * kCodeHash; i += blockDim.x) {
+    const int l = i / kCodeHash;
+    if (s_n[l] > kCodeMax) {
+      if (i % kCodeHash == 0) atomicMax(&n_values[l], kCodeOverflow);
+      continue;
+    }
+    const uint32_t k = (&s_keys[0][0])[i];
+    if (k == 0u || *(volatile int32_t*)&n_values[l] > kCodeMax) continue;
+    const int r = code_set_insert(keys + l * kCodeHash, k);
+    if (r > 0) atomicAdd(&n_values[l], 1);
+    if (r < 0) atomicMax(&n_values[l], kCodeOverflow);
+  }
+}
+
+// Pass 2 (one CTA per layer): code of a value = 1 + its rank among the layer's values (ascending: for non-negative
+// floats the bit patterns order as the values), into slot_code (3, kCodeHash) and the dictionary.
+__global__ void __launch_bounds__(kCodeHash) code_dict_kernel(const uint32_t* __restrict__ keys,
+                                                              const int32_t* __restrict__ n_values,
+                                                              uint8_t* slot_code, float* dict) {
+  const int l = blockIdx.x;
+  __shared__ uint32_t s_k[kCodeHash];
+  const uint32_t k = keys[l * kCodeHash + threadIdx.x];
+  s_k[threadIdx.x] = k;
+  __syncthreads();
+  if (n_values[l] > kCodeMax || k == 0u) return;
+  int rank = 0;
+  for (int i = 0; i < kCodeHash; ++i) rank += (s_k[i] != 0u && s_k[i] < k) ? 1 : 0;
+  slot_code[l * kCodeHash + threadIdx.x] = (uint8_t)(rank + 1);
+  dict[l * 256 + rank + 1] = __uint_as_float(k);
+}
+
+__device__ __forceinline__ uint32_t code_lookup(const uint32_t* keys, const uint8_t* codes, uint32_t bits) {
+  if ((bits & 0x7fffffffu) == 0u) return 0u;
+  uint32_t h = code_hash(bits);
+  for (int i = 0; i < kCodeHash; ++i, h = (h + 1) & (kCodeHash - 1))
+    if (keys[h] == bits) return codes[h];
+  return 0u;   // not reached: pass 1 saw every value
+}
+
+// Pass 3: code words, four elements per thread.
+__global__ void __launch_bounds__(256) code_write_kernel(const float* __restrict__ c1, const float* __restrict__ c2,
+                                                         const float* __restrict__ c3, int64_t n4,
+                                                         const uint32_t* __restrict__ keys,
+                                                         const uint8_t* __restrict__ slot_code,
+                                                         const int32_t* __restrict__ n_values, uint4* out) {
+  if (n_values[0] > kCodeMax || n_values[1] > kCodeMax || n_values[2] > kCodeMax) return;
+  __shared__ uint32_t s_keys[3 * kCodeHash];
+  __shared__ uint8_t s_code[3 * kCodeHash];
+  for (int i = threadIdx.x; i < 3 * kCodeHash; i += blockDim.x) {
+    s_keys[i] = keys[i];
+    s_code[i] = slot_code[i];
+  }
+  __syncthreads();
+  const float* cs[3] = {c1, c2, c3};
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int l = 0; l < 3; ++l) {
+      if (!cs[l]) continue;
+      const uint4 v = reinterpret_cast<const uint4*>(cs[l])[i];
+      const uint32_t b[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        w[j] |= code_lookup(s_keys + l * kCodeHash, s_code + l * kCodeHash, b[j]) << (8 * l);
+    }
+    out[i] = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+}
+
 namespace {
 int stats_chunks(int64_t n_cells, int64_t ld, int64_t* rows_per_chunk) {
   const int64_t tiles = ceil_div(ld, 128);
@@ -195,6 +321,31 @@ int brie_gene_stats(int64_t n_cells, int64_t ld, const float* c1, const float* c
   BRIE_CUDA(cudaGetLastError());
   gene_stats_reduce_kernel<<<(unsigned)ceil_div(kStatFields * ld, 256), 256, 0, s>>>((const double*)scratch, chunks,
                                                                                       ld, stats);
+  BRIE_CUDA(cudaGetLastError());
+  return BRIE_OK;
+}
+
+size_t brie_encode_counts_scratch_bytes(void) { return (size_t)3 * kCodeHash * (sizeof(uint32_t) + sizeof(uint8_t)); }
+
+int brie_encode_counts(int64_t n_cells, int64_t ld, const float* c1, const float* c2, const float* c3,
+                       uint32_t* codes, float* dict, int32_t* n_values, void* scratch, void* stream) {
+  if (n_cells <= 0 || ld <= 0 || ld % 4 != 0) return fail(BRIE_ERR_ARG, "bad shape (ld must be a multiple of 4)");
+  if (!c1 || !c2 || !codes || !dict || !n_values || !scratch) return fail(BRIE_ERR_ARG, "null argument");
+  if ((((uintptr_t)c1) | ((uintptr_t)c2) | ((uintptr_t)c3) | ((uintptr_t)codes)) & 15u)
+    return fail(BRIE_ERR_ARG, "tiles and codes must be 16-byte aligned");
+  cudaStream_t s = (cudaStream_t)stream;
+  uint32_t* keys = (uint32_t*)scratch;
+  uint8_t* slot_code = (uint8_t*)(keys + 3 * kCodeHash);
+  BRIE_CUDA(cudaMemsetAsync(scratch, 0, brie_encode_counts_scratch_bytes(), s));
+  BRIE_CUDA(cudaMemsetAsync(n_values, 0, 3 * sizeof(int32_t), s));
+  BRIE_CUDA(cudaMemsetAsync(dict, 0, 3 * 256 * sizeof(float), s));
+  const int64_t n4 = n_cells * ld / 4;
+  const int64_t blocks = ceil_div(n4, 256) < 148 * 8 ? ceil_div(n4, 256) : 148 * 8;
+  code_collect_kernel<<<(unsigned)blocks, 256, 0, s>>>(c1, c2, c3, n4, keys, n_values);
+  BRIE_CUDA(cudaGetLastError());
+  code_dict_kernel<<<3, kCodeHash, 0, s>>>(keys, n_values, slot_code, dict);
+  BRIE_CUDA(cudaGetLastError());
+  code_write_kernel<<<(unsigned)blocks, 256, 0, s>>>(c1, c2, c3, n4, keys, slot_code, n_values, (uint4*)codes);
   BRIE_CUDA(cudaGetLastError());
   return BRIE_OK;
 }

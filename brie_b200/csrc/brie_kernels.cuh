@@ -5,8 +5,9 @@
 // keras Adam update and the Variable constraints (:68-69, :80-81).  The reference
 // materialises ~17 (S,Nc,Ng[,3]) tensors forward and as many backward; here one
 // pass over the (cells, events) state does sampling, likelihood, KL, analytic
-// gradients and Adam, reading 24 B + writing 24 B of state and reading 12 B of
-// counts per cell x event (HBM-bound; see DESIGN.md).
+// gradients and Adam, reading 24 B + writing 24 B of state and reading 4 B of
+// counts (packed dictionary codes; 12 B as float32 tiles) per cell x event
+// (HBM-bound; see DESIGN.md).
 //
 // Layout: every (cells, events) array is row-major, events contiguous, leading
 // dimension ld (ld % 4 == 0 is all the kernels need; the Python layer pads ld to 128
@@ -79,6 +80,11 @@ struct StepArgs {
   // GEMMs that turn it into d loss / d Wc = -Xc^T r and d loss / d Wg = -r Xg (brie_abi.cu).
   const float* PM;
   float* R;
+  // Packed-code counts (CODE8 instantiations, brie_encode_counts): one word per element, byte l = index of layer l's
+  // value in dict[l * 256 + .] (entry 0 is 0.0f, so word != 0 iff the element has reads).
+  const uint32_t* codes;
+  int64_t code_mstride;    // words between the code tiles of consecutive models (gathered sub-fits), 0 = shared
+  const float* dict;       // (3, 256)
 };
 
 constexpr int kBlkCols = 8;   // events per compaction block = one 32-byte sector of every f32 array
@@ -356,9 +362,16 @@ __device__ __forceinline__ void cp_async_lane(uint32_t dst_smem, const void* src
 //     real data, cost nothing here and the lanes stay converged;
 //   C (dense): owners subtract their slots (zeros where there were no reads),
 //     Adam-update and store (16 B stores at EPL = 4).
+// CODE8 (counts as packed dictionary codes, StepArgs.codes): the ring carries one code word per element in place of
+// the three count arrays (7 arrays, 4 B of counts per element instead of 12), phase A's read test is word != 0,
+// phase B decodes its items' counts from the (3, 256) dictionary in shared memory and leaves its sums in a per-warp
+// scratch area, which the owners read only for their elements with reads.  The decoded values are the f32 tiles'
+// bit patterns, so both forms compute the same bits.
 constexpr int kQueueFields = 1;   // tile column of the element; its data is read from, and its results written to, the row's ring slots
 constexpr int kRingArrays = 9;    // Z_loc, Z_std_log, c1, c2, c3, m_loc, v_loc, m_std, v_std
+constexpr int kRingArraysCode8 = 7;   // Z_loc, Z_std_log, code, m_loc, v_loc, m_std, v_std
 constexpr int kRingStages = 2;
+constexpr int kDictSize = 256;    // values per layer of the count dictionary (code 0 = 0.0f)
 __host__ __device__ constexpr int step_tile_cols(int KC, int KG = 0) { return 32 * step_epl(KC, KG); }
 // Rows a warp processes per loop iteration.  The 2-events-per-lane instantiations take two adjacent rows at a time:
 // their 64-event row holds ~10 elements with reads, a third of a warp, so the Monte-Carlo phase (Philox, Box-Muller,
@@ -389,17 +402,26 @@ __host__ __device__ constexpr int step_n_consts(int KC, int KG, bool CELL, bool 
   return step_consts_in_smem(KC, KG, LOSS) ? KC + KG + (CELL ? 0 : 3) : 0;
 }
 constexpr int kRowConstSlots = 32;   // per warp and ring stage: Xc[c, :], Wg[c, :], per-cell intercept / sigma_log of the row
-__host__ __device__ constexpr int step_smem_bytes(int KC, int KG, bool CELL, bool LOSS, bool EXT = false) {
-  return ((kWarps * kRingStages * (kRingArrays + (EXT ? 1 : 0)) + kWarps * kQueueFields) * step_rpi(KC, KG) + 7 +
-          step_n_consts(KC, KG, CELL, LOSS)) *
+// CODE8: per warp and row of an iteration, the Monte-Carlo sums d/dZ_loc, d/dZ_std_log and (LOSS) the log-likelihood
+__host__ __device__ constexpr int step_n_scratch(bool LOSS) { return LOSS ? 3 : 2; }
+__host__ __device__ constexpr int step_smem_bytes(int KC, int KG, bool CELL, bool LOSS, bool EXT = false,
+                                                  bool CODE8 = false) {
+  return ((kWarps * kRingStages * ((CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0)) +
+           kWarps * kQueueFields + (CODE8 ? kWarps * step_n_scratch(LOSS) : 0)) *
+              step_rpi(KC, KG) +
+          7 + step_n_consts(KC, KG, CELL, LOSS)) *
              step_tile_cols(KC, KG) * 4 +
-         kWarps * kRingStages * step_rpi(KC, KG) * kRowConstSlots * 4;
+         kWarps * kRingStages * step_rpi(KC, KG) * kRowConstSlots * 4 + (CODE8 ? 3 * kDictSize * 4 : 0);
 }
 
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false>
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false, bool CODE8 = false>
 __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(const StepArgs a) {
   static_assert(!EXT || (KC == 0 && KG == 0), "the wide-design form takes all covariates through PM / R");
-  constexpr int NRA = kRingArrays + (EXT ? 1 : 0);   // ring arrays per row slot (EXT: + the prior-mean tile)
+  // ring arrays per row slot (EXT: + the prior-mean tile) and the slots of the Adam moments / prior-mean tile in it
+  constexpr int NRA = (CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0);
+  constexpr int IA = CODE8 ? 3 : 5;                  // m_loc, v_loc, m_std, v_std at IA .. IA + 3
+  constexpr int IPM = IA + 4;
+  constexpr int NSCR = step_n_scratch(LOSS);
   constexpr int RPI = step_rpi(KC, KG);              // rows per loop iteration = row slots per ring stage
   using T = StepTraits<KC, KG, CELL, LOSS>;
   constexpr int NEV = T::NEV;
@@ -457,9 +479,16 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
   for (int t = 0; t < KGB; ++t) pk |= ((lane >> (4 - t)) & 1) << (KGB - 1 - t);
   constexpr int NRC = KC + KG + (CELL ? 2 : 0);   // per-row (cell) constants: Xc[c, :], Wg[c, :], b[c], tau[c]
   static_assert(NRC <= kRowConstSlots, "row constants must fit one slot per lane");
-  float* s_rc = smem + ((kWarps * kRingStages * NRA + kWarps * kQueueFields) * RPI + 7 +
-                        step_n_consts(KC, KG, CELL, LOSS)) * TC +
-                warp * (kRingStages * RPI * kRowConstSlots);
+  constexpr int kRcBase = ((kWarps * kRingStages * NRA + kWarps * kQueueFields) * RPI + 7 +
+                           step_n_consts(KC, KG, CELL, LOSS)) * TC;
+  float* s_rc = smem + kRcBase + warp * (kRingStages * RPI * kRowConstSlots);
+  // CODE8: this warp's Monte-Carlo sums (row r, sum k at (r * NSCR + k) * TC) and the count dictionary
+  constexpr int kScrBase = kRcBase + kWarps * kRingStages * RPI * kRowConstSlots;
+  float* const s_scr = smem + kScrBase + warp * (NSCR * RPI * TC);
+  float* const s_dict = smem + kScrBase + kWarps * NSCR * RPI * TC;
+  if (CODE8) {   // published by the barrier below
+    for (int i = threadIdx.x; i < 3 * kDictSize; i += kThreads) s_dict[i] = a.dict[i];
+  }
 
   // Per-event constants of the tile go to shared memory before the barrier that decides whether the tile has
   // any active event: their loads overlap the `active` loads and that barrier also publishes them.
@@ -516,6 +545,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
   const float* const bC0 = a.c[0] + cnt_off;
   const float* const bC1 = a.c[1] + cnt_off;
   const float* const bC2 = has_c3 ? a.c[2] + cnt_off : a.c[0];
+  const uint32_t* const bW = CODE8 ? a.codes + ((int64_t)m * a.code_mstride + row_begin * a.ld) : nullptr;
   const int64_t cell0 = (int64_t)m * a.Nc + row_begin;            // first cell of the CTA in the (M, Nc, .) row constants
   const uint32_t ld32 = (uint32_t)a.ld;
   const uint32_t col32 = in_ld ? (uint32_t)g0 : 0u;
@@ -537,7 +567,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
     mbar_init(bar0 + 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (seg_bytes < (uint32_t)TC * 4u || !has_c3) {   // slots no bulk copy ever fills must read as zero counts / state
+  if (seg_bytes < (uint32_t)TC * 4u || (!CODE8 && !has_c3)) {   // slots no bulk copy ever fills must read as zero counts / state
     for (int i = lane; i < kRingStages * RPI * SLOT; i += 32) s_ring[i] = 0.f;
   }
   __syncwarp();
@@ -550,20 +580,25 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       fence_proxy_async();                        // the warp's generic reads / writes of this stage (two iterations ago) come first
       const uint32_t bar = bar0 + stage * 8;
       const int nr = min(RPI, n_rows - lrb);
-      mbar_expect_tx(bar, seg_bytes * (8u + (has_c3 ? 1u : 0u) + (EXT ? 1u : 0u)) * (uint32_t)nr);
+      const uint32_t n_cnt = CODE8 ? 1u : (has_c3 ? 3u : 2u);
+      mbar_expect_tx(bar, seg_bytes * (6u + n_cnt + (EXT ? 1u : 0u)) * (uint32_t)nr);
       for (int r = 0; r < nr; ++r) {
         const uint32_t relw = (uint32_t)(lrb + r) * ld32 + (uint32_t)tile * TC;
         const uint32_t dstw = ring_base + (stage * RPI + r) * (SLOT * 4);
         bulk_g2s(dstw + 0 * TC * 4, bZl + relw, seg_bytes, bar);
         bulk_g2s(dstw + 1 * TC * 4, bZs + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 2 * TC * 4, bC0 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 3 * TC * 4, bC1 + relw, seg_bytes, bar);
-        if (has_c3) bulk_g2s(dstw + 4 * TC * 4, bC2 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 5 * TC * 4, bA0 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 6 * TC * 4, bA1 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 7 * TC * 4, bA2 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 8 * TC * 4, bA3 + relw, seg_bytes, bar);
-        if (EXT) bulk_g2s(dstw + 9 * TC * 4, bPM + relw, seg_bytes, bar);
+        if (CODE8) {
+          bulk_g2s(dstw + 2 * TC * 4, bW + relw, seg_bytes, bar);
+        } else {
+          bulk_g2s(dstw + 2 * TC * 4, bC0 + relw, seg_bytes, bar);
+          bulk_g2s(dstw + 3 * TC * 4, bC1 + relw, seg_bytes, bar);
+          if (has_c3) bulk_g2s(dstw + 4 * TC * 4, bC2 + relw, seg_bytes, bar);
+        }
+        bulk_g2s(dstw + (IA + 0) * TC * 4, bA0 + relw, seg_bytes, bar);
+        bulk_g2s(dstw + (IA + 1) * TC * 4, bA1 + relw, seg_bytes, bar);
+        bulk_g2s(dstw + (IA + 2) * TC * 4, bA2 + relw, seg_bytes, bar);
+        bulk_g2s(dstw + (IA + 3) * TC * 4, bA3 + relw, seg_bytes, bar);
+        if (EXT) bulk_g2s(dstw + IPM * TC * 4, bPM + relw, seg_bytes, bar);
       }
     }
 #endif
@@ -576,14 +611,18 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       const uint32_t dst = ring_lane + (stage * RPI + r) * (SLOT * 4);
       cp_async_lane<EPL * 4>(dst + 0 * TC * 4, bZl + rel, ok);
       cp_async_lane<EPL * 4>(dst + 1 * TC * 4, bZs + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 2 * TC * 4, bC0 + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 3 * TC * 4, bC1 + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 4 * TC * 4, bC2 + (has_c3 ? rel : 0u), ok && has_c3);
-      cp_async_lane<EPL * 4>(dst + 5 * TC * 4, bA0 + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 6 * TC * 4, bA1 + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 7 * TC * 4, bA2 + rel, ok);
-      cp_async_lane<EPL * 4>(dst + 8 * TC * 4, bA3 + rel, ok);
-      if (EXT) cp_async_lane<EPL * 4>(dst + 9 * TC * 4, bPM + rel, ok);
+      if (CODE8) {
+        cp_async_lane<EPL * 4>(dst + 2 * TC * 4, bW + rel, ok);
+      } else {
+        cp_async_lane<EPL * 4>(dst + 2 * TC * 4, bC0 + rel, ok);
+        cp_async_lane<EPL * 4>(dst + 3 * TC * 4, bC1 + rel, ok);
+        cp_async_lane<EPL * 4>(dst + 4 * TC * 4, bC2 + (has_c3 ? rel : 0u), ok && has_c3);
+      }
+      cp_async_lane<EPL * 4>(dst + (IA + 0) * TC * 4, bA0 + rel, ok);
+      cp_async_lane<EPL * 4>(dst + (IA + 1) * TC * 4, bA1 + rel, ok);
+      cp_async_lane<EPL * 4>(dst + (IA + 2) * TC * 4, bA2 + rel, ok);
+      cp_async_lane<EPL * 4>(dst + (IA + 3) * TC * 4, bA3 + rel, ok);
+      if (EXT) cp_async_lane<EPL * 4>(dst + IPM * TC * 4, bPM + rel, ok);
 #endif
       if (NRC > 0) {
         // The row's warp-uniform constants ride in the same commit group, one float per lane.  (As plain
@@ -708,12 +747,17 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       float c1[EPL], c2[EPL], c3[EPL], pmx[EPL];
 #pragma unroll
       for (int j = 0; j < EPL; ++j) pmx[j] = 0.f;
-      if (EXT) vec_get<EPL>(st[9 * 32], pmx);
+      if (EXT) vec_get<EPL>(st[IPM * 32], pmx);
       vec_get<EPL>(st[0 * 32], mu[r]);
       vec_get<EPL>(st[1 * 32], lam[r]);
-      vec_get<EPL>(st[2 * 32], c1);
-      vec_get<EPL>(st[3 * 32], c2);
-      vec_get<EPL>(st[4 * 32], c3);
+      vec_get<EPL>(st[2 * 32], c1);       // CODE8: the code words (as float bits)
+      if (!CODE8) {
+        vec_get<EPL>(st[3 * 32], c2);
+        vec_get<EPL>(st[4 * 32], c3);
+      }
+      auto has_reads = [&](int j) {
+        return CODE8 ? __float_as_uint(c1[j]) != 0u : c1[j] + c2[j] + c3[j] > 0.f;
+      };
       float is2_row = 1.f;
       if (CELL) is2_row = fast_exp(-2.0f * tau_row);
       float caccr[NCELL > 0 ? NCELL : 1];
@@ -758,8 +802,8 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         const float2 e2m1 = f2_add(e2, f2_splat(-1.0f));
         gmu[r][j0] = rr.x; gmu[r][j1] = rr.y;
         glam[r][j0] = e2m1.x; glam[r][j1] = e2m1.y;
-        if (c1[j0] + c2[j0] + c3[j0] > 0.f) nz |= 1u << (r * EPL + j0);
-        if (c1[j1] + c2[j1] + c3[j1] > 0.f) nz |= 1u << (r * EPL + j1);
+        if (has_reads(j0)) nz |= 1u << (r * EPL + j0);
+        if (has_reads(j1)) nz |= 1u << (r * EPL + j1);
         const float2 gt = f2_sub(f2_sub(f2_splat(1.0f), q2), e2);            // d loss / d sigma_log
 #pragma unroll
         for (int k = 0; k < KC; ++k) {
@@ -808,7 +852,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         const float q2 = diff * rr;                        // ((mu - m) / sigma)^2
         gmu[r][j] = rr;
         glam[r][j] = e2 - 1.0f;
-        if (c1[j] + c2[j] + c3[j] > 0.f) nz |= 1u << (r * EPL + j);
+        if (has_reads(j)) nz |= 1u << (r * EPL + j);
         const float gt = 1.0f - q2 - e2;                   // d loss / d sigma_log
 #pragma unroll
         for (int k = 0; k < KC; ++k) acc[k][j] = fmaf(-xc[k], rr, acc[k][j]);
@@ -863,24 +907,44 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         const int r = RPI > 1 ? item / TC : 0, col = RPI > 1 ? item % TC : item;
         float* rs = rs0 + r * SLOT;
         const float imu = rs[col], is = fast_exp(rs[TC + col]);
-        const float ic1 = rs[2 * TC + col], ic2 = rs[3 * TC + col], ic3 = rs[4 * TC + col];
+        float ic1, ic2, ic3;
+        if (CODE8) {
+          const uint32_t w = __float_as_uint(rs[2 * TC + col]);
+          ic1 = s_dict[w & 255u];
+          ic2 = s_dict[kDictSize + ((w >> 8) & 255u)];
+          ic3 = s_dict[2 * kDictSize + ((w >> 16) & 255u)];
+        } else {
+          ic1 = rs[2 * TC + col]; ic2 = rs[3 * TC + col]; ic3 = rs[4 * TC + col];
+        }
         const float in = ic1 + ic2 + ic3;
         const float l1 = s_L[0][col], l2 = s_L[1][col], l3 = s_L[2][col];
         float gs, ge, ls;
         mc_samples<LOSS>(imu, is, ic1, ic2, in, l1, l2, l3, l1 - l2, a.S, s_ev[col], (uint32_t)(row_begin + lrb + r),
                          a.step, stream0, a.seed, gs, ge, ls);
-        rs[2 * TC + col] = gs * a.inv_S;
-        rs[3 * TC + col] = ge * is * a.inv_S;
+        float* const out = CODE8 ? s_scr + r * (NSCR * TC) : rs + 2 * TC;
+        out[col] = gs * a.inv_S;
+        out[TC + col] = ge * is * a.inv_S;
         if (LOSS)
-          rs[4 * TC + col] = fmaf(ls, a.inv_S, fmaf(ic1, s_L[3][col], fmaf(ic2, s_L[4][col], ic3 * s_L[5][col])));
+          out[2 * TC + col] = fmaf(ls, a.inv_S, fmaf(ic1, s_L[3][col], fmaf(ic2, s_L[4][col], ic3 * s_L[5][col])));
       }
       __syncwarp();
 #pragma unroll
       for (int r = 0; r < RPI; ++r) {
-        const Vec* st = reinterpret_cast<const Vec*>(rs0 + r * SLOT) + lane;
+        // CODE8: the scratch holds sums only where this row had items, stale values elsewhere -- an element without
+        // reads subtracts 0, as it subtracts its zero counts in the f32 form
+        const Vec* st = CODE8 ? reinterpret_cast<const Vec*>(s_scr + r * (NSCR * TC)) + lane
+                              : reinterpret_cast<const Vec*>(rs0 + r * SLOT + 2 * TC) + lane;
         float r1[EPL], r2[EPL];
-        vec_get<EPL>(st[2 * 32], r1);
-        vec_get<EPL>(st[3 * 32], r2);
+        vec_get<EPL>(st[0 * 32], r1);
+        vec_get<EPL>(st[1 * 32], r2);
+        if (CODE8) {
+#pragma unroll
+          for (int j = 0; j < EPL; ++j) {
+            const bool hit = (nz >> (r * EPL + j)) & 1u;
+            r1[j] = hit ? r1[j] : 0.f;
+            r2[j] = hit ? r2[j] : 0.f;
+          }
+        }
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
           gmu[r][j] -= r1[j];
@@ -888,9 +952,9 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         }
         if (LOSS) {
           float r3[EPL];
-          vec_get<EPL>(st[4 * 32], r3);
+          vec_get<EPL>(st[2 * 32], r3);
 #pragma unroll
-          for (int j = 0; j < EPL; ++j) acc[T::kLoss][j] -= r3[j];
+          for (int j = 0; j < EPL; ++j) acc[T::kLoss][j] -= CODE8 && !((nz >> (r * EPL + j)) & 1u) ? 0.f : r3[j];
         }
       }
     }
@@ -902,10 +966,10 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       if (act != 0 && (RPI == 1 || lr < n_rows)) {
         const Vec* st = reinterpret_cast<const Vec*>(rs0 + r * SLOT) + lane;
         float m1[EPL], v1[EPL], m2[EPL], v2[EPL];
-        vec_get<EPL>(st[5 * 32], m1);
-        vec_get<EPL>(st[6 * 32], v1);
-        vec_get<EPL>(st[7 * 32], m2);
-        vec_get<EPL>(st[8 * 32], v2);
+        vec_get<EPL>(st[(IA + 0) * 32], m1);
+        vec_get<EPL>(st[(IA + 1) * 32], v1);
+        vec_get<EPL>(st[(IA + 2) * 32], m2);
+        vec_get<EPL>(st[(IA + 3) * 32], v2);
         if (all_act) {
 #if BRIE_F32X2
 #pragma unroll

@@ -40,22 +40,43 @@ def _round_up(x, m):
     return (x + m - 1) // m * m
 
 
-def gathered_round_is_cheaper(cols, n_events, n_cells, n_layers, n_steps):
+def encode_counts(lib, counts, device):
+    """Packed count codes of padded (Nc, ld) float32 tiles (brie_encode_counts): (codes (Nc, ld) int32, dict (3, 256)
+    float32), or None when a layer has more than 255 distinct non-zero values (or a value that is negative or NaN).
+    Synchronises once, to read the number of values per layer."""
+    Nc, ld = counts[0].shape
+    codes = torch.empty((Nc, ld), dtype=torch.int32, device=device)
+    dct = torch.empty((3, 256), dtype=torch.float32, device=device)
+    n_values = torch.empty(3, dtype=torch.int32, device=device)
+    scratch = torch.empty(int(lib.brie_encode_counts_scratch_bytes()), dtype=torch.uint8, device=device)
+    st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    with torch.cuda.device(device):
+        _lib.check(lib.brie_encode_counts(Nc, ld, counts[0].data_ptr(), counts[1].data_ptr(),
+                                          counts[2].data_ptr() if len(counts) > 2 else None, codes.data_ptr(),
+                                          dct.data_ptr(), n_values.data_ptr(), scratch.data_ptr(), st))
+    if int(n_values.max()) > 255:
+        return None
+    return codes, dct
+
+
+def gathered_round_is_cheaper(cols, n_events, n_cells, n_layers, n_steps, count_bytes=None):
     """Extension round on gathered sub-fits or in place?  cols[m]: local event indices still active in model m.
 
-    Bytes per cell and step.  In place, every 8-event block (one 32-byte sector of each float32 array) that
+    Bytes per cell and step.  In place, every 8-event block (one 32-byte sector of each 4-byte array) that
     holds an active event moves whole: 48 B of state per model, and the counts once for the models
     co-resident on the tile.  Gathered, only active events move, but each model reads its own copy of the
     counts; add the gather and scatter passes (about 3 step-equivalents) and ~15 ms of set-up per round,
-    expressed in the same unit.  Gathered must win by 10 % to be chosen."""
+    expressed in the same unit.  Gathered must win by 10 % to be chosen.  count_bytes: bytes of counts per
+    element the step kernel reads, 4 * n_layers for float32 tiles (default), 4 for packed codes."""
+    cb = 4 * n_layers if count_bytes is None else count_bytes
     M = len(cols)
     n_act = sum(len(c) for c in cols)
     ev = np.zeros((M, _round_up(max(n_events, 1), 8)), bool)
     for m in range(M):
         ev[m, cols[m]] = True
     blk = ev.reshape(M, -1, 8).any(axis=2)
-    in_place = 8.0 * (48 * blk.sum() + 4 * n_layers * blk.any(axis=0).sum())
-    gathered = n_act * (48 + 4 * n_layers) * (1.0 + 3.0 / max(n_steps, 1)) + 1e11 / max(n_cells * n_steps, 1)
+    in_place = 8.0 * (48 * blk.sum() + cb * blk.any(axis=0).sum())
+    gathered = n_act * (48 + cb) * (1.0 + 3.0 / max(n_steps, 1)) + 1e11 / max(n_cells * n_steps, 1)
     return gathered <= 0.9 * in_place
 
 
@@ -81,12 +102,19 @@ class FitEngine:
     target : "ELBO" (default) or "marginLik" (model_TFProb.py:156-157, 188-189, 202-205).
     dist_group : torch.distributed process group for event-sharded fits with shared
         per-cell parameters (Kg > 0 or intercept_mode 'cell'); None = single GPU.
+    count_format : None (default) lets the fused step kernel read the counts as packed 8-bit
+        dictionary codes (4 B per element instead of 4 B per layer, bit-identical results) whenever
+        every layer has at most 255 distinct non-zero values; 'f32' keeps it on the float32 tiles.
+        The chosen form is `self.count_format` ('code8' or 'f32').
+    count_codes : `count_codes` of another engine over the same count tiles, reused instead of
+        encoding them again (the engines of one fit_BRIE_matrix chunk share one code tile).
     """
 
     def __init__(self, counts, effLen=None, Xc=None, Xg=None, masks=None, model_ids=None,
                  intercept=None, intercept_mode='gene', sigma=None, MC_size=1, seed=0,
                  group_size=None, event_offset=0, n_events_total=None, device=None,
-                 trace_cap=None, dist_group=None, n_events=None, target="ELBO"):
+                 trace_cap=None, dist_group=None, n_events=None, target="ELBO", count_format=None,
+                 count_codes=None):
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise RuntimeError("brie_b200: no CUDA device (there is no CPU fallback)")
@@ -153,6 +181,14 @@ class FitEngine:
         # zeros in every layer, brie_kernels.cuh phase B)
         if float(torch.stack([c.min() for c in self.counts]).min()) < 0:      # one device sync for all layers
             raise ValueError("brie_b200: count layers must be non-negative")
+        if count_format not in (None, 'f32'):
+            raise ValueError("brie_b200: count_format must be None or 'f32', got %r" % (count_format,))
+        # Only the ELBO step kernel reads codes (marginLik streams the float32 tiles itself).
+        if count_format is None and target == "ELBO":
+            self.count_codes = count_codes if count_codes is not None else encode_counts(self.lib, self.counts, dev)
+        else:
+            self.count_codes = None
+        self.count_format = 'f32' if self.count_codes is None else 'code8'
         self.h2d_bytes = sum(int(np.prod(c.shape)) * 4 for c in counts)
         if effLen is not None:
             eff = np.ones((3, ld), np.float32)
@@ -215,6 +251,9 @@ class FitEngine:
         b.active, b.loss_trace, b.scratch = self.active.data_ptr(), self.loss_trace.data_ptr(), self.scratch.data_ptr()
         self.bufs = b
         _lib.check(self.lib.brie_fit_bind(h, C.byref(b)))
+        if self.count_codes is not None:
+            _lib.check(self.lib.brie_fit_set_count_codes(h, self.count_codes[0].data_ptr(), 0,
+                                                         self.count_codes[1].data_ptr()))
         # Shared per-cell parameters on an event shard: the library all-reduces their gradients itself,
         # in stream order inside brie_fit_run_steps (BRIE_HOST_ALLREDUCE=1 keeps the older per-step
         # torch.distributed round trip, for A/B only).
@@ -379,9 +418,10 @@ class FitEngine:
         n_act = sum(len(c) for c in cols)
         if n_act == 0 or n_act == M * self.Ng:
             return False
-        if not force and not gathered_round_is_cheaper(cols, self.Ng, Nc, L, n_steps):
+        n_cnt = 1 if self.count_codes is not None else L                  # 4-byte count arrays per model column
+        if not force and not gathered_round_is_cheaper(cols, self.Ng, Nc, L, n_steps, count_bytes=4 * n_cnt):
             return False
-        per_col = M * Nc * (L + 6) * 4 * 1.05 + M * (n_steps + 64) * 4
+        per_col = M * Nc * (n_cnt + 6) * 4 * 1.05 + M * (n_steps + 64) * 4
         max_ld = int(0.8 * self._free_bytes() / per_col) // 128 * 128
         nmax = max(len(c) for c in cols)
         if max_ld < min(_lib.leading_dim(nmax), 256):
@@ -552,7 +592,8 @@ class FitEngine:
 class _GatheredFit:
     """Sub-fit over gathered columns of a parent FitEngine (brie_fit_buffers.event_ids): model m's
     column j is the parent's local event cols[m][j].  Holds its own dense tiles of the state, the
-    Adam moments, the counts and the lengths; shares Xc with the parent."""
+    Adam moments, the counts (the parent's code words when it steps on packed codes, else its float32
+    layers) and the lengths; shares Xc and the code dictionary with the parent."""
 
     def __init__(self, parent, cols, trace_cap):
         p = self.p = parent
@@ -581,7 +622,12 @@ class _GatheredFit:
             act[m, :len(c)] = 1
         self.ev_ids = torch.from_numpy(ev).to(dev)
         self.active = torch.from_numpy(act).to(dev)
-        self.counts = torch.empty((L, M, Nc, ld), dtype=f32, device=dev)
+        if p.count_codes is not None:
+            self.counts = None
+            self.codes = torch.empty((M, Nc, ld), dtype=torch.int32, device=dev)
+        else:
+            self.counts = torch.empty((L, M, Nc, ld), dtype=f32, device=dev)
+            self.codes = None
         self.Z_loc = torch.empty((M, Nc, ld), dtype=f32, device=dev)
         self.Z_std_log = torch.empty((M, Nc, ld), dtype=f32, device=dev)
         self.adam_Z = torch.empty((4, M, Nc, ld), dtype=f32, device=dev)
@@ -600,9 +646,10 @@ class _GatheredFit:
                 self.eff[m, :, self.n[m]:] = 1.0          # padding columns: harmless lengths
 
         b = _lib.FitBuffers()
-        for i in range(3):
-            b.counts[i] = self.counts[i].data_ptr() if i < L else None
-        b.counts_model_stride = Nc * ld
+        if self.counts is not None:
+            for i in range(3):
+                b.counts[i] = self.counts[i].data_ptr() if i < L else None
+            b.counts_model_stride = Nc * ld
         b.efflen3 = self.eff.data_ptr() if self.eff is not None else None
         b.efflen_model_stride = 3 * ld if self.eff is not None else 0
         b.event_ids = self.ev_ids.data_ptr()
@@ -613,6 +660,9 @@ class _GatheredFit:
         b.active, b.loss_trace, b.scratch = self.active.data_ptr(), self.loss_trace.data_ptr(), self.scratch.data_ptr()
         self.bufs = b
         _lib.check(lib.brie_fit_bind(self.h, C.byref(b)))
+        if self.codes is not None:
+            _lib.check(lib.brie_fit_set_count_codes(self.h, self.codes.data_ptr(), Nc * ld,
+                                                    p.count_codes[1].data_ptr()))
 
     def __del__(self):
         h = getattr(self, "h", None)
@@ -634,7 +684,10 @@ class _GatheredFit:
         out += [(p.intercept[m:m + 1], self.intercept[m:m + 1]), (p.sigma_log[m:m + 1], self.sigma_log[m:m + 1])]
         out += [(pmom[j, m], self.mom[j, m]) for j in range(2)]
         if inputs:
-            out += [(p.counts[i], self.counts[i, m]) for i in range(p.n_layers)]
+            if self.codes is not None:
+                out.append((p.count_codes[0], self.codes[m]))    # moved as 4-byte words: the bits are kept
+            else:
+                out += [(p.counts[i], self.counts[i, m]) for i in range(p.n_layers)]
             if self.eff is not None:
                 out.append((p.eff, self.eff[m]))
         if trace_rows:

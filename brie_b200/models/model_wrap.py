@@ -412,6 +412,7 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     brie_results = None
     n_iter_rows, lg_tests, wc_last, launches = [None] * (T + 1), [None] * T, [None] * T, 0
     lg_perm = {}                                                    # (t, b) -> loss_gene of permuted model (t, b)
+    codes = None                                                    # the chunk's packed count codes, encoded once
     for masks_e, ids_e, mode_e in plan:
         io, kw_e = None, common
         if ids_e[0] > T:                                            # permuted models: their columns appended to Xc
@@ -420,7 +421,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
             kw_e = dict(common, Xc=np.concatenate([Xc, np.stack(cols, axis=1)], axis=1))
         elif init_objs is not None:
             io = [init_objs[i] for i in ids_e]
-        eng = FitEngine(data, masks=masks_e, model_ids=ids_e, intercept_mode=mode_e, **kw_e)
+        eng = FitEngine(data, masks=masks_e, model_ids=ids_e, intercept_mode=mode_e, count_codes=codes, **kw_e)
+        codes = eng.count_codes
         eng.fit(n_eval=n_eval, init_objs=io, **keyargs)             # :144, :180
         t_ph = _tick("fit", t_ph)
         if timing is not None:
@@ -529,10 +531,10 @@ def _balanced_chunk(n_events, budget, n_gene):
 
 
 def _device_event_budget(Nc, n_models, n_layers, device=None, frac=0.7):
-    """Events per device chunk so that counts + (1+T) model states + outputs fit in HBM."""
+    """Events per device chunk so that counts, their packed codes, (1+T) model states and outputs fit in HBM."""
     import torch
     free, _ = torch.cuda.mem_get_info(device)
-    per_event = Nc * 4 * (n_layers + 6 * n_models + 3 + 1) * 1.05
+    per_event = Nc * 4 * (n_layers + 1 + 6 * n_models + 3 + 1) * 1.05
     return max(int(free * frac / per_event), 1)
 
 

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BRIE_ABI_VERSION 7
+#define BRIE_ABI_VERSION 8
 #define BRIE_MAX_MODELS 32
 #define BRIE_MAX_KC 16   /* widest design whose covariate contraction stays in registers / shared memory */
 #define BRIE_MAX_KG 8
@@ -111,7 +111,8 @@ typedef struct brie_fit_buffers {
    *  counts_model_stride: floats between the count tiles of consecutive models, 0 = all models share one tile;
    *  efflen_model_stride: likewise for efflen3 ((3, ld) per model), 0 = shared.
    * Only the step entry points work on such a fit (Kg = 0, cell_mode = 0, target ELBO); results go back with
-   * brie_scatter_events. */
+   * brie_scatter_events.  A sub-fit that steps on packed count codes (brie_fit_set_count_codes) may leave counts[]
+   * all NULL. */
   const int32_t* event_ids;
   int64_t counts_model_stride;
   int64_t efflen_model_stride;
@@ -161,6 +162,15 @@ int brie_fit_run_steps(brie_fit* fit, int32_t n_steps, int32_t trace_slot0, void
  * uncompacted step.  blk_ids = NULL restores the dense walk.  The list must cover every event
  * with active = 1 and must stay valid until replaced.  Needs ld % 8 == 0, Kg = 0, cell_mode = 0,
  * target ELBO. */
+/* Packed count codes for the fused step kernel (brie_encode_counts).  From now on the step kernel reads one 32-bit
+ * code word per element from `codes` ((Nc, ld) per model, codes_model_stride words apart, 0 = one tile shared by all
+ * models, as counts_model_stride) and decodes the counts of elements with reads from dict (DEVICE, (3, 256) floats),
+ * instead of streaming the float32 count tiles: 4 B of counts per element and step instead of 12 (8 with two layers).
+ * The decoded values are the tiles' own bit patterns, so results are bit-identical.  Everything else that reads
+ * counts (loss_gene, element terms, target marginLik) keeps reading the float32 tiles.  codes = NULL returns to the
+ * float32 tiles.  Both arrays must stay valid while set. */
+int brie_fit_set_count_codes(brie_fit* fit, const uint32_t* codes, int64_t codes_model_stride, const float* dict);
+
 int brie_fit_set_active_blocks(brie_fit* fit, const int32_t* blk_ids, int64_t blk_stride,
                                const int32_t* n_blk_host);
 
@@ -290,6 +300,19 @@ int brie_add_pseudo_count(int64_t n_cells, int64_t ld, float pseudo_count, float
 size_t brie_gene_stats_scratch_bytes(int64_t n_cells, int64_t ld);
 int brie_gene_stats(int64_t n_cells, int64_t ld, const float* c1, const float* c2, const float* c3,
                     double* stats, void* scratch, void* stream);
+
+/* Dictionary coding of the count tiles for brie_fit_set_count_codes.  Read counts (plus the pseudo-count) take few
+ * distinct values, so each element's layers fit one 32-bit word: byte l (l = 0, 1, 2) is the index of layer l's
+ * value in dict[l * 256 + .], byte 3 is 0.  dict[l * 256] = 0.0f (+0 and -0 both map to it), so a word is non-zero
+ * iff c1 + c2 + c3 > 0; the other entries are the layer's distinct non-zero values in ascending order, bit for bit.
+ * One pass over the (n_cells, ld) tiles (c3 may be NULL: its byte is 0) collects each layer's values, a second
+ * writes the code words.  n_values (DEVICE, 3 int32) receives the number of distinct non-zero values per layer; a
+ * value above 255 means the tiles cannot be coded -- more than 255 distinct non-zero values in a layer, or a
+ * negative or NaN count -- and then `codes` is left unwritten.  dict: (3, 256) floats.  scratch needs
+ * brie_encode_counts_scratch_bytes() bytes.  Nothing synchronises: read n_values after the stream. */
+size_t brie_encode_counts_scratch_bytes(void);
+int brie_encode_counts(int64_t n_cells, int64_t ld, const float* c1, const float* c2, const float* c3,
+                       uint32_t* codes, float* dict, int32_t* n_values, void* scratch, void* stream);
 
 /* Column gather of a dense tile (`adata._inplace_subset_var`, preprocessing.py:63, without a
  * host round trip): out[r, j] = in[r, src[j]] for j < n_out, zero padding up to ld_out. */
