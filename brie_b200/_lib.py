@@ -8,7 +8,7 @@ import ctypes as C
 import os
 
 BRIE_MAX_MODELS = 32
-ABI_VERSION = 8
+ABI_VERSION = 9
 TARGETS = {"ELBO": 0, "marginLik": 1}
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BRIE_LIB_PATH", os.path.join(_HERE, "libbrie_b200.so"))
@@ -76,6 +76,8 @@ SYMBOLS = {
     "brie_fit_set_comm": (C.c_int, [_P, _P]),
     "brie_fit_eval_loss_gene": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P]),
     "brie_fit_posterior": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P]),
+    "brie_fit_wald_sizes": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_size_t), C.POINTER(C.c_int32)]),
+    "brie_fit_wald_info": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
     "brie_fit_element_terms": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, C.c_uint32, C.c_int32, _P, _P, _P, _P]),
     "brie_resample_counts": (C.c_int, [C.c_uint64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, _P, _P, _P, _P, _P,
                                        _P, _P]),

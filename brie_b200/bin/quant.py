@@ -37,7 +37,7 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
           intercept=None, intercept_mode='gene', nproc=1, min_counts=50,
           min_counts_uniq=10, min_cells_uniq=30, min_MIF_uniq=0.001,
           min_iter=5000, max_iter=20000, MC_size=1, batch_size=500000,
-          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0):
+          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0, wald=False):
     """CLI driver (quant.py:13-130).  `nproc` is accepted for compatibility (host threads are
     not on the hot path any more); `seed` keys the counter-based noise (new, default 0).
     `out_dir` (new): directory for `.npy` memory maps of the dense (cells, events) output layers
@@ -47,7 +47,9 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     torchrun it defaults to `<out_file stem>.layers/`, so no (cells, events) array ever travels through a
     collective.  `resume` (new, needs out_dir): skip the event chunks a previous run of the same fit left
     there (checkpoint / restart).  `n_perm` (new): permutation replicates per tested covariate; adds the
-    pooled permutation p-values and their FDR to the container (varm) and the table (fitBRIE).
+    pooled permutation p-values and their FDR to the container (varm) and the table (fitBRIE).  `wald`
+    (new): standard errors, Wald p-values and their FDR for every cell coefficient, from the fitted
+    posterior without refits (fitBRIE); in the container (varm) and the table.
 
     Multi-GPU: launch one process per GPU (`python -m torch.distributed.run --nproc-per-node N
     -m brie_b200.bin.quant ...`); every rank reads the input, fits its own event shard
@@ -107,7 +109,7 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     fitBRIE(adata, Xc=Xc, Xg=Xg, LRT_index=LRT_index, layer_keys=layer_keys,
             intercept=intercept, intercept_mode=intercept_mode,
             min_iter=min_iter, max_iter=max_iter, MC_size=MC_size, batch_size=batch_size,
-            pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed, n_perm=n_perm,
+            pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed, n_perm=n_perm, wald=wald,
             **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
 
     adata.uns['brie_version'] = brie_b200.__version__
@@ -184,6 +186,10 @@ def main():
         help="Permutation replicates per tested feature: refit the model with that feature's cells permuted "
              "--nPerm times and add p-values against the permutation null pooled over all events, with their "
              "FDR (columns <feature>_pval_perm, <feature>_FDR_perm) [default: %default]")
+    group4.add_option("--wald", action="store_true", dest="wald", default=False,
+        help="Standard errors and Wald p-values of every cell coefficient from the fitted posterior, without "
+             "refits, with their FDR over all events (columns <feature>_se, <feature>_pval_wald, "
+             "<feature>_FDR_wald); covers every feature, also those not in --LRTindex")
     parser.add_option_group(group1)
     parser.add_option_group(group2)
     parser.add_option_group(group3)
@@ -218,7 +224,7 @@ def main():
           options.min_uniq_count, options.min_cell, options.min_MIF,
           options.min_iter, options.max_iter, options.MC_size,
           options.batch_size, options.pseudo_count, options.test_base, options.seed,
-          options.out_dir, options.resume, options.n_perm)
+          options.out_dir, options.resume, options.n_perm, options.wald)
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         if dist.is_initialized():

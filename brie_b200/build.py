@@ -11,7 +11,7 @@ from concurrent.futures import ThreadPoolExecutor
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_HERE, "csrc")
 UNITS = ["brie_abi.cu", "brie_ingest.cu", "brie_comm.cu"]
-HEADERS = [os.path.join(_CSRC, h) for h in ("brie_kernels.cuh", "brie_margin.cuh", "brie_philox.h", "brie_host.h")] + \
+HEADERS = [os.path.join(_CSRC, h) for h in ("brie_kernels.cuh", "brie_margin.cuh", "brie_wald.cuh", "brie_philox.h", "brie_host.h")] + \
     [os.path.join(os.path.dirname(_HERE), "include", "brie_b200.h")]
 OBJ_DIR = os.path.join(_HERE, "build")
 OUT = os.path.join(_HERE, "libbrie_b200.so")

@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <string>
 #include <vector>
@@ -15,6 +16,7 @@
 #include "../../include/brie_b200.h"
 #include "brie_kernels.cuh"
 #include "brie_margin.cuh"
+#include "brie_wald.cuh"
 
 #include "brie_host.h"
 
@@ -798,6 +800,99 @@ int brie_fit_element_terms(brie_fit* f, int32_t model, const float* c1, const fl
   element_terms_kernel<<<grid_1d(d.n_cells * d.ld, 256), 256, 0, (cudaStream_t)stream>>>(a);
   BRIE_CUDA(cudaGetLastError());
   f->launches += 1;
+  return BRIE_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Geometry of the Wald information pass of model m (brie_wald.cuh): x~ width, pair block, row chunks.
+struct WaldPlan {
+  int width, has_b, kt, n_pairs, pb, n_pblk, n_tiles, n_chunks;
+  int64_t rows_per_chunk;
+  size_t scratch_bytes;
+};
+
+int wald_plan(const brie_fit* f, int32_t model, WaldPlan* w) {
+  if (!f || !f->bound) return fail(BRIE_ERR_ARG, "fit not bound");
+  const brie_fit_desc& d = f->d;
+  if (model < 0 || model >= d.n_models) return fail(BRIE_ERR_ARG, "model index out of range");
+  if (d.target != BRIE_TARGET_ELBO)
+    return fail(BRIE_ERR_UNSUPPORTED, "Wald information needs a trained posterior (target ELBO)");
+  if (f->buf.event_ids || f->buf.counts_model_stride || f->buf.efflen_model_stride)
+    return fail(BRIE_ERR_UNSUPPORTED, "Wald information is computed on the parent fit, not on a gathered sub-fit");
+  w->width = f->wide ? d.xc_width[model] : __builtin_popcount(d.xc_mask[model]);
+  w->has_b = (!d.cell_mode && d.train_intercept) ? 1 : 0;
+  w->kt = w->width + w->has_b;
+  w->n_pairs = w->kt * (w->kt + 1) / 2;
+  w->pb = w->n_pairs <= 4 ? 4 : (w->n_pairs <= 12 ? 12 : kWaldMaxPairs);
+  w->n_pblk = (int)ceil_div(w->n_pairs, w->pb);
+  w->n_tiles = (int)ceil_div(d.n_events, kWaldCols);
+  // Row chunks of >= kWaldMinRows cells, at most kWaldMaxChunks of them: a function of n_cells alone, so the float64
+  // sums over cells associate the same way whatever the event count -- an event chunk or shard of a fit gets the
+  // same bits as the whole -- and the scratch stays within kWaldMaxChunks partials per output.
+  const int64_t blocks = (int64_t)w->n_tiles * w->n_pblk;
+  const int64_t n_chunks = std::min<int64_t>(ceil_div(d.n_cells, kWaldMinRows), kWaldMaxChunks);
+  w->rows_per_chunk = ceil_div(ceil_div(d.n_cells, n_chunks), kWaldBatch) * kWaldBatch;
+  w->n_chunks = (int)ceil_div(d.n_cells, w->rows_per_chunk);
+  if (blocks > 0x7fffffffLL) return fail(BRIE_ERR_UNSUPPORTED, "too many event tiles x pair blocks");
+  w->scratch_bytes = (size_t)w->n_chunks * w->n_pairs * d.ld * sizeof(double);
+  return BRIE_OK;
+}
+
+template <int PB>
+cudaError_t launch_wald(const WaldArgs& a, dim3 grid, cudaStream_t s) {
+  wald_info_kernel<PB><<<grid, kWaldCols * kWaldRowGroups, 0, s>>>(a);
+  return cudaGetLastError();
+}
+
+}  // namespace
+
+extern "C" {
+
+int brie_fit_wald_sizes(const brie_fit* f, int32_t model, size_t* scratch_bytes, int32_t* k_tilde) {
+  if (!scratch_bytes || !k_tilde) return fail(BRIE_ERR_ARG, "null argument");
+  WaldPlan w;
+  int rc = wald_plan(f, model, &w);
+  if (rc) return rc;
+  *scratch_bytes = w.scratch_bytes;
+  *k_tilde = w.kt;
+  return BRIE_OK;
+}
+
+int brie_fit_wald_info(brie_fit* f, int32_t model, double* info, void* scratch, void* stream) {
+  WaldPlan w;
+  int rc = wald_plan(f, model, &w);
+  if (rc) return rc;
+  if (w.n_pairs == 0) return BRIE_OK;
+  if (!info || !scratch) return fail(BRIE_ERR_ARG, "info and scratch required");
+  if ((((uintptr_t)info) & 7u) != 0 || (((uintptr_t)scratch) & 7u) != 0)
+    return fail(BRIE_ERR_ARG, "info and scratch must be 8-byte aligned");
+  const brie_fit_desc& d = f->d;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t plane = d.n_cells * d.ld;
+  WaldArgs a;
+  memset(&a, 0, sizeof a);
+  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld;
+  a.Zs = f->buf.Z_std_log + model * plane;
+  a.tau = f->buf.sigma_log + (int64_t)model * (d.cell_mode ? d.n_cells : d.ld);
+  a.xc_stride = d.Kc > 0 ? d.Kc : 1;
+  a.Xc = f->buf.Xc ? f->buf.Xc + (int64_t)model * d.n_cells * a.xc_stride : nullptr;
+  a.width = w.width; a.xc_mask = d.xc_mask[model]; a.wide = f->wide ? 1 : 0; a.has_b = w.has_b;
+  a.n_pairs = w.n_pairs; a.cell_tau = d.cell_mode; a.rows_per_chunk = w.rows_per_chunk; a.n_tiles = w.n_tiles;
+  a.part = (double*)scratch;
+  if (w.width > 0 && !a.Xc) return fail(BRIE_ERR_ARG, "Xc required");
+  const dim3 grid((unsigned)((int64_t)w.n_tiles * w.n_pblk), (unsigned)w.n_chunks);
+  switch (w.pb) {
+    case 4: BRIE_CUDA(launch_wald<4>(a, grid, s)); break;
+    case 12: BRIE_CUDA(launch_wald<12>(a, grid, s)); break;
+    default: BRIE_CUDA(launch_wald<kWaldMaxPairs>(a, grid, s)); break;
+  }
+  const int64_t n_out = d.n_events * w.n_pairs;
+  wald_reduce_kernel<<<(unsigned)ceil_div(n_out, 256), 256, 0, s>>>(a.part, w.n_chunks, w.n_pairs, d.ld, d.n_events, info);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 2;
   return BRIE_OK;
 }
 

@@ -80,6 +80,57 @@ def gathered_round_is_cheaper(cols, n_events, n_cells, n_layers, n_steps, count_
     return gathered <= 0.9 * in_place
 
 
+def pair_index(kt):
+    """(rows, cols) of the packed pairs k <= l of a kt x kt symmetric matrix, row-major over the upper triangle
+    (the order of brie_fit_wald_info's output)."""
+    return np.triu_indices(kt)
+
+
+def unpack_pairs(packed, kt):
+    """(..., kt (kt + 1) / 2) packed upper triangles -> (..., kt, kt) symmetric matrices."""
+    packed = np.asarray(packed)
+    k, l = pair_index(kt)
+    out = np.zeros(packed.shape[:-1] + (kt, kt), packed.dtype)
+    out[..., k, l] = packed
+    out[..., l, k] = packed
+    return out
+
+
+WALD_RCOND = 1e-12
+
+
+def wald_from_info(coef, info):
+    """Wald standard errors and p-values of per-event coefficients `coef` (Ng, K) from their observed information
+    `info` (Ng, K, K): se = sqrt(diag(info^-1)), pval = chi2.sf((coef / se)^2, 1).  An event whose information is
+    not positive definite -- Cholesky fails, or the reciprocal condition number of the unit-diagonal rescaling is
+    below WALD_RCOND (e.g. too few cells with reads) -- gets se NaN and pval 1.0, so BH still works.
+    Returns (se, pval), both (Ng, K) float64."""
+    from scipy.stats import chi2
+    coef = np.asarray(coef, np.float64)
+    info = np.asarray(info, np.float64)
+    Ng, K = coef.shape
+    se = np.full((Ng, K), np.nan)
+    if K > 0 and Ng > 0:
+        with np.errstate(invalid='ignore'):
+            d = np.sqrt(np.diagonal(info, axis1=1, axis2=2))         # rescale to a unit diagonal first
+        ok = np.all(np.isfinite(info), axis=(1, 2)) & np.all(d > 0, axis=1)
+        dd = np.where(ok[:, None], d, 1.0)
+        with np.errstate(invalid='ignore'):
+            R = np.where(ok[:, None, None], info / dd[:, :, None] / dd[:, None, :], np.eye(K))
+        ev = np.linalg.eigvalsh(R)
+        ok &= ev[:, 0] > WALD_RCOND * ev[:, -1]
+        idx = np.flatnonzero(ok)
+        if idx.size:
+            L = np.linalg.cholesky(R[idx])                            # batched; PD after the checks above
+            Linv = np.linalg.solve(L, np.broadcast_to(np.eye(K), L.shape))
+            diag_inv = (Linv ** 2).sum(axis=1)                        # diag(R^-1) = column sums of Linv^2
+            se[idx] = np.sqrt(diag_inv) / d[idx]
+    with np.errstate(invalid='ignore', divide='ignore'):
+        pval = chi2.sf((coef / se) ** 2, df=1)
+    pval[~np.isfinite(se)] = 1.0
+    return se, pval
+
+
 class FitEngine:
     """Device-resident batched fit.
 
@@ -491,6 +542,23 @@ class FitEngine:
                 int(mc_size), int(noise_step), int(bool(margin)), ptr(o_ll), ptr(o_kl), ptr(o_pm), self._stream()))
         cut = lambda t: t[:, :self.Ng] if t is not None else None
         return cut(o_ll), cut(o_kl), cut(o_pm)
+
+    def wald_info(self, m=0):
+        """(Ng, K~, K~) float64 observed information of model m's per-event regression parameters from the fitted
+        posterior (brie_fit_wald_info): x~ = model m's Xc columns in mask order (its Wc rows), then the intercept
+        when it is per-event and trained."""
+        nbytes, kt = C.c_size_t(), C.c_int32()
+        _lib.check(self.lib.brie_fit_wald_sizes(self.h, int(m), C.byref(nbytes), C.byref(kt)))
+        kt = kt.value
+        n_pairs = kt * (kt + 1) // 2
+        if n_pairs == 0:
+            return np.zeros((self.Ng, 0, 0))
+        packed = torch.empty((self.Ng, n_pairs), dtype=torch.float64, device=self.device)
+        scratch = torch.empty(max(int(nbytes.value), 8), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.brie_fit_wald_info(self.h, int(m), packed.data_ptr(), scratch.data_ptr(),
+                                                   self._stream()))
+        return unpack_pairs(packed.cpu().numpy(), kt)
 
     # ------------------------------------------------------------------ schedule
     def fit(self, min_iter=1000, max_iter=5000, add_iter=500, epsilon_conv=1e-2, n_eval=500,

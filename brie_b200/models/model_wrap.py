@@ -12,7 +12,7 @@ import time
 import numpy as np
 from scipy.stats import chi2
 
-from ..engine import FitEngine
+from ..engine import FitEngine, wald_from_info
 from ..sharding import event_shards
 from ..utils.layer_store import LayerStore, BIG_KEYS
 from ..settings import verbosity
@@ -112,6 +112,60 @@ def _set_perm_outputs(res):
         res.fdr_perm[:, i] = fdr_bh(res.pval_perm[:, i])
 
 
+def check_wald(wald, target):
+    """Validate `wald` against the fit's `target` (before any device work): a marginLik fit trains no posterior."""
+    wald = bool(wald)
+    if wald and target == "marginLik":
+        raise ValueError("wald=True needs target 'ELBO': a marginLik fit has no trained posterior")
+    return wald
+
+
+def _wald_of_model(eng, j):
+    """(se, pval, width) of model j of a fitted engine: Wald statistics of its Wc rows, then of its intercept when
+    that is per-event and trained, from the observed information of its posterior (FitEngine.wald_info)."""
+    import torch
+    w = len(eng.masks[j])
+    coef = [eng.Wc[j, :w, :eng.Ng].T.double()]
+    if not eng.cell_mode and eng.intercept_const is None:
+        coef.append(eng.intercept[j, :eng.Ng, None].double())
+    se, pval = wald_from_info(torch.cat(coef, dim=1).cpu().numpy(), eng.wald_info(j))
+    return se, pval, w
+
+
+def _set_fdr_wald(res):
+    """fdr_wald: BH over all events of the result, per cell_coeff row (the pooled scope of fdr_perm)."""
+    res.fdr_wald = np.zeros(res.pval_wald.shape)
+    for i in range(res.fdr_wald.shape[1]):
+        res.fdr_wald[:, i] = fdr_bh(res.pval_wald[:, i])
+
+
+def _set_wald_outputs(res, per_model, full, base_cols, tested):
+    """Wald outputs in the layout of cell_coeff: model 0's Xc rows, then (base_mode 'null') the last row of each
+    test model t, from model t's own information.  per_model[m] = _wald_of_model of model id m."""
+    se0, p0, w0 = per_model[0]
+    se, pv = [se0[:, :w0]], [p0[:, :w0]]
+    if not full:
+        for t in range(len(tested)):
+            se_t, p_t, w_t = per_model[1 + t]
+            se.append(se_t[:, w_t - 1:w_t])
+            pv.append(p_t[:, w_t - 1:w_t])
+    res.cell_coeff_se = np.concatenate(se, axis=1).T                # (rows, Ng), as cell_coeff
+    res.pval_wald = np.concatenate(pv, axis=1)                      # (Ng, rows)
+    if se0.shape[1] > w0:
+        res.intercept_se = se0[:, w0][None, :]                      # (1, Ng), as a per-event intercept
+    res.wald_columns = [int(k) for k in base_cols] + ([] if full else [int(k) for k in tested])
+    _set_fdr_wald(res)
+
+
+def _append_wald(out, r):
+    """Event-axis concatenation of the Wald outputs of two results (fdr_wald is recomputed over all events)."""
+    out.cell_coeff_se = np.append(out.cell_coeff_se, r.cell_coeff_se, axis=1)
+    for k in ('pval_wald', 'fdr_wald'):
+        setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
+    if hasattr(r, 'intercept_se'):
+        out.intercept_se = np.append(out.intercept_se, r.intercept_se, axis=1)
+
+
 class BRIE_RV():
     """Return value object for BRIE2 model (model_wrap.py:15-76)."""
 
@@ -166,6 +220,8 @@ class BRIE_RV():
         if hasattr(new_RV, 'ELBO_gain_perm'):           # pval_perm / fdr_perm: fitBRIE recomputes them over all events
             for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
                 setattr(self, k, np.append(getattr(self, k), getattr(new_RV, k), axis=0))
+        if hasattr(new_RV, 'pval_wald'):
+            _append_wald(self, new_RV)
         if hasattr(new_RV, 'n_iter'):
             self.n_iter = np.append(self.n_iter, new_RV.n_iter, axis=1)
         if getattr(self, 'timing', None) is not None and getattr(new_RV, 'timing', None) is not None:
@@ -297,7 +353,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     init key, default 0), `group_size` / `event_offset` / `n_events_total` (reference
     batch geometry when called from fitBRIE), `device`, `init_objs` (per-model
     injected initial values: [base, refit_0, ...]), `n_eval` (loss_gene evaluations,
-    500 in the reference), `dist_group`, `n_perm` (permutation null, default 0: see below).
+    500 in the reference), `dist_group`, `n_perm` (permutation null, default 0: see below), `wald`
+    (Wald tests from the fitted posterior, default False: see below).
     All other **keyargs go to the fit schedule as in the reference (`min_iter, max_iter,
     add_iter, epsilon_conv, MC_size`).
 
@@ -308,6 +365,12 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     against the gains of every event and replicate (`perm_pvalue`); and `fdr_perm`, BH over all
     events.  Permuted models only evaluate `loss_gene`; the observed outputs are bit-identical to
     the n_perm = 0 fit.
+
+    `wald=True` adds Wald statistics of the cell coefficients from the observed information of the fitted
+    posterior (FitEngine.wald_info; no refit): `cell_coeff_se` in the layout of `cell_coeff` (model 0's rows;
+    base_mode 'null': then the last row of each test model, from that model's own information), `intercept_se`
+    (1, Ng) when the intercept is per-event and trained, `pval_wald` / `fdr_wald` (Ng, rows of cell_coeff; BH
+    over all events) and `wald_columns`, the Xc column of each cell_coeff row.  Every other output is unchanged.
     """
     from scipy.sparse import issparse
     seed = keyargs.pop('seed', 0)
@@ -324,6 +387,7 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     out_sink = keyargs.pop('out_sink', None)                        # _ChunkSink: fitBRIE's output arrays
     n_tests = len(LRT_index) if LRT_index is not None else (0 if Xc is None else np.shape(Xc)[1])
     n_perm = check_n_perm(keyargs.pop('n_perm', 0), n_tests)
+    wald = check_wald(keyargs.pop('wald', False), target)
     for k in ('optimizer', 'learn_rate', 'verbose'):                # accepted and ignored (:214-237)
         keyargs.pop(k, None)
 
@@ -412,6 +476,7 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     brie_results = None
     n_iter_rows, lg_tests, wc_last, launches = [None] * (T + 1), [None] * T, [None] * T, 0
     lg_perm = {}                                                    # (t, b) -> loss_gene of permuted model (t, b)
+    wald_out = {}                                                   # model id -> _wald_of_model (base, null-mode tests)
     codes = None                                                    # the chunk's packed count codes, encoded once
     for masks_e, ids_e, mode_e in plan:
         io, kw_e = None, common
@@ -433,6 +498,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
                 lg_perm[divmod(mid - 1 - T, n_perm)] = eng.loss_gene[j].cpu().numpy()
                 continue
             n_iter_rows[mid] = eng.n_iter[j]
+            if wald and (mid == 0 or not full):
+                wald_out[mid] = _wald_of_model(eng, j)
             if mid == 0:
                 brie_results = _rv_from_engine(eng, j, Xc[:, base_cols], Xg, intercept_mode, out_sink)   # :146
             else:
@@ -446,6 +513,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     brie_results.launch_count = launches
     brie_results.h2d_bytes = h2d_bytes
     brie_results.timing = timing
+    if wald:
+        _set_wald_outputs(brie_results, wald_out, full, base_cols, LRT_index)
     if T == 0:                                                      # :152-153
         return brie_results
 
@@ -499,6 +568,8 @@ def _merge_shared(parts):
         if hasattr(r, 'ELBO_gain_perm'):
             for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
                 setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
+        if hasattr(r, 'pval_wald'):
+            _append_wald(out, r)
     out.shape = (out.Nc, out.Ng)
     if hasattr(out, 'pval'):               # one fit => one multiple-testing scope over all events
         for i in range(out.fdr.shape[1]):
@@ -555,6 +626,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     `n_perm` (not in the reference, default 0): permutation replicates per tested covariate, see
     fit_BRIE_matrix; `pval_perm` / `fdr_perm` are pooled over all events of the fit (every chunk and
     rank) and stored as varm['ELBO_gain_perm', 'pval_perm', 'fdr_perm'] with uns['brie_param']['n_perm'].
+    `wald` (not in the reference, default False): Wald tests from the fitted posterior, see fit_BRIE_matrix;
+    stored as varm['cell_coeff_se', 'pval_wald', 'fdr_wald'] (and varm['intercept_se'] in gene mode) with
+    uns['brie_param']['wald'] and ['wald_columns']; fdr_wald is BH over all events of the fit.
 
     Returns the BRIE_RV result and adds to `adata` exactly the keys the reference adds
     (obsm['Xc'], varm['cell_coeff'], varm['Xg'], obsm['gene_coeff'], varm|obsm['intercept',
@@ -572,6 +646,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     n_perm = check_n_perm(keyargs.pop('n_perm', 0), len(LRT_index))
     if n_perm > 0:                         # (absent at 0: the fit signature of a checkpoint stays as it was)
         keyargs['n_perm'] = n_perm
+    wald = check_wald(keyargs.pop('wald', False), keyargs.get('target', "ELBO"))
+    if wald:                               # (likewise absent when False)
+        keyargs['wald'] = True
     out_dir = keyargs.pop('out_dir', None)
     resume = keyargs.pop('resume', False)
     out_keys = tuple(keyargs.pop('out_keys', None) or BIG_KEYS)
@@ -673,6 +750,8 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
 
     if n_perm > 0:                         # one pooled null over every event of the fit, the same on every rank
         _set_perm_outputs(ResVal)
+    if wald:                               # one BH scope over every event of the fit
+        _set_fdr_wald(ResVal)
 
     # update adata (:271-311)
     if Xc.shape[0] > 0:
@@ -704,6 +783,12 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     if n_perm > 0:
         for k in ('ELBO_gain_perm', 'pval_perm', 'fdr_perm'):
             adata.varm[k] = getattr(ResVal, k)
+    if wald:
+        adata.varm['cell_coeff_se'] = ResVal.cell_coeff_se.T
+        adata.varm['pval_wald'] = ResVal.pval_wald
+        adata.varm['fdr_wald'] = ResVal.fdr_wald
+        if hasattr(ResVal, 'intercept_se') and ResVal.intercept_mode == 'gene':
+            adata.varm['intercept_se'] = ResVal.intercept_se.T
 
     adata.uns['brie_param'] = {
         'LRT_index': LRT_index,
@@ -716,4 +801,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     }
     if n_perm > 0:
         adata.uns['brie_param']['n_perm'] = n_perm
+    if wald:
+        adata.uns['brie_param']['wald'] = True
+        adata.uns['brie_param']['wald_columns'] = list(ResVal.wald_columns)
     return ResVal

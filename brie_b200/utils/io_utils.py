@@ -90,4 +90,10 @@ def dump_results(adata):
             label = names[feature] if names is not None else 'X%d' % pos
             table[label + '_pval_perm'] = adata.varm['pval_perm'][:, pos]
             table[label + '_FDR_perm'] = adata.varm['fdr_perm'][:, pos]
+    if 'pval_wald' in adata.varm:          # Wald tests (brie-quant --wald): one set per cell_coeff row, labelled by
+        for j, feature in enumerate(adata.uns['brie_param']['wald_columns']):    # its covariate, after all others
+            label = names[feature] if names is not None else 'X%d' % feature
+            table[label + '_se'] = adata.varm['cell_coeff_se'][:, j]
+            table[label + '_pval_wald'] = adata.varm['pval_wald'][:, j]
+            table[label + '_FDR_wald'] = adata.varm['fdr_wald'][:, j]
     return table

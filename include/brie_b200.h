@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BRIE_ABI_VERSION 8
+#define BRIE_ABI_VERSION 9
 #define BRIE_MAX_MODELS 32
 #define BRIE_MAX_KC 16   /* widest design whose covariate contraction stays in registers / shared memory */
 #define BRIE_MAX_KG 8
@@ -215,6 +215,24 @@ int brie_fit_eval_loss_gene(brie_fit* fit, int32_t n_eval, int32_t mc_size, floa
 /* Replaces the Psi / Psi95CI / Z_std properties (model_TFProb.py:88-106) for one model. */
 int brie_fit_posterior(brie_fit* fit, int32_t model, float* Psi, float* Psi95CI, float* Z_std,
                        void* stream);
+
+/* Observed information of model `model`'s per-event regression parameters from its fitted posterior (no reference
+ * counterpart; DESIGN §2.2).  Given W, b and sigma the exact posterior of Z factorises over (cell, event), so Louis'
+ * missing-information formula gives, per event g,
+ *   I_g = sum_c w_cg x~_c x~_c^T,  w_cg = max(sigma^2 - s_cg^2, 0) / sigma^4,  s_cg = exp(Z_std_log[model, c, g]),
+ * sigma = exp(sigma_log) of the event (or, cell_mode, of the cell).  x~_c is the model's design row: its Xc columns in
+ * mask order (xc_mask bits, or the first xc_width columns of the wide form: the order of its Wc rows), then a 1 when
+ * the intercept is per-event and trained (cell_mode 0, train_intercept 1).  Wg and a per-cell intercept / sigma are
+ * known offsets.  K~ = that width.
+ *  brie_fit_wald_sizes : scratch bytes and K~ of `model`;
+ *  brie_fit_wald_info  : info (DEVICE, (n_events, K~ (K~ + 1) / 2) float64, row-major) receives the upper triangle
+ *                        of each I_g, pairs (k <= l) row-major over x~; scratch needs the size above.  Reads only
+ *                        the step entry points' state (Z_std_log, sigma_log, Xc), so it works on a fit whose
+ *                        extension rounds ran on gathered sub-fits (not on a sub-fit itself).  Deterministic: no
+ *                        atomics, repeated calls give bit-identical output.  Target ELBO only (marginLik trains no
+ *                        posterior). */
+int brie_fit_wald_sizes(const brie_fit* fit, int32_t model, size_t* scratch_bytes, int32_t* k_tilde);
+int brie_fit_wald_info(brie_fit* fit, int32_t model, double* info, void* scratch, void* stream);
 
 /* Replaces the tensors the public model API returns for one model (BRIE2.logLik_MC model_TFProb.py:130-191,
  * Z_prior :118-127, the KL of get_loss :208), as dense (Nc, ld) arrays; any output may be NULL.
