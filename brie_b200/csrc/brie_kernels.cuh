@@ -732,6 +732,12 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
 #pragma unroll
     for (int r = 0; r < RPI; ++r) {
       const int lr = lrb + r;
+      // In a chunk with an odd number of rows the second row of the last iteration does not exist.  Its slot and row
+      // constants are zero-filled (mu = 0, log s = 0, x_c = 0), so its prior mean is the event's intercept b and it
+      // would add b / sigma^2, 1 - (b^2 + 1) / sigma^2 and a KL term to the per-event intercept, sigma_log and loss
+      // sums; those take zero for it (warp-uniform).  Its Wc terms are x_c * r = 0, and in cell mode (b = tau = 0
+      // from the zero-filled row constants) every term is exactly 0.
+      const bool real_row = RPI == 1 || CELL || lr < n_rows;
       const Vec* st = reinterpret_cast<const Vec*>(rs0 + r * SLOT) + lane;
       float xc[KC > 0 ? KC : 1], wg[KG > 0 ? KG : 1];
       float b_row = 0.f, tau_row = 0.f;
@@ -810,14 +816,16 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
           const float2 t = f2_fma(f2_splat(xc[k]), nr, make_float2(acc[k][j0], acc[k][j1]));
           acc[k][j0] = t.x; acc[k][j1] = t.y;
         }
+        const float2 rrs = real_row ? rr : f2_splat(0.f), gts = real_row ? gt : f2_splat(0.f);
         if (!CELL) {
-          const float2 t = f2_sub(make_float2(acc[T::kGB][j0], acc[T::kGB][j1]), rr);
+          const float2 t = f2_sub(make_float2(acc[T::kGB][j0], acc[T::kGB][j1]), rrs);
           acc[T::kGB][j0] = t.x; acc[T::kGB][j1] = t.y;
-          const float2 u = f2_add(make_float2(acc[T::kGT][j0], acc[T::kGT][j1]), gt);
+          const float2 u = f2_add(make_float2(acc[T::kGT][j0], acc[T::kGT][j1]), gts);
           acc[T::kGT][j0] = u.x; acc[T::kGT][j1] = u.y;
         }
         if (LOSS) {                                                          // TFP _kl_normal_normal
-          const float2 kl = f2_sub(f2_fma(f2_splat(0.5f), q2, f2_mul(f2_splat(0.5f), e2m1)), d);
+          float2 kl = f2_sub(f2_fma(f2_splat(0.5f), q2, f2_mul(f2_splat(0.5f), e2m1)), d);
+          if (!real_row) kl = f2_splat(0.f);
           const float2 t = f2_add(make_float2(acc[T::kLoss][j0], acc[T::kLoss][j1]), kl);
           acc[T::kLoss][j0] = t.x; acc[T::kLoss][j1] = t.y;
         }
@@ -857,10 +865,10 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
 #pragma unroll
         for (int k = 0; k < KC; ++k) acc[k][j] = fmaf(-xc[k], rr, acc[k][j]);
         if (!CELL) {
-          acc[T::kGB][j] -= rr;
-          acc[T::kGT][j] += gt;
+          acc[T::kGB][j] -= real_row ? rr : 0.f;
+          acc[T::kGT][j] += real_row ? gt : 0.f;
         }
-        if (LOSS) acc[T::kLoss][j] += 0.5f * q2 + 0.5f * (e2 - 1.0f) - d;  // TFP _kl_normal_normal
+        if (LOSS) acc[T::kLoss][j] += real_row ? 0.5f * q2 + 0.5f * (e2 - 1.0f) - d : 0.f;  // TFP _kl_normal_normal
         if (NCELL > 0 && (g0 + j) < a.Ng) {
 #pragma unroll
           for (int k = 0; k < KG; ++k) cacc[k] = fmaf(-xg[k][j], rr, cacc[k]);
@@ -871,6 +879,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         }
       }
 #endif
+      static_assert(!EXT || RPI == 1, "the wide-design store below writes every row of an iteration");
       if (EXT && act != 0)   // r = (mu - m) / sigma^2 of this row, for the gradient GEMMs (frozen lanes keep their old values: unused)
         __stcs(reinterpret_cast<Vec*>(bR + ((uint32_t)lr * ld32 + col32)), vec_make<EPL>(gmu[r]));
       if (RPI > 1 && NCELL > 0 && lr < n_rows) cell_reduce_store(cacc, row_begin + lr);
