@@ -11,7 +11,7 @@ BRIE_MAX_MODELS = 32
 ABI_VERSION = 9
 TARGETS = {"ELBO": 0, "marginLik": 1}
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("BRIE_LIB_PATH", os.path.join(_HERE, "libbrie_b200.so"))
+LIB_PATH = os.path.join(_HERE, "libbrie_b200.so")
 
 
 class FitDesc(C.Structure):
@@ -110,8 +110,7 @@ def leading_dim(n_events):
     ld 2 560: 0.958; profiles/r2_ab_rpi_tma.md) -- the full-size C3 (ld 10 016) paid the same.  Padding columns are
     inactive: their lanes copy nothing, so the padding costs memory (at most 127 columns), not traffic."""
     n = int(n_events)
-    align = int(os.environ.get("BRIE_LD_ALIGN", "128"))        # measurement aid (multiple of 32)
-    return (n + align - 1) // align * align if n > 96 else (n + 31) // 32 * 32
+    return (n + 127) // 128 * 128 if n > 96 else (n + 31) // 32 * 32
 
 
 _lib = None

@@ -36,22 +36,19 @@ def build(force=False, verbose=False):
     if not force and up_to_date():
         return OUT
     nvcc = os.environ.get("NVCC", "nvcc")
-    extra = os.environ.get("BRIE_NVCC_EXTRA", "").split()
-    out = os.environ.get("BRIE_LIB_OUT", OUT)
     os.makedirs(OBJ_DIR, exist_ok=True)
-    tag = "" if not extra else "_x"        # objects built with extra flags never shadow the normal ones
 
     def compile_unit(u):
         src = os.path.join(_CSRC, u)
-        obj = os.path.join(OBJ_DIR, u.replace(".cu", tag + ".o"))
-        if force or extra or _stale(obj, [src] + HEADERS):
-            cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+        obj = os.path.join(OBJ_DIR, u.replace(".cu", ".o"))
+        if force or _stale(obj, [src] + HEADERS):
+            cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
             subprocess.run(cmd, check=True)
         return obj
 
     with ThreadPoolExecutor(len(UNITS)) as ex:
         objs = list(ex.map(compile_unit, UNITS))
-    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", out] + objs + ["-ldl", "-lcublas"], check=True)
+    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", OUT] + objs + ["-ldl", "-lcublas"], check=True)
     return OUT
 
 

@@ -25,16 +25,13 @@
 
 #include "brie_philox.h"
 
-#ifndef BRIE_MIN_CTAS
-#define BRIE_MIN_CTAS 2  // resident CTAs per SM the step kernel is register-budgeted for
-#endif
-
 namespace brie {
 
 constexpr int kTileCols = 128;  // events per warp row segment
 constexpr int kWarps = 8;
 constexpr int kThreads = kWarps * 32;
 constexpr int kMaxModels = 32;
+constexpr int kMinCtas = 2;  // resident CTAs per SM the step kernel is register-budgeted for
 
 constexpr float kB1c = 0.1f;     // 1 - beta_1 (keras Adam)
 constexpr float kB2c = 0.001f;   // 1 - beta_2
@@ -130,38 +127,6 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
-// ---- TMA-bulk form of the row ring (measurement variant, -DBRIE_RING_TMA=1; default: LDGSTS) ---------------------
-// One elected lane per warp issues one cp.async.bulk (global -> shared, completion on an mbarrier) per array and
-// row -- a TC * 4-byte contiguous segment -- instead of every lane issuing one 16-byte cp.async per array.
-// A/B on hardware: profiles/r2_ab_tma_ring.md.  The variant covers the dense column walk only (no active-block
-// list): a compacted tile is 16 separate 32-byte blocks per array, below the bulk copy's 16-byte granule economy.
-#ifndef BRIE_RING_TMA
-#define BRIE_RING_TMA 0
-#endif
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "BRIE_MBAR_WAIT:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra BRIE_MBAR_DONE;\n\t"
-      "bra BRIE_MBAR_WAIT;\n\t"
-      "BRIE_MBAR_DONE:\n\t}" ::"r"(bar),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 // keras Adam update_step (TF 2.15): m += (g-m)(1-b1); v += (g^2-v)(1-b2);
 // x -= alpha_t * m / (sqrt(v) + eps)
 __device__ __forceinline__ void adam_update(float& x, float& m, float& v, float g, float alpha) {
@@ -171,12 +136,9 @@ __device__ __forceinline__ void adam_update(float& x, float& m, float& v, float 
 }
 
 // Packed FP32 pairs (sm_100a FFMA2 / FADD2 / FMUL2: one issue slot, two IEEE-rounded results) in the dense phases
-// and the Monte-Carlo samples of the step kernel.  A/B on one B200 against the scalar build (-DBRIE_F32X2=0),
-// profiles/r2_ab_f32x2.md: C2 unchanged (0.936), C3 with loss trace 0.930 -> 0.949, C4 0.947 -> 0.958 / with loss
-// trace 0.900 -> 0.923, Kc 16 0.730 -> 0.761 / 0.700 -> 0.742; the whole parity suite passes on either build.
-#ifndef BRIE_F32X2
-#define BRIE_F32X2 1
-#endif
+// and the Monte-Carlo samples of the step kernel.  A/B on one B200 against the scalar form, profiles/r2_ab_f32x2.md:
+// C2 unchanged (0.936), C3 with loss trace 0.930 -> 0.949, C4 0.947 -> 0.958 / with loss trace 0.900 -> 0.923,
+// Kc 16 0.730 -> 0.761 / 0.700 -> 0.742; the whole parity suite passed on either form.
 #define BRIE_F2_BINARY(name, ptx)                                                                          \
   __device__ __forceinline__ float2 name(float2 a, float2 b) {                                             \
     float2 d;                                                                                              \
@@ -239,7 +201,6 @@ __device__ __forceinline__ void mc_samples(float mu, float s, float c1, float c2
   for (int s0 = 0; s0 < S; s0 += 4) {
     float eps[4];
     brie_normals4(event, cell, step, stream0 + (uint32_t)(s0 >> 2), seed, eps);
-#if BRIE_F32X2
     // two samples per instruction where both exist (S = 3: samples 0 and 1 as a pair, sample 2 alone)
 #pragma unroll
     for (int j = 0; j < 4; j += 2) {
@@ -271,14 +232,9 @@ __device__ __forceinline__ void mc_samples(float mu, float s, float c1, float c2
         }
       }
     }
-#endif
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-#if BRIE_F32X2
       if (s0 + j < S && !(s0 + (j | 1) < S)) {   // the unpaired last sample
-#else
-      if (s0 + j < S) {
-#endif
         const float z = fmaf(s, eps[j], mu);
         const float e = ex2_approx(-kLog2e * fabsf(z));      // exp(-|z|)
         const float inv = rcp_approx(1.0f + e);
@@ -378,28 +334,18 @@ __host__ __device__ constexpr int step_tile_cols(int KC, int KG = 0) { return 32
 // S likelihood samples: ~200 instructions whatever the number of items) ran mostly idle; the items of two rows
 // share one pass.  Ring stages, queue and per-lane state then match the 4-events-per-lane kernels byte for byte.
 // (16 covariates together with gene features keep one row per iteration: two rows' state next to 32 per-event and
-// up to 10 per-cell accumulators would spill.)
-#ifndef BRIE_FORCE_RPI1
-#define BRIE_FORCE_RPI1 0   // A/B aid (scripts/ab.sh): 1 = one row per iteration everywhere
-#endif
+// up to 10 per-cell accumulators would spill.)  A/B against one row per iteration: profiles/r2_ab_rpi_tma.md.
 __host__ __device__ constexpr int step_rpi(int KC, int KG = 0) {
-  return (!BRIE_FORCE_RPI1 && step_epl(KC, KG) == 2 && !(KC > 8 && KG > 0)) ? 2 : 1;
+  return (step_epl(KC, KG) == 2 && !(KC > 8 && KG > 0)) ? 2 : 1;
 }
 // Per-event constants of a column tile (Wc rows, Xg columns, intercept, sigma_log, 1/sigma^2) stay in
 // registers for narrow designs; wider ones (Kc + Kg >= 3) keep them in shared memory and re-read them
 // every row, so they are not live across the Monte-Carlo phase (no spills).  A/B on one box
 // (profiles/r1_ab_smem_consts.md, r1_ab_row_consts.md): C3 with loss trace +11 %, C4 +10 % / +23 %,
 // Kc 15 +9 %; C3 without the loss trace runs 1 % slower from shared memory but spills from registers.
-#ifndef BRIE_SMEM_CONSTS_MODE
-#define BRIE_SMEM_CONSTS_MODE 0   // A/B aid (scripts/ab.sh): 1 = registers for Kc <= 4 without Kg / loss trace, 2 = never
-#endif
-__host__ __device__ constexpr bool step_consts_in_smem(int KC, int KG, bool LOSS) {
-  if (BRIE_SMEM_CONSTS_MODE == 1) return KC + KG >= 3 && !(KG == 0 && KC <= 4 && !LOSS);
-  if (BRIE_SMEM_CONSTS_MODE == 2) return false;
-  return KC + KG >= 3;
-}
-__host__ __device__ constexpr int step_n_consts(int KC, int KG, bool CELL, bool LOSS) {
-  return step_consts_in_smem(KC, KG, LOSS) ? KC + KG + (CELL ? 0 : 3) : 0;
+__host__ __device__ constexpr bool step_consts_in_smem(int KC, int KG) { return KC + KG >= 3; }
+__host__ __device__ constexpr int step_n_consts(int KC, int KG, bool CELL) {
+  return step_consts_in_smem(KC, KG) ? KC + KG + (CELL ? 0 : 3) : 0;
 }
 constexpr int kRowConstSlots = 32;   // per warp and ring stage: Xc[c, :], Wg[c, :], per-cell intercept / sigma_log of the row
 // CODE8: per warp and row of an iteration, the Monte-Carlo sums d/dZ_loc, d/dZ_std_log and (LOSS) the log-likelihood
@@ -409,13 +355,13 @@ __host__ __device__ constexpr int step_smem_bytes(int KC, int KG, bool CELL, boo
   return ((kWarps * kRingStages * ((CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0)) +
            kWarps * kQueueFields + (CODE8 ? kWarps * step_n_scratch(LOSS) : 0)) *
               step_rpi(KC, KG) +
-          7 + step_n_consts(KC, KG, CELL, LOSS)) *
+          7 + step_n_consts(KC, KG, CELL)) *
              step_tile_cols(KC, KG) * 4 +
          kWarps * kRingStages * step_rpi(KC, KG) * kRowConstSlots * 4 + (CODE8 ? 3 * kDictSize * 4 : 0);
 }
 
 template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false, bool CODE8 = false>
-__global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(const StepArgs a) {
+__global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const StepArgs a) {
   static_assert(!EXT || (KC == 0 && KG == 0), "the wide-design form takes all covariates through PM / R");
   // ring arrays per row slot (EXT: + the prior-mean tile) and the slots of the Adam moments / prior-mean tile in it
   constexpr int NRA = (CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0);
@@ -428,7 +374,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
   constexpr int NCELL = T::NCELL;
   constexpr int EPL = step_epl(KC, KG);
   constexpr int TC = 32 * EPL;              // events per warp row segment (column tile)
-  constexpr bool kSm = step_consts_in_smem(KC, KG, LOSS);
+  constexpr bool kSm = step_consts_in_smem(KC, KG);
   using Vec = typename LaneVec<EPL>::type;
   const int m = blockIdx.x;
   if (!((a.model_mask >> m) & 1u)) return;
@@ -480,7 +426,7 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
   constexpr int NRC = KC + KG + (CELL ? 2 : 0);   // per-row (cell) constants: Xc[c, :], Wg[c, :], b[c], tau[c]
   static_assert(NRC <= kRowConstSlots, "row constants must fit one slot per lane");
   constexpr int kRcBase = ((kWarps * kRingStages * NRA + kWarps * kQueueFields) * RPI + 7 +
-                           step_n_consts(KC, KG, CELL, LOSS)) * TC;
+                           step_n_consts(KC, KG, CELL)) * TC;
   float* s_rc = smem + kRcBase + warp * (kRingStages * RPI * kRowConstSlots);
   // CODE8: this warp's Monte-Carlo sums (row r, sum k at (r * NSCR + k) * TC) and the count dictionary
   constexpr int kScrBase = kRcBase + kWarps * kRingStages * RPI * kRowConstSlots;
@@ -556,56 +502,10 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
   // zero-filled, they compute on zeros and store nothing, so a partly active tile only pays for the
   // 32-byte sectors that hold active events.
   const uint32_t rc_lane = (uint32_t)__cvta_generic_to_shared(s_rc) + lane * 4;
-#if BRIE_RING_TMA
-  __shared__ __align__(8) uint64_t s_bar[kWarps][kRingStages];
-  const uint32_t bar0 = (uint32_t)__cvta_generic_to_shared(&s_bar[warp][0]);
-  // bytes of this tile's row segment inside ld (the last tile of a row may be partial; ld % 32 == 0)
-  const uint32_t seg_bytes = (uint32_t)min((int64_t)TC, a.ld - (int64_t)tile * TC) * 4u;
-  if (a.blk_ids != nullptr) __trap();             // measurement variant: dense column walk only
-  if (lane == 0) {
-    mbar_init(bar0, 1);
-    mbar_init(bar0 + 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (seg_bytes < (uint32_t)TC * 4u || (!CODE8 && !has_c3)) {   // slots no bulk copy ever fills must read as zero counts / state
-    for (int i = lane; i < kRingStages * RPI * SLOT; i += 32) s_ring[i] = 0.f;
-  }
-  __syncwarp();
-  uint32_t ring_phase = 0;                        // bit s: parity the next wait on stage s expects
-  const uint32_t ring_base = (uint32_t)__cvta_generic_to_shared(s_ring);
-#endif
   auto issue_rows = [&](int lrb, int stage) {     // lrb: first of the RPI adjacent rows (index within the CTA)
-#if BRIE_RING_TMA
-    if (lrb < n_rows && lane == 0) {
-      fence_proxy_async();                        // the warp's generic reads / writes of this stage (two iterations ago) come first
-      const uint32_t bar = bar0 + stage * 8;
-      const int nr = min(RPI, n_rows - lrb);
-      const uint32_t n_cnt = CODE8 ? 1u : (has_c3 ? 3u : 2u);
-      mbar_expect_tx(bar, seg_bytes * (6u + n_cnt + (EXT ? 1u : 0u)) * (uint32_t)nr);
-      for (int r = 0; r < nr; ++r) {
-        const uint32_t relw = (uint32_t)(lrb + r) * ld32 + (uint32_t)tile * TC;
-        const uint32_t dstw = ring_base + (stage * RPI + r) * (SLOT * 4);
-        bulk_g2s(dstw + 0 * TC * 4, bZl + relw, seg_bytes, bar);
-        bulk_g2s(dstw + 1 * TC * 4, bZs + relw, seg_bytes, bar);
-        if (CODE8) {
-          bulk_g2s(dstw + 2 * TC * 4, bW + relw, seg_bytes, bar);
-        } else {
-          bulk_g2s(dstw + 2 * TC * 4, bC0 + relw, seg_bytes, bar);
-          bulk_g2s(dstw + 3 * TC * 4, bC1 + relw, seg_bytes, bar);
-          if (has_c3) bulk_g2s(dstw + 4 * TC * 4, bC2 + relw, seg_bytes, bar);
-        }
-        bulk_g2s(dstw + (IA + 0) * TC * 4, bA0 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + (IA + 1) * TC * 4, bA1 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + (IA + 2) * TC * 4, bA2 + relw, seg_bytes, bar);
-        bulk_g2s(dstw + (IA + 3) * TC * 4, bA3 + relw, seg_bytes, bar);
-        if (EXT) bulk_g2s(dstw + IPM * TC * 4, bPM + relw, seg_bytes, bar);
-      }
-    }
-#endif
 #pragma unroll
     for (int r = 0; r < RPI; ++r) {
       const int lr = lrb + r;
-#if !BRIE_RING_TMA
       const bool ok = act != 0 && lr < n_rows;
       const uint32_t rel = ok ? (uint32_t)lr * ld32 + col32 : 0u;
       const uint32_t dst = ring_lane + (stage * RPI + r) * (SLOT * 4);
@@ -623,7 +523,6 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       cp_async_lane<EPL * 4>(dst + (IA + 2) * TC * 4, bA2 + rel, ok);
       cp_async_lane<EPL * 4>(dst + (IA + 3) * TC * 4, bA3 + rel, ok);
       if (EXT) cp_async_lane<EPL * 4>(dst + IPM * TC * 4, bPM + rel, ok);
-#endif
       if (NRC > 0) {
         // The row's warp-uniform constants ride in the same commit group, one float per lane.  (As plain
         // loads issued a row ahead they shared a scoreboard with the tile constants loaded before the loop,
@@ -713,15 +612,8 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
 
   int stage = 0;
   for (int lrb = warp * RPI; lrb < n_rows; lrb += kWarps * RPI, stage ^= 1) {
-#if BRIE_RING_TMA
-    __syncwarp();                         // every lane is done with the other stage (phase B / C of the previous iteration)
-#endif
     issue_rows(lrb + kWarps * RPI, stage ^ 1);   // prefetch the next rows (zero-size copies past the end)
     cp_async_wait<1>();                   // this iteration's group has landed
-#if BRIE_RING_TMA
-    mbar_wait(bar0 + stage * 8, (ring_phase >> stage) & 1u);
-    ring_phase ^= 1u << stage;
-#endif
     __syncwarp();                         // other lanes read this lane's copies (row constants, Monte-Carlo items)
     float* const rs0 = s_ring + stage * (RPI * SLOT);                 // row slot r of this stage: rs0 + r * SLOT
     float mu[RPI][EPL], lam[RPI][EPL], gmu[RPI][EPL], glam[RPI][EPL];
@@ -782,7 +674,6 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
           vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[KC + KG + 2][lane * EPL]), is2);
         }
       }
-#if BRIE_F32X2
       static_assert(EPL % 2 == 0, "packed pairs need an even number of events per lane");
       float2 cacc2[NCELL > 0 ? NCELL : 1];
 #pragma unroll
@@ -842,43 +733,6 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
       }
 #pragma unroll
       for (int i = 0; i < NCELL; ++i) cacc[i] = cacc2[i].x + cacc2[i].y;
-#else
-#pragma unroll
-      for (int j = 0; j < EPL; ++j) {
-        const float tj = CELL ? tau_row : tau[j];
-        const float i2 = CELL ? is2_row : is2[j];
-        float pm = CELL ? b_row : bb[j];
-        if (EXT) pm += pmx[j];
-#pragma unroll
-        for (int k = 0; k < KC; ++k) pm = fmaf(xc[k], wc[k][j], pm);
-#pragma unroll
-        for (int k = 0; k < KG; ++k) pm = fmaf(wg[k], xg[k][j], pm);
-        const float d = lam[r][j] - tj;
-        const float e2 = ex2_approx((2.0f * kLog2e) * d);  // s^2 / sigma^2
-        const float diff = mu[r][j] - pm;
-        const float rr = diff * i2;                        // (mu - m) / sigma^2
-        const float q2 = diff * rr;                        // ((mu - m) / sigma)^2
-        gmu[r][j] = rr;
-        glam[r][j] = e2 - 1.0f;
-        if (has_reads(j)) nz |= 1u << (r * EPL + j);
-        const float gt = 1.0f - q2 - e2;                   // d loss / d sigma_log
-#pragma unroll
-        for (int k = 0; k < KC; ++k) acc[k][j] = fmaf(-xc[k], rr, acc[k][j]);
-        if (!CELL) {
-          acc[T::kGB][j] -= real_row ? rr : 0.f;
-          acc[T::kGT][j] += real_row ? gt : 0.f;
-        }
-        if (LOSS) acc[T::kLoss][j] += real_row ? 0.5f * q2 + 0.5f * (e2 - 1.0f) - d : 0.f;  // TFP _kl_normal_normal
-        if (NCELL > 0 && (g0 + j) < a.Ng) {
-#pragma unroll
-          for (int k = 0; k < KG; ++k) cacc[k] = fmaf(-xg[k][j], rr, cacc[k]);
-          if (CELL) {
-            cacc[KG] -= rr;
-            cacc[KG + 1] += gt;
-          }
-        }
-      }
-#endif
       static_assert(!EXT || RPI == 1, "the wide-design store below writes every row of an iteration");
       if (EXT && act != 0)   // r = (mu - m) / sigma^2 of this row, for the gradient GEMMs (frozen lanes keep their old values: unused)
         __stcs(reinterpret_cast<Vec*>(bR + ((uint32_t)lr * ld32 + col32)), vec_make<EPL>(gmu[r]));
@@ -889,16 +743,12 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
     // ---- phase B: compacted Monte-Carlo work (the items of all RPI rows share the passes) ----
     uint32_t bal[RPI * EPL];
     int base = 0;
-#ifdef BRIE_SKELETON   // measurement aid (scripts/ab.sh): memory skeleton only, no Monte-Carlo work
-    const int n_items = 0;
-#else
     int n_items = 0;
 #pragma unroll
     for (int j = 0; j < RPI * EPL; ++j) {
       bal[j] = __ballot_sync(0xffffffffu, nz & (1u << j));
       n_items += __popc(bal[j]);
     }
-#endif
     if (n_items > 0) {
 #pragma unroll
       for (int j = 0; j < RPI * EPL; ++j) base += __popc(bal[j] & lt_mask);
@@ -980,7 +830,6 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
         vec_get<EPL>(st[(IA + 2) * 32], m2);
         vec_get<EPL>(st[(IA + 3) * 32], v2);
         if (all_act) {
-#if BRIE_F32X2
 #pragma unroll
           for (int p = 0; p < EPL / 2; ++p) {
             const int j0 = 2 * p, j1 = 2 * p + 1;
@@ -989,14 +838,6 @@ __global__ void __launch_bounds__(kThreads, BRIE_MIN_CTAS) elbo_step_kernel(cons
             mu[r][j0] = clip9(mu[r][j0]);  // Variable constraint (model_TFProb.py:80-81)
             mu[r][j1] = clip9(mu[r][j1]);
           }
-#else
-#pragma unroll
-          for (int j = 0; j < EPL; ++j) {
-            adam_update(mu[r][j], m1[j], v1[j], gmu[r][j], a.alpha);
-            adam_update(lam[r][j], m2[j], v2[j], glam[r][j], a.alpha);
-            mu[r][j] = clip9(mu[r][j]);  // Variable constraint (model_TFProb.py:80-81)
-          }
-#endif
         } else {
 #pragma unroll
           for (int j = 0; j < EPL; ++j) {

@@ -306,10 +306,9 @@ class FitEngine:
             _lib.check(self.lib.brie_fit_set_count_codes(h, self.count_codes[0].data_ptr(), 0,
                                                          self.count_codes[1].data_ptr()))
         # Shared per-cell parameters on an event shard: the library all-reduces their gradients itself,
-        # in stream order inside brie_fit_run_steps (BRIE_HOST_ALLREDUCE=1 keeps the older per-step
-        # torch.distributed round trip, for A/B only).
+        # in stream order inside brie_fit_run_steps.
         self._comm = None
-        if dist_group is not None and self.shared and not os.environ.get("BRIE_HOST_ALLREDUCE"):
+        if dist_group is not None and self.shared:
             from . import comm
             self._comm = comm.get(dist_group)
             _lib.check(self.lib.brie_fit_set_comm(h, self._comm.h))
@@ -386,19 +385,7 @@ class FitEngine:
 
     def run_steps(self, n, trace_slot0=-1):
         with torch.cuda.device(self.device):
-            if self.dist_group is None or not self.shared or self._comm is not None:
-                _lib.check(self.lib.brie_fit_run_steps(self.h, int(n), int(trace_slot0), self._stream()))
-                return
-            import torch.distributed as dist
-            p, nf = C.c_void_p(), C.c_int64()
-            _lib.check(self.lib.brie_fit_cell_grad(self.h, C.byref(p), C.byref(nf)))
-            off = (p.value - self.scratch.data_ptr()) // 4
-            G = self.scratch[off:off + nf.value]
-            for i in range(n):
-                slot = trace_slot0 + i if trace_slot0 >= 0 else -1
-                _lib.check(self.lib.brie_fit_step_phase(self.h, 0, slot, self._stream()))
-                dist.all_reduce(G, group=self.dist_group)   # NCCL: shared-weight gradients only
-                _lib.check(self.lib.brie_fit_step_phase(self.h, 1, slot, self._stream()))
+            _lib.check(self.lib.brie_fit_run_steps(self.h, int(n), int(trace_slot0), self._stream()))
 
     def group_trace(self, n_slots):
         """(M, n_groups, n_slots) float64 sums of the per-event loss trace per reference batch."""
@@ -461,7 +448,7 @@ class FitEngine:
         e.g. 100 events at 5k cells, where the per-model count tiles of the gathered form (12 B per
         model instead of 12 B shared) outweigh the few half-empty blocks: the caller then steps in
         place.  `force` skips that cost comparison (tests)."""
-        if self.shared or self.wide or self.target != "ELBO" or os.environ.get("BRIE_NO_GATHER"):
+        if self.shared or self.wide or self.target != "ELBO":
             return False
         M, Nc, L = self.M, self.Nc, self.n_layers
         g = (np.arange(self.Ng) + self.event_offset) // self.group_size - self.first_group
