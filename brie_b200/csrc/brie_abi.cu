@@ -44,8 +44,10 @@ struct brie_fit {
   brie_fit_sizes sz;
   brie_fit_buffers buf;
   bool bound = false;
+  bool subfit = false;       // bound as a gathered sub-fit (event_ids or a per-model count / length stride)
   int nev_max = 0, ncell = 0;
   size_t off_part_ev = 0, off_part_cell = 0, off_G = 0;  // scratch carve-up (float offsets)
+  size_t off_mom_cell = 0;   // adam_small: per-event moments (2, M, Kc + 2, ld) first, per-cell (2, M, Nc, Kg + 2) here
   bool stage_open = false;   // begin_stage has set the learning rate and cleared the Adam moments
   float lr = 0.f;
   int64_t t = 0;             // Adam step within the current stage
@@ -81,33 +83,33 @@ constexpr int kMaxDevices = 64;
 bool kc_supported(int k) { return k == 0 || k == 1 || k == 2 || k == 4 || k == 8 || k == 16; }
 bool kg_supported(int k) { return k == 0 || k == 4 || k == 8; }
 
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool CODE8>
-cudaError_t launch_step(const StepArgs& a, dim3 grid, cudaStream_t s) {
-  // per instantiation and per device: opt in to > 48 KB dynamic shared memory (the attribute is per device)
+// Opt Kernel in to `bytes` of dynamic shared memory (needed above 48 KB) once per device: the attribute is per device.
+template <auto* Kernel>
+cudaError_t opt_in_smem(int bytes) {
   static bool configured[kMaxDevices] = {false};
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
-  if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
-    e = cudaFuncSetAttribute(elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8));
-    if (e != cudaSuccess) return e;
-    if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
-  }
-  elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8><<<grid, kThreads, step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8), s>>>(a);
+  const bool known = dev >= 0 && dev < kMaxDevices;
+  if (known && configured[dev]) return cudaSuccess;
+  e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e == cudaSuccess && known) configured[dev] = true;
+  return e;
+}
+
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool CODE8>
+cudaError_t launch_step(const StepArgs& a, dim3 grid, cudaStream_t s) {
+  constexpr int smem = step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8);
+  cudaError_t e = opt_in_smem<elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8>>(smem);
+  if (e != cudaSuccess) return e;
+  elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8><<<grid, kThreads, smem, s>>>(a);
   return cudaGetLastError();
 }
 
 // the count form (f32 tiles or packed codes) is the innermost choice
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false>
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT>
 cudaError_t launch_step_fmt(const StepArgs& a, dim3 grid, cudaStream_t s) {
   return a.codes ? launch_step<KC, KG, CELL, LOSS, EXT, true>(a, grid, s) : launch_step<KC, KG, CELL, LOSS, EXT, false>(a, grid, s);
-}
-
-cudaError_t dispatch_step_wide(const StepArgs& a, bool cell, bool loss, dim3 grid, cudaStream_t s) {
-  if (cell)
-    return loss ? launch_step_fmt<0, 0, true, true, true>(a, grid, s) : launch_step_fmt<0, 0, true, false, true>(a, grid, s);
-  return loss ? launch_step_fmt<0, 0, false, true, true>(a, grid, s) : launch_step_fmt<0, 0, false, false, true>(a, grid, s);
 }
 
 const char* blas_status(cublasStatus_t st) {
@@ -177,11 +179,12 @@ int wide_gradients(brie_fit* f, cudaStream_t s) {
   return BRIE_OK;
 }
 
-template <int KC, int KG>
+// EXT: the wide form, whose kernels contract no covariates themselves (KC = KG = 0)
+template <int KC, int KG, bool EXT = false>
 cudaError_t dispatch_step2(const StepArgs& a, bool cell, bool loss, dim3 grid, cudaStream_t s) {
   if (cell)
-    return loss ? launch_step_fmt<KC, KG, true, true>(a, grid, s) : launch_step_fmt<KC, KG, true, false>(a, grid, s);
-  return loss ? launch_step_fmt<KC, KG, false, true>(a, grid, s) : launch_step_fmt<KC, KG, false, false>(a, grid, s);
+    return loss ? launch_step_fmt<KC, KG, true, true, EXT>(a, grid, s) : launch_step_fmt<KC, KG, true, false, EXT>(a, grid, s);
+  return loss ? launch_step_fmt<KC, KG, false, true, EXT>(a, grid, s) : launch_step_fmt<KC, KG, false, false, EXT>(a, grid, s);
 }
 
 template <int KC>
@@ -194,8 +197,9 @@ cudaError_t dispatch_step1(const StepArgs& a, int KG, bool cell, bool loss, dim3
   return cudaErrorInvalidValue;
 }
 
-cudaError_t dispatch_step(const StepArgs& a, int KC, int KG, bool cell, bool loss, dim3 grid,
+cudaError_t dispatch_step(const StepArgs& a, bool wide, int KC, int KG, bool cell, bool loss, dim3 grid,
                           cudaStream_t s) {
+  if (wide) return dispatch_step2<0, 0, true>(a, cell, loss, grid, s);
   switch (KC) {
     case 0: return dispatch_step1<0>(a, KG, cell, loss, grid, s);
     case 1: return dispatch_step1<1>(a, KG, cell, loss, grid, s);
@@ -212,6 +216,138 @@ cudaError_t dispatch_step(const StepArgs& a, int KC, int KG, bool cell, bool los
 // the kernels consult `active` per event and this mask stays all-ones.
 uint32_t g_all_models(const brie_fit* f) {
   return f->d.n_models >= 32 ? 0xffffffffu : ((1u << f->d.n_models) - 1u);
+}
+
+// The fields that StepArgs, MarginArgs, EvalArgs and TermsArgs share under the same names; the rest are zero.
+template <class A>
+A fit_args(const brie_fit* f) {
+  const brie_fit_desc& d = f->d;
+  const brie_fit_buffers& b = f->buf;
+  A a;
+  memset(&a, 0, sizeof a);
+  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.event_offset = d.event_offset; a.seed = d.seed;
+  a.c[0] = b.counts[0]; a.c[1] = b.counts[1]; a.c[2] = b.counts[2];
+  a.eff = b.efflen3; a.Xc = b.Xc; a.Xg = b.Xg;
+  a.Wc = b.Wc; a.b = b.intercept; a.tau = b.sigma_log; a.Wg = b.Wg;
+  a.M = d.n_models;
+  return a;
+}
+
+// Arguments of both per-cell kernels; n_tiles: the column tiles of per-cell partials that cell_reduce_kernel sums.
+CellArgs cell_args(const brie_fit* f, int n_tiles) {
+  const brie_fit_desc& d = f->d;
+  float* scratch = (float*)f->buf.scratch;
+  CellArgs c;
+  memset(&c, 0, sizeof c);
+  c.Nc = d.n_cells; c.M = d.n_models; c.KG = d.Kg; c.NCELL = f->ncell; c.n_tiles = n_tiles;
+  c.cell_mode = d.cell_mode; c.train_b = d.train_intercept; c.train_tau = d.train_sigma;
+  c.model_mask = g_all_models(f); c.alpha = f->alpha;
+  c.part_cell = scratch + f->off_part_cell; c.G = scratch + f->off_G;
+  c.Wg = f->buf.Wg; c.b = f->buf.intercept; c.tau = f->buf.sigma_log;
+  c.mom = f->buf.adam_small + f->off_mom_cell;
+  c.n_part = f->wide ? (d.cell_mode ? 2 : 0) : f->ncell;   // wide: d/dWg is already in G (wide_gradients)
+  c.part_off = f->wide ? d.Kg : 0;
+  return c;
+}
+
+// The launchers of one step, in stream order (brie_fit_step_phase).  Each launches only if its kernel has work.
+// target marginLik: the prior-sampled objective reads counts only, no per-element state (brie_margin.cuh)
+int launch_margin_step(brie_fit* f, int nev, int cell_tiles, cudaStream_t s) {
+  const brie_fit_desc& d = f->d;
+  float* scratch = (float*)f->buf.scratch;
+  MarginArgs g = fit_args<MarginArgs>(f);
+  g.active = f->buf.active;
+  g.part_ev = scratch + f->off_part_ev; g.part_cell = scratch + f->off_part_cell;
+  g.step = f->global_step; g.model_mask = g_all_models(f);
+  g.S = d.mc_size; g.rows_per_cta = f->sz.rows_per_cta;
+  g.KC = d.Kc; g.KG = d.Kg; g.cell_mode = d.cell_mode; g.NEV = nev; g.NCELL = f->ncell;
+  for (int m = 0; m < d.n_models; ++m) g.model_id[m] = d.model_id[m];
+  // the opt-in covers the widest per-event partials (Kc = BRIE_MAX_KC); the launch asks for this fit's
+  BRIE_CUDA(opt_in_smem<margin_step_kernel>(kWarps * (BRIE_MAX_KC + 3) * kMarginTile * (int)sizeof(float)));
+  const size_t smem = (size_t)kWarps * nev * kMarginTile * sizeof(float);
+  margin_step_kernel<<<dim3(d.n_models, cell_tiles, f->sz.n_row_chunks), kThreads, smem, s>>>(g);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 1;
+  return BRIE_OK;
+}
+
+// target ELBO: the fused step kernel, between the wide form's prior-mean and gradient GEMMs.  The timing events
+// (brie_fit_kernel_timing) bracket the fused kernel alone.
+int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s) {
+  const brie_fit_desc& d = f->d;
+  float* scratch = (float*)f->buf.scratch;
+  StepArgs a = fit_args<StepArgs>(f);
+  a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log; a.aZ = f->buf.adam_Z;
+  a.active = f->buf.active;
+  a.part_ev = scratch + f->off_part_ev; a.part_cell = scratch + f->off_part_cell;
+  a.alpha = f->alpha; a.inv_S = 1.0f / (float)d.mc_size;
+  a.step = f->global_step; a.model_mask = g_all_models(f);
+  a.S = d.mc_size; a.rows_per_cta = f->sz.rows_per_cta;
+  for (int m = 0; m < d.n_models; ++m) a.model_id[m] = d.model_id[m];
+  a.ev_ids = f->buf.event_ids; a.c_mstride = f->buf.counts_model_stride; a.eff_mstride = f->buf.efflen_model_stride;
+  a.codes = f->codes; a.code_mstride = f->code_mstride; a.dict = f->code_dict;
+  dim3 grid(d.n_models, f->sz.n_col_tiles, f->sz.n_row_chunks);
+  if (f->blk_ids) {
+    a.blk_ids = f->blk_ids; a.blk_stride = f->blk_stride;
+    for (int m = 0; m < d.n_models; ++m) a.n_blk[m] = f->n_blk[m];
+    grid.y = (unsigned)(f->blk_tiles > 0 ? f->blk_tiles : 1);
+  }
+  if (f->wide) {
+    a.PM = scratch + f->off_PM; a.R = scratch + f->off_R;
+    int rc = wide_prior_mean(f, s);
+    if (rc) return rc;
+  }
+  const bool timed = f->ev_used < (int)f->ev0.size();
+  if (timed) BRIE_CUDA(cudaEventRecord(f->ev0[f->ev_used], s));
+  BRIE_CUDA(dispatch_step(a, f->wide, d.Kc, d.Kg, d.cell_mode != 0, loss, grid, s));
+  if (timed) BRIE_CUDA(cudaEventRecord(f->ev1[f->ev_used++], s));
+  f->launches += 1;
+  return f->wide ? wide_gradients(f, s) : BRIE_OK;
+}
+
+// Per-event reduce of the row-chunk partials (nev rows, the loss last if loss_row), Adam on Wc and the per-event
+// intercept / sigma_log, and the loss trace if trace_slot >= 0.  The wide form's d/dWc comes from wide_gradients.
+int launch_event_update(brie_fit* f, int nev, bool loss_row, int32_t trace_slot, cudaStream_t s) {
+  const brie_fit_desc& d = f->d;
+  if (nev == 0 && !(f->wide && d.Kc > 0)) return BRIE_OK;
+  float* scratch = (float*)f->buf.scratch;
+  const int kc_kernel = f->wide ? 0 : d.Kc;
+  EventArgs e;
+  memset(&e, 0, sizeof e);
+  e.ld = d.ld; e.Ng = d.n_events; e.M = d.n_models; e.KC = d.Kc; e.NEV = nev; e.n_chunks = f->sz.n_row_chunks;
+  e.idx_gb = d.cell_mode ? -1 : kc_kernel; e.idx_gt = d.cell_mode ? -1 : kc_kernel + 1;
+  e.idx_loss = loss_row ? kc_kernel + (d.cell_mode ? 0 : 2) : -1;
+  e.wc_grad = f->wide ? scratch + f->off_gWc : nullptr;
+  e.train_b = d.train_intercept; e.train_tau = d.train_sigma;
+  e.trace_slot = trace_slot; e.trace_cap = d.trace_cap;
+  e.alpha = f->alpha; e.part_ev = scratch + f->off_part_ev;
+  e.Wc = f->buf.Wc; e.b = f->buf.intercept; e.tau = f->buf.sigma_log;
+  e.mom = f->buf.adam_small; e.active = f->buf.active; e.trace = f->buf.loss_trace;
+  for (int m = 0; m < d.n_models; ++m) { e.xc_mask[m] = d.xc_mask[m]; e.xc_width[m] = d.xc_width[m]; }
+  event_update_kernel<<<dim3((unsigned)ceil_div(d.n_events, 32), d.n_models), 256, 0, s>>>(e);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 1;
+  return BRIE_OK;
+}
+
+// Per-cell sum of the column-tile partials into G, which the all-reduce and launch_cell_update read.
+int launch_cell_reduce(brie_fit* f, int cell_tiles, cudaStream_t s) {
+  const CellArgs c = cell_args(f, cell_tiles);
+  if (c.n_part == 0) return BRIE_OK;
+  cell_reduce_kernel<<<dim3((unsigned)ceil_div(f->d.n_cells * c.n_part, 256), f->d.n_models), 256, 0, s>>>(c);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 1;
+  return BRIE_OK;
+}
+
+// Adam on Wg and the per-cell intercept / sigma_log from G.
+int launch_cell_update(brie_fit* f, cudaStream_t s) {
+  if (f->ncell == 0) return BRIE_OK;
+  cell_update_kernel<<<dim3((unsigned)ceil_div(f->d.n_cells, 256), f->d.n_models), 256, 0, s>>>(
+      cell_args(f, f->sz.n_col_tiles));
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 1;
+  return BRIE_OK;
 }
 
 }  // namespace
@@ -306,8 +442,8 @@ int brie_fit_create(const brie_fit_desc* desc, brie_fit** out) {
     off += (size_t)d.n_models * (d.Kc > 0 ? d.Kc : 1) * d.ld;
   }
   f->sz.scratch_bytes = (off + 4) * sizeof(float);
-  f->sz.adam_small_floats =
-      (size_t)2 * d.n_models * (d.Kc + 2) * d.ld + (size_t)2 * d.n_models * d.n_cells * (d.Kg + 2);
+  f->off_mom_cell = (size_t)2 * d.n_models * (d.Kc + 2) * d.ld;
+  f->sz.adam_small_floats = f->off_mom_cell + (size_t)2 * d.n_models * d.n_cells * (d.Kg + 2);
   *out = f;
   return BRIE_OK;
 }
@@ -360,8 +496,9 @@ int brie_fit_get_sizes(const brie_fit* fit, brie_fit_sizes* out) {
 int brie_fit_bind(brie_fit* fit, const brie_fit_buffers* b) {
   if (!fit || !b) return fail(BRIE_ERR_ARG, "null argument");
   const brie_fit_desc& d = fit->d;
+  const bool subfit = b->event_ids || b->counts_model_stride != 0 || b->efflen_model_stride != 0;
   // a gathered sub-fit may step on packed codes alone (brie_fit_set_count_codes) and bind no count tiles
-  const bool no_counts = b->event_ids && !b->counts[0] && !b->counts[1] && !b->counts[2];
+  const bool no_counts = subfit && !b->counts[0] && !b->counts[1] && !b->counts[2];
   if (!no_counts && (!b->counts[0] || !b->counts[1])) return fail(BRIE_ERR_ARG, "counts[0], counts[1] required");
   if (!no_counts && (d.n_layers == 3) != (b->counts[2] != nullptr))
     return fail(BRIE_ERR_ARG, "counts[2] must be given iff n_layers == 3");
@@ -377,15 +514,15 @@ int brie_fit_bind(brie_fit* fit, const brie_fit_buffers* b) {
                            b->adam_Z,    b->Wc,        b->intercept, b->sigma_log, b->active, b->scratch};
   for (const void* p : aligned)
     if (((uintptr_t)p & 15u) != 0) return fail(BRIE_ERR_ARG, "device buffers must be 16-byte aligned");
-  if (b->event_ids || b->counts_model_stride != 0 || b->efflen_model_stride != 0) {
+  if (subfit) {
     if (fit->ncell > 0 || d.target != BRIE_TARGET_ELBO)
       return fail(BRIE_ERR_UNSUPPORTED, "a gathered sub-fit needs per-event parameters only (Kg = 0, gene intercept) and target ELBO");
     if (b->counts_model_stride < 0 || b->counts_model_stride % 4 != 0 || b->efflen_model_stride < 0)
       return fail(BRIE_ERR_ARG, "model strides must be >= 0 (counts: a multiple of 4 floats)");
+    if (fit->wide) return fail(BRIE_ERR_UNSUPPORTED, "gathered sub-fits are limited to Kc <= %d", BRIE_MAX_KC);
   }
-  if (fit->wide && (b->event_ids || b->counts_model_stride || b->efflen_model_stride))
-    return fail(BRIE_ERR_UNSUPPORTED, "gathered sub-fits are limited to Kc <= %d", BRIE_MAX_KC);
   fit->buf = *b;
+  fit->subfit = subfit;
   fit->bound = true;
   if (fit->wide) {   // residuals of never-active (padding) columns must be finite for the gradient GEMMs
     float* scratch = (float*)b->scratch;
@@ -493,164 +630,33 @@ int brie_fit_step_phase(brie_fit* f, int32_t phase, int32_t trace_slot, void* st
   if (!f || !f->bound) return fail(BRIE_ERR_ARG, "fit not bound");
   cudaStream_t s = (cudaStream_t)stream;
   const brie_fit_desc& d = f->d;
-  float* scratch = (float*)f->buf.scratch;
   const bool loss = trace_slot >= 0;
   if (loss && trace_slot >= d.trace_cap) return fail(BRIE_ERR_ARG, "trace_slot %d >= trace_cap %d", trace_slot, d.trace_cap);
-  const int M = d.n_models;
-  const uint32_t mmask = g_all_models(f);
   if (phase == 0) {
+    const bool margin = d.target == BRIE_TARGET_MARGINLIK;
     if (f->step_open) return fail(BRIE_ERR_ARG, "phase 0 called twice");
     if (!f->stage_open) return fail(BRIE_ERR_ARG, "brie_fit_begin_stage must be called before the first step");
+    if (!f->codes && !f->buf.counts[0]) return fail(BRIE_ERR_ARG, "neither count tiles nor count codes bound");
+    // checked: a refused call leaves the Adam step as it was
     f->t += 1;
     const double t = (double)f->t;
     f->alpha = (float)((double)f->lr * sqrt(1.0 - pow(0.999, t)) / (1.0 - pow(0.9, t)));
-    const bool margin = d.target == BRIE_TARGET_MARGINLIK;
-    const int kc_kernel = f->wide ? 0 : d.Kc;     // covariates the fused kernel contracts itself
-    int nev = kc_kernel + (d.cell_mode ? 0 : 2) + (loss ? 1 : 0);
-    int cell_tiles = f->sz.n_col_tiles;
-    if (margin && f->buf.event_ids) return fail(BRIE_ERR_UNSUPPORTED, "marginLik on a gathered sub-fit");
-    if (margin) {
-      // prior-sampled objective: counts only, no per-element state (brie_margin.cuh)
-      nev = d.Kc + (d.cell_mode ? 0 : 2) + 1;
-      cell_tiles = (int)ceil_div(d.ld, kMarginTile);
-      MarginArgs g;
-      memset(&g, 0, sizeof g);
-      g.Nc = d.n_cells; g.Ng = d.n_events; g.ld = d.ld; g.event_offset = d.event_offset; g.seed = d.seed;
-      g.c[0] = f->buf.counts[0]; g.c[1] = f->buf.counts[1]; g.c[2] = f->buf.counts[2];
-      g.eff = f->buf.efflen3; g.Xc = f->buf.Xc; g.Xg = f->buf.Xg;
-      g.Wc = f->buf.Wc; g.b = f->buf.intercept; g.tau = f->buf.sigma_log; g.Wg = f->buf.Wg;
-      g.active = f->buf.active;
-      g.part_ev = scratch + f->off_part_ev;
-      g.part_cell = scratch + f->off_part_cell;
-      g.step = f->global_step; g.model_mask = mmask;
-      g.M = M; g.S = d.mc_size; g.rows_per_cta = f->sz.rows_per_cta;
-      g.KC = d.Kc; g.KG = d.Kg; g.cell_mode = d.cell_mode; g.NEV = nev; g.NCELL = f->ncell;
-      for (int m = 0; m < M; ++m) g.model_id[m] = d.model_id[m];
-      const size_t smem = (size_t)kWarps * nev * kMarginTile * sizeof(float);
-      static bool configured[kMaxDevices] = {false};   // per device, as in launch_step
-      int dev = 0;
-      BRIE_CUDA(cudaGetDevice(&dev));
-      if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
-        BRIE_CUDA(cudaFuncSetAttribute(margin_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       kWarps * (BRIE_MAX_KC + 3) * kMarginTile * (int)sizeof(float)));
-        if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
-      }
-      const dim3 grid(M, cell_tiles, f->sz.n_row_chunks);
-      margin_step_kernel<<<grid, kThreads, smem, s>>>(g);
-      BRIE_CUDA(cudaGetLastError());
-      f->launches += 1;
-    } else {
-    if (!f->codes && !f->buf.counts[0]) return fail(BRIE_ERR_ARG, "neither count tiles nor count codes bound");
-    StepArgs a;
-    memset(&a, 0, sizeof a);
-    a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.event_offset = d.event_offset; a.seed = d.seed;
-    a.c[0] = f->buf.counts[0]; a.c[1] = f->buf.counts[1]; a.c[2] = f->buf.counts[2];
-    a.eff = f->buf.efflen3; a.Xc = f->buf.Xc; a.Xg = f->buf.Xg;
-    a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log; a.aZ = f->buf.adam_Z;
-    a.Wc = f->buf.Wc; a.b = f->buf.intercept; a.tau = f->buf.sigma_log; a.Wg = f->buf.Wg;
-    a.active = f->buf.active;
-    a.part_ev = scratch + f->off_part_ev;
-    a.part_cell = scratch + f->off_part_cell;
-    a.alpha = f->alpha;
-    a.inv_S = 1.0f / (float)d.mc_size;
-    a.step = f->global_step;
-    a.model_mask = mmask;
-    a.M = M; a.S = d.mc_size; a.rows_per_cta = f->sz.rows_per_cta;
-    for (int m = 0; m < M; ++m) a.model_id[m] = d.model_id[m];
-    a.ev_ids = f->buf.event_ids;
-    a.c_mstride = f->buf.counts_model_stride;
-    a.eff_mstride = f->buf.efflen_model_stride;
-    a.codes = f->codes;
-    a.code_mstride = f->code_mstride;
-    a.dict = f->code_dict;
-    dim3 grid(M, f->sz.n_col_tiles, f->sz.n_row_chunks);
-    if (f->blk_ids) {
-      a.blk_ids = f->blk_ids;
-      a.blk_stride = f->blk_stride;
-      for (int m = 0; m < M; ++m) a.n_blk[m] = f->n_blk[m];
-      grid.y = (unsigned)(f->blk_tiles > 0 ? f->blk_tiles : 1);
-    }
-    if (f->wide) {
-      a.PM = scratch + f->off_PM;
-      a.R = scratch + f->off_R;
-      int rc = wide_prior_mean(f, s);
-      if (rc) return rc;
-    }
-    const bool timed = f->ev_used < (int)f->ev0.size();
-    if (timed) BRIE_CUDA(cudaEventRecord(f->ev0[f->ev_used], s));
-    if (f->wide)
-      BRIE_CUDA(dispatch_step_wide(a, d.cell_mode != 0, loss, grid, s));
-    else
-      BRIE_CUDA(dispatch_step(a, d.Kc, d.Kg, d.cell_mode != 0, loss, grid, s));
-    if (timed) BRIE_CUDA(cudaEventRecord(f->ev1[f->ev_used++], s));
-    f->launches += 1;
-    if (f->wide) {
-      int rc = wide_gradients(f, s);
-      if (rc) return rc;
-    }
-    }
-
-    if (nev > 0 || (f->wide && d.Kc > 0)) {
-      EventArgs e;
-      memset(&e, 0, sizeof e);
-      e.ld = d.ld; e.Ng = d.n_events; e.M = M; e.KC = d.Kc; e.NEV = nev; e.n_chunks = f->sz.n_row_chunks;
-      e.idx_gb = d.cell_mode ? -1 : kc_kernel;
-      e.idx_gt = d.cell_mode ? -1 : kc_kernel + 1;
-      e.idx_loss = (loss || margin) ? kc_kernel + (d.cell_mode ? 0 : 2) : -1;   // trace written only if trace_slot >= 0
-      if (f->wide) {
-        e.wc_grad = scratch + f->off_gWc;
-        for (int m = 0; m < M; ++m) e.xc_width[m] = d.xc_width[m];
-      }
-      e.train_b = d.train_intercept; e.train_tau = d.train_sigma;
-      e.trace_slot = trace_slot; e.trace_cap = d.trace_cap;
-      e.alpha = f->alpha;
-      e.part_ev = scratch + f->off_part_ev;
-      e.Wc = f->buf.Wc; e.b = f->buf.intercept; e.tau = f->buf.sigma_log;
-      e.mom = f->buf.adam_small;
-      e.active = f->buf.active;
-      e.trace = f->buf.loss_trace;
-      for (int m = 0; m < M; ++m) e.xc_mask[m] = d.xc_mask[m];
-      const dim3 g2((unsigned)ceil_div(d.n_events, 32), M);
-      event_update_kernel<<<g2, 256, 0, s>>>(e);
-      BRIE_CUDA(cudaGetLastError());
-      f->launches += 1;
-    }
-    if (f->ncell > 0) {
-      CellArgs c;
-      memset(&c, 0, sizeof c);
-      c.Nc = d.n_cells; c.M = M; c.KG = d.Kg; c.NCELL = f->ncell; c.n_tiles = cell_tiles;
-      c.model_mask = mmask;
-      c.part_cell = scratch + f->off_part_cell;
-      c.G = scratch + f->off_G;
-      c.n_part = f->wide ? (d.cell_mode ? 2 : 0) : f->ncell;   // wide: d/dWg is already in G (wide_gradients)
-      c.part_off = f->wide ? d.Kg : 0;
-      if (c.n_part > 0) {
-        const dim3 g3((unsigned)ceil_div(d.n_cells * c.n_part, 256), M);
-        cell_reduce_kernel<<<g3, 256, 0, s>>>(c);
-        BRIE_CUDA(cudaGetLastError());
-        f->launches += 1;
-      }
-    }
+    // per-event partials: the covariates the step kernel contracts itself, intercept and sigma (gene mode), then the
+    // loss, which the marginLik kernel always sums; marginLik tiles its columns its own way
+    const bool loss_row = loss || margin;
+    const int nev = (f->wide ? 0 : d.Kc) + (d.cell_mode ? 0 : 2) + (loss_row ? 1 : 0);
+    const int cell_tiles = margin ? (int)ceil_div(d.ld, kMarginTile) : f->sz.n_col_tiles;
+    int rc = margin ? launch_margin_step(f, nev, cell_tiles, s) : launch_fused_step(f, loss, s);
+    if (!rc) rc = launch_event_update(f, nev, loss_row, trace_slot, s);
+    if (!rc) rc = launch_cell_reduce(f, cell_tiles, s);
+    if (rc) return rc;
     f->step_open = true;
     return BRIE_OK;
   }
   if (phase == 1) {
     if (!f->step_open) return fail(BRIE_ERR_ARG, "phase 1 without phase 0");
-    if (f->ncell > 0) {
-      CellArgs c;
-      memset(&c, 0, sizeof c);
-      c.Nc = d.n_cells; c.M = M; c.KG = d.Kg; c.NCELL = f->ncell; c.n_tiles = f->sz.n_col_tiles;
-      c.cell_mode = d.cell_mode; c.train_b = d.train_intercept; c.train_tau = d.train_sigma;
-      c.model_mask = mmask;
-      c.alpha = f->alpha;
-      c.G = scratch + f->off_G;
-      c.Wg = f->buf.Wg; c.b = f->buf.intercept; c.tau = f->buf.sigma_log;
-      c.mom = f->buf.adam_small + (size_t)2 * M * (d.Kc + 2) * d.ld;
-      const dim3 g4((unsigned)ceil_div(d.n_cells, 256), M);
-      cell_update_kernel<<<g4, 256, 0, s>>>(c);
-      BRIE_CUDA(cudaGetLastError());
-      f->launches += 1;
-    }
+    int rc = launch_cell_update(f, s);
+    if (rc) return rc;
     f->global_step += 1;
     f->step_open = false;
     return BRIE_OK;
@@ -739,21 +745,15 @@ int brie_fit_cell_grad(brie_fit* f, float** ptr, int64_t* n_floats) {
 int brie_fit_eval_loss_gene(brie_fit* f, int32_t n_eval, int32_t mc_size, float* loss_gene, void* stream) {
   if (!f || !f->bound || !loss_gene) return fail(BRIE_ERR_ARG, "null argument or fit not bound");
   if (n_eval < 1) return fail(BRIE_ERR_ARG, "n_eval must be >= 1");
-  if (f->buf.event_ids || f->buf.counts_model_stride || f->buf.efflen_model_stride)
-    return fail(BRIE_ERR_UNSUPPORTED, "loss_gene is evaluated on the parent fit, not on a gathered sub-fit");
+  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "loss_gene is evaluated on the parent fit, not on a gathered sub-fit");
   if (mc_size < 1 || mc_size > 4096) return fail(BRIE_ERR_ARG, "mc_size out of range");
   cudaStream_t s = (cudaStream_t)stream;
   const brie_fit_desc& d = f->d;
   float* scratch = (float*)f->buf.scratch;
-  EvalArgs a;
-  memset(&a, 0, sizeof a);
-  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.event_offset = d.event_offset; a.seed = d.seed;
-  a.c[0] = f->buf.counts[0]; a.c[1] = f->buf.counts[1]; a.c[2] = f->buf.counts[2];
-  a.eff = f->buf.efflen3; a.Xc = f->buf.Xc; a.Xg = f->buf.Xg;
+  EvalArgs a = fit_args<EvalArgs>(f);
   a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log;
-  a.Wc = f->buf.Wc; a.b = f->buf.intercept; a.tau = f->buf.sigma_log; a.Wg = f->buf.Wg;
   a.part_ev = scratch + f->off_part_ev;
-  a.M = d.n_models; a.S = mc_size; a.n_eval = n_eval; a.rows_per_cta = f->sz.rows_per_cta;
+  a.S = mc_size; a.n_eval = n_eval; a.rows_per_cta = f->sz.rows_per_cta;
   a.KC = d.Kc; a.KG = d.Kg; a.cell_mode = d.cell_mode;
   a.margin = d.target == BRIE_TARGET_MARGINLIK;
   for (int m = 0; m < d.n_models; ++m) a.model_id[m] = d.model_id[m];
@@ -785,17 +785,13 @@ int brie_fit_element_terms(brie_fit* f, int32_t model, const float* c1, const fl
   if (model < 0 || model >= f->d.n_models) return fail(BRIE_ERR_ARG, "model index out of range");
   if (loglik && (!c1 || !c2)) return fail(BRIE_ERR_ARG, "count tiles required for loglik");
   if (loglik && (mc_size < 1 || mc_size > 4096)) return fail(BRIE_ERR_ARG, "mc_size out of range");
-  if (f->buf.event_ids) return fail(BRIE_ERR_UNSUPPORTED, "element terms are evaluated on the parent fit");
+  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "element terms are evaluated on the parent fit");
   const brie_fit_desc& d = f->d;
-  TermsArgs a;
-  memset(&a, 0, sizeof a);
-  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.event_offset = d.event_offset; a.seed = d.seed;
-  a.c[0] = c1; a.c[1] = c2; a.c[2] = c3;
-  a.eff = f->buf.efflen3; a.Xc = f->buf.Xc; a.Xg = f->buf.Xg;
+  TermsArgs a = fit_args<TermsArgs>(f);
+  a.c[0] = c1; a.c[1] = c2; a.c[2] = c3;   // the caller's count tiles, not the fitted ones
   a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log;
-  a.Wc = f->buf.Wc; a.b = f->buf.intercept; a.tau = f->buf.sigma_log; a.Wg = f->buf.Wg;
   a.loglik = loglik; a.kl = kl; a.prior_mean = prior_mean;
-  a.M = d.n_models; a.m = model; a.S = mc_size; a.KC = d.Kc; a.KG = d.Kg; a.cell_mode = d.cell_mode;
+  a.m = model; a.S = mc_size; a.KC = d.Kc; a.KG = d.Kg; a.cell_mode = d.cell_mode;
   a.margin = margin != 0; a.model_id = d.model_id[model]; a.noise_step = noise_step;
   element_terms_kernel<<<grid_1d(d.n_cells * d.ld, 256), 256, 0, (cudaStream_t)stream>>>(a);
   BRIE_CUDA(cudaGetLastError());
@@ -820,8 +816,7 @@ int wald_plan(const brie_fit* f, int32_t model, WaldPlan* w) {
   if (model < 0 || model >= d.n_models) return fail(BRIE_ERR_ARG, "model index out of range");
   if (d.target != BRIE_TARGET_ELBO)
     return fail(BRIE_ERR_UNSUPPORTED, "Wald information needs a trained posterior (target ELBO)");
-  if (f->buf.event_ids || f->buf.counts_model_stride || f->buf.efflen_model_stride)
-    return fail(BRIE_ERR_UNSUPPORTED, "Wald information is computed on the parent fit, not on a gathered sub-fit");
+  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "Wald information is computed on the parent fit, not on a gathered sub-fit");
   w->width = f->wide ? d.xc_width[model] : __builtin_popcount(d.xc_mask[model]);
   w->has_b = (!d.cell_mode && d.train_intercept) ? 1 : 0;
   w->kt = w->width + w->has_b;
@@ -913,7 +908,7 @@ int brie_fit_group_trace(brie_fit* f, int32_t n_slots, int64_t group_size, int64
   const brie_fit_desc& d = f->d;
   if (n_slots < 1 || n_slots > d.trace_cap) return fail(BRIE_ERR_ARG, "n_slots out of range");
   if (group_size < 1 || n_groups < 1) return fail(BRIE_ERR_ARG, "bad group geometry");
-  if (f->buf.event_ids) return fail(BRIE_ERR_UNSUPPORTED, "scatter the trace of a gathered sub-fit back to its parent first");
+  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "scatter the trace of a gathered sub-fit back to its parent first");
   const int64_t first_group = d.event_offset / group_size;
   const dim3 grid(n_slots, d.n_models);
   group_trace_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(f->buf.loss_trace, d.trace_cap, d.ld, d.n_events,

@@ -644,6 +644,12 @@ class FitEngine:
         return out
 
 
+def _event_moments(adam_small, M, Kc, ld):
+    """The per-event Adam moments (2, M, Kc + 2, ld) at the front of a fit's adam_small (brie_fit_create); the per-cell
+    moments follow them."""
+    return adam_small[:2 * M * (Kc + 2) * ld].view(2, M, Kc + 2, ld)
+
+
 class _GatheredFit:
     """Sub-fit over gathered columns of a parent FitEngine (brie_fit_buffers.event_ids): model m's
     column j is the parent's local event cols[m][j].  Holds its own dense tiles of the state, the
@@ -689,9 +695,8 @@ class _GatheredFit:
         self.Wc = torch.zeros((M, max(Kc, 1), ld), dtype=f32, device=dev)
         self.intercept = torch.empty((M, ld), dtype=f32, device=dev)
         self.sigma_log = torch.empty((M, ld), dtype=f32, device=dev)
-        n_mom = 2 * M * (Kc + 2) * ld                       # per-event moments come first (brie_abi.cu)
-        self.adam_small = torch.zeros(max(int(sz.adam_small_floats), n_mom, 4), dtype=f32, device=dev)
-        self.mom = self.adam_small[:n_mom].view(2, M, Kc + 2, ld)
+        self.adam_small = torch.zeros(max(int(sz.adam_small_floats), 4), dtype=f32, device=dev)
+        self.mom = _event_moments(self.adam_small, M, Kc, ld)
         self.eff = torch.empty((M, 3, ld), dtype=f32, device=dev) if p.eff is not None else None
         self.loss_trace = torch.zeros((M, trace_cap, ld), dtype=f32, device=dev)
         self.scratch = torch.empty(int(sz.scratch_bytes // 4) + 4, dtype=f32, device=dev)
@@ -731,7 +736,7 @@ class _GatheredFit:
     def _pairs(self, m, inputs, trace_rows):
         """(parent view, sub view) of model m, each rows x columns with the columns to move."""
         p, Kc = self.p, self.p.Kc
-        pmom = p.adam_small[:2 * p.M * (Kc + 2) * p.ld].view(2, p.M, Kc + 2, p.ld)
+        pmom = _event_moments(p.adam_small, p.M, Kc, p.ld)
         out = [(p.Z_loc[m], self.Z_loc[m]), (p.Z_std_log[m], self.Z_std_log[m])]
         out += [(p.adam_Z[k, m], self.adam_Z[k, m]) for k in range(4)]
         if Kc > 0:

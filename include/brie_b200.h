@@ -153,15 +153,6 @@ int brie_fit_get_step(const brie_fit* fit, int64_t* adam_t, uint32_t* global_ste
  * loss_trace[:, trace_slot0 + i, :]; if < 0 the loss is not evaluated. */
 int brie_fit_run_steps(brie_fit* fit, int32_t n_steps, int32_t trace_slot0, void* stream);
 
-/* Column compaction for the convergence-extension rounds (model_TFProb.py:250-258).  The
- * reference extends each event batch on its own (model_wrap.py:241-260); batches that have
- * converged stay frozen through `active`.  Once most are frozen the step kernel can visit only
- * the 8-event column blocks (one 32-byte sector of every f32 array) that still hold an active
- * event: blk_ids (DEVICE, (n_models, blk_stride) int32, ascending block indices col / 8) lists
- * them per model, n_blk_host (HOST, n_models) their counts.  Results are bit-identical to the
- * uncompacted step.  blk_ids = NULL restores the dense walk.  The list must cover every event
- * with active = 1 and must stay valid until replaced.  Needs ld % 8 == 0, Kg = 0, cell_mode = 0,
- * target ELBO. */
 /* Packed count codes for the fused step kernel (brie_encode_counts).  From now on the step kernel reads one 32-bit
  * code word per element from `codes` ((Nc, ld) per model, codes_model_stride words apart, 0 = one tile shared by all
  * models, as counts_model_stride) and decodes the counts of elements with reads from dict (DEVICE, (3, 256) floats),
@@ -171,11 +162,20 @@ int brie_fit_run_steps(brie_fit* fit, int32_t n_steps, int32_t trace_slot0, void
  * float32 tiles.  Both arrays must stay valid while set. */
 int brie_fit_set_count_codes(brie_fit* fit, const uint32_t* codes, int64_t codes_model_stride, const float* dict);
 
+/* Column compaction for the convergence-extension rounds (model_TFProb.py:250-258).  The
+ * reference extends each event batch on its own (model_wrap.py:241-260); batches that have
+ * converged stay frozen through `active`.  Once most are frozen the step kernel can visit only
+ * the 8-event column blocks (one 32-byte sector of every f32 array) that still hold an active
+ * event: blk_ids (DEVICE, (n_models, blk_stride) int32, ascending block indices col / 8) lists
+ * them per model, n_blk_host (HOST, n_models) their counts.  Results are bit-identical to the
+ * uncompacted step.  blk_ids = NULL restores the dense walk.  The list must cover every event
+ * with active = 1 and must stay valid until replaced.  Needs ld % 8 == 0, Kg = 0, cell_mode = 0,
+ * target ELBO. */
 int brie_fit_set_active_blocks(brie_fit* fit, const int32_t* blk_ids, int64_t blk_stride,
                                const int32_t* n_blk_host);
 
 /* All-reduce hook for event-sharded fits with shared per-cell parameters
- * (Kg > 0 or cell_mode).  brie_fit_run_steps_split runs ONE step in two halves:
+ * (Kg > 0 or cell_mode).  brie_fit_step_phase runs ONE step in two halves:
  * phase 0 leaves the summed per-cell gradients in cell_grad (M, Nc, n_cell_acc)
  * (pointer returned by brie_fit_cell_grad) for the caller to all-reduce; phase 1
  * applies Adam to Wg / per-cell intercept / sigma_log. */

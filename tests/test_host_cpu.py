@@ -84,6 +84,61 @@ def test_create_validates_arguments(lib):
     lib.brie_fit_destroy(h)
 
 
+def _bind_fake(lib, counts, **buffers):
+    """A narrow fit (Kc = 1, no lengths) bound to fake 16-byte-aligned addresses: brie_fit_bind reads no memory of
+    such a fit, so the argument checks run without a device.  None of these addresses may reach a launch."""
+    from brie_b200 import _lib
+    h = C.c_void_p()
+    assert lib.brie_fit_create(C.byref(_desc(has_efflen=0)), C.byref(h)) == 0
+    b = _lib.FitBuffers()
+    fake = iter(range(0x10000, 0x1000000, 0x1000))
+    for name in ("Xc", "Z_loc", "Z_std_log", "adam_Z", "Wc", "intercept", "sigma_log", "adam_small", "active",
+                 "loss_trace", "scratch"):
+        setattr(b, name, next(fake))
+    for i in range(3 if counts else 0):
+        b.counts[i] = next(fake)
+    for name, v in buffers.items():
+        setattr(b, name, next(fake) if v is True else v)
+    assert lib.brie_fit_bind(h, C.byref(b)) == 0, lib.brie_last_error()
+    return h, b
+
+
+def test_refused_step_leaves_the_adam_step_alone(lib):
+    """A step that phase 0 refuses (here: a sub-fit with neither count tiles nor count codes) changes no state."""
+    h, _ = _bind_fake(lib, counts=False, event_ids=True)
+    assert lib.brie_fit_resume_stage(h, 0.01, 0, 0) == 0
+    assert lib.brie_fit_run_steps(h, 1, -1, None) == -1
+    assert b"neither count tiles nor count codes" in lib.brie_last_error()
+    t, step = C.c_int64(-1), C.c_uint32(7)
+    assert lib.brie_fit_get_step(h, C.byref(t), C.byref(step)) == 0
+    assert (t.value, step.value) == (0, 0)
+    assert lib.brie_fit_launch_count(h) == 0
+    lib.brie_fit_destroy(h)
+
+
+def test_subfit_is_refused_by_every_entry_but_the_step(lib):
+    """A per-model count stride alone makes a sub-fit (brie_fit_buffers): loss_gene, element terms, Wald and the group
+    trace work on the parent fit only and refuse it before any launch."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("a refusal missed here would launch on fake addresses")
+    h, b = _bind_fake(lib, counts=True, counts_model_stride=100 * 64)
+    out = 0x2000000
+    nbytes, kt = C.c_size_t(), C.c_int32()
+    calls = {
+        "eval_loss_gene": lambda: lib.brie_fit_eval_loss_gene(h, 1, 1, out, None),
+        "element_terms": lambda: lib.brie_fit_element_terms(h, 0, b.counts[0], b.counts[1], b.counts[2], 1, 0, 0,
+                                                            out, None, None, None),
+        "wald_sizes": lambda: lib.brie_fit_wald_sizes(h, 0, C.byref(nbytes), C.byref(kt)),
+        "group_trace": lambda: lib.brie_fit_group_trace(h, 1, 1, 1, out, None),
+    }
+    for name, call in calls.items():
+        assert call() == -3, name
+        assert b"parent" in lib.brie_last_error(), name
+    assert lib.brie_fit_launch_count(h) == 0
+    lib.brie_fit_destroy(h)
+
+
 def test_host_normals_match_numpy_spec(lib):
     from brie_b200 import _lib
     S, R, Cn, off = 5, 7, 19, 4000
