@@ -178,6 +178,13 @@ __device__ __forceinline__ void adam_update2(float& x0, float& x1, float& m0, fl
 
 __device__ __forceinline__ float clip9(float x) { return fminf(fmaxf(x, -9.0f), 9.0f); }
 
+// adam_update of one stored parameter *x with its moments *m, *v; `clip` applies the +-9 constraint to the result.
+__device__ __forceinline__ void adam_at(float* x, float* m, float* v, float g, float alpha, bool clip = false) {
+  float xx = *x, mm = *m, vv = *v;
+  adam_update(xx, mm, vv, g, alpha);
+  *x = clip ? clip9(xx) : xx; *m = mm; *v = vv;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -926,31 +933,17 @@ __global__ void __launch_bounds__(256) event_update_kernel(const EventArgs a) {
     return s;
   };
   const int64_t mstride = (int64_t)a.M * (a.KC + 2) * a.ld;
+  auto adam_slot = [&](float* x, int slot, float grad, bool clip) {
+    const int64_t qi = ((int64_t)m * (a.KC + 2) + slot) * a.ld + g;
+    adam_at(x, a.mom + qi, a.mom + mstride + qi, grad, a.alpha, clip);
+  };
   for (int k = 0; k < a.KC; ++k) {
     if (a.wc_grad ? k >= a.xc_width[m] : !((a.xc_mask[m] >> k) & 1u)) continue;
     const float grad = a.wc_grad ? a.wc_grad[((int64_t)m * a.KC + k) * a.ld + g] : (float)red(k);
-    const int64_t pi = ((int64_t)m * a.KC + k) * a.ld + g;
-    const int64_t qi = ((int64_t)m * (a.KC + 2) + k) * a.ld + g;
-    float x = a.Wc[pi], mm = a.mom[qi], vv = a.mom[mstride + qi];
-    adam_update(x, mm, vv, grad, a.alpha);
-    a.Wc[pi] = x; a.mom[qi] = mm; a.mom[mstride + qi] = vv;
+    adam_slot(a.Wc + ((int64_t)m * a.KC + k) * a.ld + g, k, grad, false);
   }
-  if (a.idx_gb >= 0 && a.train_b) {
-    const float grad = (float)red(a.idx_gb);
-    const int64_t pi = (int64_t)m * a.ld + g;
-    const int64_t qi = ((int64_t)m * (a.KC + 2) + a.KC) * a.ld + g;
-    float x = a.b[pi], mm = a.mom[qi], vv = a.mom[mstride + qi];
-    adam_update(x, mm, vv, grad, a.alpha);
-    a.b[pi] = clip9(x); a.mom[qi] = mm; a.mom[mstride + qi] = vv;
-  }
-  if (a.idx_gt >= 0 && a.train_tau) {
-    const float grad = (float)red(a.idx_gt);
-    const int64_t pi = (int64_t)m * a.ld + g;
-    const int64_t qi = ((int64_t)m * (a.KC + 2) + a.KC + 1) * a.ld + g;
-    float x = a.tau[pi], mm = a.mom[qi], vv = a.mom[mstride + qi];
-    adam_update(x, mm, vv, grad, a.alpha);
-    a.tau[pi] = x; a.mom[qi] = mm; a.mom[mstride + qi] = vv;
-  }
+  if (a.idx_gb >= 0 && a.train_b) adam_slot(a.b + (int64_t)m * a.ld + g, a.KC, (float)red(a.idx_gb), true);
+  if (a.idx_gt >= 0 && a.train_tau) adam_slot(a.tau + (int64_t)m * a.ld + g, a.KC + 1, (float)red(a.idx_gt), false);
   if (a.idx_loss >= 0 && a.trace_slot >= 0)
     a.trace[((int64_t)m * a.trace_cap + a.trace_slot) * a.ld + g] = (float)red(a.idx_loss);
 }
@@ -989,24 +982,77 @@ __global__ void __launch_bounds__(256) cell_update_kernel(const CellArgs a) {
   const float* G = a.G + ((int64_t)m * a.Nc + c) * a.NCELL;
   const int64_t mstride = (int64_t)a.M * a.Nc * (a.KG + 2);
   float* mom = a.mom + ((int64_t)m * a.Nc + c) * (a.KG + 2);
-  for (int k = 0; k < a.KG; ++k) {
-    float x = a.Wg[((int64_t)m * a.Nc + c) * a.KG + k], mm = mom[k], vv = mom[mstride + k];
-    adam_update(x, mm, vv, G[k], a.alpha);
-    a.Wg[((int64_t)m * a.Nc + c) * a.KG + k] = x; mom[k] = mm; mom[mstride + k] = vv;
-  }
+  for (int k = 0; k < a.KG; ++k)
+    adam_at(a.Wg + ((int64_t)m * a.Nc + c) * a.KG + k, mom + k, mom + mstride + k, G[k], a.alpha);
   if (a.cell_mode) {
-    if (a.train_b) {
-      float x = a.b[(int64_t)m * a.Nc + c], mm = mom[a.KG], vv = mom[mstride + a.KG];
-      adam_update(x, mm, vv, G[a.KG], a.alpha);
-      a.b[(int64_t)m * a.Nc + c] = clip9(x); mom[a.KG] = mm; mom[mstride + a.KG] = vv;
-    }
-    if (a.train_tau) {
-      float x = a.tau[(int64_t)m * a.Nc + c], mm = mom[a.KG + 1], vv = mom[mstride + a.KG + 1];
-      adam_update(x, mm, vv, G[a.KG + 1], a.alpha);
-      a.tau[(int64_t)m * a.Nc + c] = x; mom[a.KG + 1] = mm; mom[mstride + a.KG + 1] = vv;
-    }
+    if (a.train_b)
+      adam_at(a.b + (int64_t)m * a.Nc + c, mom + a.KG, mom + mstride + a.KG, G[a.KG], a.alpha, true);
+    if (a.train_tau)
+      adam_at(a.tau + (int64_t)m * a.Nc + c, mom + a.KG + 1, mom + mstride + a.KG + 1, G[a.KG + 1], a.alpha);
   }
 }
+
+// IEEE-accurate model terms of eval_loss_kernel, element_terms_kernel and margin_step_kernel (brie_margin.cuh).
+// The fused step kernel has its own fast-math forms (mc_samples).
+//
+// Effective lengths of event g: the (3, ld) effLen table, or (1, 1, 0) -- the binomial branch,
+// model_TFProb.py:162-167 -- without one.
+__device__ __forceinline__ void event_lengths(const float* eff, int64_t ld, int64_t g, float& L1, float& L2,
+                                              float& L3) {
+  L1 = 1.f; L2 = 1.f; L3 = 0.f;
+  if (eff) { L1 = eff[g]; L2 = eff[ld + g]; L3 = eff[2 * ld + g]; }
+}
+
+// The length constant c1 log L1 + c2 log L2 + c3 log L3 of the log-likelihood (0 without effLen).
+__device__ __forceinline__ float log_length_const(bool eff, float c1, float c2, float c3, float L1, float L2,
+                                                  float L3) {
+  return eff ? fmaf(c1, logf(L1), fmaf(c2, logf(L2), c3 * logf(L3))) : 0.f;
+}
+
+// Prior mean intercept + Xc Wc + Wg Xg^T of (row, event g) for model m (model_TFProb.py:118-126); `base` is the
+// intercept.  A is any argument struct with the fields Nc, ld, KC, KG, Xc, Wc, Wg, Xg.
+template <class A>
+__device__ __forceinline__ float prior_mean(const A& a, int m, int64_t row, int64_t g, float base) {
+  float pm = base;
+  for (int k = 0; k < a.KC; ++k)
+    pm = fmaf(a.Xc[((int64_t)m * a.Nc + row) * a.KC + k], a.Wc[((int64_t)m * a.KC + k) * a.ld + g], pm);
+  for (int k = 0; k < a.KG; ++k) pm = fmaf(a.Wg[((int64_t)m * a.Nc + row) * a.KG + k], a.Xg[g * a.KG + k], pm);
+  return pm;
+}
+
+// KL(N(mu, exp(lam)) || N(pm, exp(tau))) (model_TFProb.py:208).
+__device__ __forceinline__ float kl_normal(float mu, float lam, float pm, float tau) {
+  const float d = lam - tau;
+  const float r0 = (mu - pm) * expf(-tau);
+  return 0.5f * r0 * r0 + 0.5f * expm1f(2.0f * d) - d;
+}
+
+// Log-likelihood of one sample z (logLik_MC, model_TFProb.py:159-185) without the length constant:
+//   l = c1 log psi + c2 log(1-psi) - n log D,   D = psi L1 + (1-psi) L2 + L3   (no n log D without effLen).
+// psi, q = 1 - psi and D come back too, for dl/dz.
+struct SampleLL { float l, psi, q, D; };
+__device__ __forceinline__ SampleLL sample_ll(float z, float c1, float c2, float n, float L1, float L2, float L3,
+                                              bool eff) {
+  SampleLL r;
+  const float e = expf(-fabsf(z));
+  const float lsp = fminf(z, 0.f) - log1pf(e);
+  const float inv = 1.0f / (1.0f + e);
+  r.psi = z >= 0.f ? inv : e * inv;
+  r.q = z >= 0.f ? e * inv : inv;
+  r.D = fmaf(r.psi, L1, fmaf(r.q, L2, L3));
+  r.l = fmaf(c1, lsp, c2 * (lsp - z)) - (eff ? n * logf(r.D) : 0.f);
+  return r;
+}
+
+// Streaming log-mean-exp of sample log-likelihoods (tfp.math.reduce_logmeanexp, model_TFProb.py:188-189).
+struct LogMeanExp {
+  float mx = -INFINITY, Z = 0.f;
+  __device__ __forceinline__ void add(float l) {
+    if (l > mx) { Z *= expf(mx - l); mx = l; }
+    Z += expf(l - mx);
+  }
+  __device__ __forceinline__ float value(int S) const { return mx + logf(Z) - logf((float)S); }
+};
 
 // Forward-only per-event loss with n_eval x S fresh-noise samples per element
 // (the 500x get_loss(axis=0) loop of model_TFProb.py:261-264 in one pass).  Only
@@ -1037,31 +1083,20 @@ __device__ __forceinline__ float eval_item(float mu, float s, float c1, float c2
                                            uint32_t cell, uint32_t stream0, uint64_t seed, int lane) {
   float acc = 0.f;
   for (int it = lane; it < n_eval; it += 32) {
-    float mx = -INFINITY, Z = 0.f;
+    LogMeanExp lme;
     for (int s0 = 0; s0 < S; s0 += 4) {
       float eps[4];
       brie_normals4(event, cell, (uint32_t)it, stream0 + (uint32_t)(s0 >> 2), seed, eps);
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         if (s0 + q < S) {
-          const float z = fmaf(s, eps[q], mu);
-          const float e = expf(-fabsf(z));
-          const float lsp = fminf(z, 0.f) - log1pf(e);
-          const float inv = 1.0f / (1.0f + e);
-          const float psi = z >= 0.f ? inv : e * inv;
-          const float qq = z >= 0.f ? e * inv : inv;
-          const float D = fmaf(psi, L1, fmaf(qq, L2, L3));
-          const float l = fmaf(c1, lsp, c2 * (lsp - z)) - (eff ? n * logf(D) : 0.f);
-          if (!margin) {
-            acc += l;
-          } else {
-            if (l > mx) { Z *= expf(mx - l); mx = l; }
-            Z += expf(l - mx);
-          }
+          const float l = sample_ll(fmaf(s, eps[q], mu), c1, c2, n, L1, L2, L3, eff).l;
+          if (!margin) acc += l;
+          else lme.add(l);
         }
       }
     }
-    if (margin) acc += (float)S * (mx + logf(Z) - logf((float)S));
+    if (margin) acc += (float)S * lme.value(S);
   }
   return warp_sum(acc);
 }
@@ -1084,7 +1119,7 @@ __global__ void __launch_bounds__(kThreads) eval_loss_kernel(const EvalArgs a) {
     const int64_t gj = g0 + j;
     L1[j] = 1.f; L2[j] = 1.f; L3[j] = 0.f; bb[j] = 0.f; tau[j] = 0.f;
     if (gj < a.ld) {
-      if (eff) { L1[j] = a.eff[gj]; L2[j] = a.eff[a.ld + gj]; L3[j] = a.eff[2 * a.ld + gj]; }
+      event_lengths(a.eff, a.ld, gj, L1[j], L2[j], L3[j]);
       if (!a.cell_mode) { bb[j] = a.b[(int64_t)m * a.ld + gj]; tau[j] = a.tau[(int64_t)m * a.ld + gj]; }
     }
   }
@@ -1116,18 +1151,9 @@ __global__ void __launch_bounds__(kThreads) eval_loss_kernel(const EvalArgs a) {
       float zc = mu[j], zsl = lam[j];       // centre and log-scale the samples are drawn around
       if (valid) {
         const float tj = a.cell_mode ? tau_row : tau[j];
-        float pm = a.cell_mode ? b_row : bb[j];
-        for (int k = 0; k < a.KC; ++k)
-          pm = fmaf(a.Xc[((int64_t)m * a.Nc + row) * a.KC + k], a.Wc[((int64_t)m * a.KC + k) * a.ld + gj], pm);
-        for (int k = 0; k < a.KG; ++k)
-          pm = fmaf(a.Wg[((int64_t)m * a.Nc + row) * a.KG + k], a.Xg[gj * a.KG + k], pm);
-        if (a.margin) {                       // prior samples, no KL term (model_TFProb.py:156-157, 202-205)
-          zc = pm; zsl = tj;
-        } else {
-          const float d = lam[j] - tj;
-          const float r0 = (mu[j] - pm) * expf(-tj);
-          kl[j] += 0.5f * r0 * r0 + 0.5f * expm1f(2.0f * d) - d;
-        }
+        const float pm = prior_mean(a, m, row, gj, a.cell_mode ? b_row : bb[j]);
+        if (a.margin) { zc = pm; zsl = tj; }   // prior samples, no KL term (model_TFProb.py:156-157, 202-205)
+        else kl[j] += kl_normal(mu[j], lam[j], pm, tj);
         n = c1[j] + c2[j] + c3[j];
       }
       // elements with reads, one at a time, all 32 lanes cooperating
@@ -1143,10 +1169,7 @@ __global__ void __launch_bounds__(kThreads) eval_loss_kernel(const EvalArgs a) {
         const uint32_t ev = (uint32_t)(a.event_offset + (int64_t)tile * kTileCols + src * 4 + j);
         const float tot = eval_item(imu, expf(ilam), ic1, ic2, in, l1, l2, l3, eff, a.margin != 0, a.n_eval, a.S, ev,
                                     (uint32_t)row, stream0, a.seed, lane);
-        if (lane == src) {
-          const float k0 = eff ? fmaf(c1[j], logf(L1[j]), fmaf(c2[j], logf(L2[j]), c3[j] * logf(L3[j]))) : 0.f;
-          ll[j] += fmaf(tot, inv_n, k0);
-        }
+        if (lane == src) ll[j] += fmaf(tot, inv_n, log_length_const(eff, c1[j], c2[j], c3[j], L1[j], L2[j], L3[j]));
       }
     }
   }
@@ -1211,49 +1234,32 @@ __global__ void __launch_bounds__(256) element_terms_kernel(const TermsArgs a) {
     float o_ll = 0.f, o_kl = 0.f, o_pm = 0.f;
     if (g < a.Ng) {
       const float tj = a.cell_mode ? a.tau[(int64_t)m * a.Nc + row] : a.tau[(int64_t)m * a.ld + g];
-      float pm = a.cell_mode ? a.b[(int64_t)m * a.Nc + row] : a.b[(int64_t)m * a.ld + g];
-      for (int k = 0; k < a.KC; ++k)
-        pm = fmaf(a.Xc[((int64_t)m * a.Nc + row) * a.KC + k], a.Wc[((int64_t)m * a.KC + k) * a.ld + g], pm);
-      for (int k = 0; k < a.KG; ++k)
-        pm = fmaf(a.Wg[((int64_t)m * a.Nc + row) * a.KG + k], a.Xg[g * a.KG + k], pm);
+      const float pm =
+          prior_mean(a, m, row, g, a.cell_mode ? a.b[(int64_t)m * a.Nc + row] : a.b[(int64_t)m * a.ld + g]);
       o_pm = pm;
       const float mu = a.Zl[(int64_t)m * a.Nc * a.ld + i], lam = a.Zs[(int64_t)m * a.Nc * a.ld + i];
-      if (a.kl) {
-        const float d = lam - tj;
-        const float r0 = (mu - pm) * expf(-tj);
-        o_kl = 0.5f * r0 * r0 + 0.5f * expm1f(2.0f * d) - d;
-      }
+      if (a.kl) o_kl = kl_normal(mu, lam, pm, tj);
       if (a.loglik) {
         const float c1 = a.c[0][i], c2 = a.c[1][i], c3 = a.c[2] ? a.c[2][i] : 0.f;
         const float n = c1 + c2 + c3;
-        float L1 = 1.f, L2 = 1.f, L3 = 0.f;
-        if (eff) { L1 = a.eff[g]; L2 = a.eff[a.ld + g]; L3 = a.eff[2 * a.ld + g]; }
+        float L1, L2, L3;
+        event_lengths(a.eff, a.ld, g, L1, L2, L3);
         const float zc = a.margin ? pm : mu, zs = expf(a.margin ? tj : lam);
-        const float k0 = eff ? fmaf(c1, logf(L1), fmaf(c2, logf(L2), c3 * logf(L3))) : 0.f;
-        float acc = 0.f, mx = -INFINITY, Z = 0.f;
+        const float k0 = log_length_const(eff, c1, c2, c3, L1, L2, L3);
+        float acc = 0.f;
+        LogMeanExp lme;
         if (n > 0.f || a.margin) {
           for (int s0 = 0; s0 < a.S; s0 += 4) {
             float eps[4];
             brie_normals4((uint32_t)(a.event_offset + g), (uint32_t)row, a.noise_step, stream0 + (uint32_t)(s0 >> 2),
                           a.seed, eps);
             for (int q = 0; q < 4 && s0 + q < a.S; ++q) {
-              const float z = fmaf(zs, eps[q], zc);
-              const float e = expf(-fabsf(z));
-              const float lsp = fminf(z, 0.f) - log1pf(e);
-              const float inv = 1.0f / (1.0f + e);
-              const float psi = z >= 0.f ? inv : e * inv;
-              const float qq = z >= 0.f ? e * inv : inv;
-              const float D = fmaf(psi, L1, fmaf(qq, L2, L3));
-              const float l = fmaf(c1, lsp, c2 * (lsp - z)) - (eff ? n * logf(D) : 0.f) + k0;
-              if (!a.margin) {
-                acc += l;
-              } else {
-                if (l > mx) { Z *= expf(mx - l); mx = l; }
-                Z += expf(l - mx);
-              }
+              const float l = sample_ll(fmaf(zs, eps[q], zc), c1, c2, n, L1, L2, L3, eff).l + k0;
+              if (!a.margin) acc += l;
+              else lme.add(l);
             }
           }
-          o_ll = a.margin ? mx + logf(Z) - logf((float)a.S) : acc / (float)a.S;
+          o_ll = a.margin ? lme.value(a.S) : acc / (float)a.S;
         }
       }
     }
@@ -1296,8 +1302,8 @@ __global__ void __launch_bounds__(256) resample_counts_kernel(uint64_t seed, int
     float o1 = 0.f, o2 = 0.f, o3 = 0.f;
     const int n = g < Ng ? (int)rintf(total[i]) : 0;
     if (n > 0) {
-      float L1 = 1.f, L2 = 1.f, L3 = 0.f;
-      if (eff) { L1 = eff[g]; L2 = eff[ld + g]; L3 = eff[2 * ld + g]; }
+      float L1, L2, L3;
+      event_lengths(eff, ld, g, L1, L2, L3);
       const float ps = psi[i];
       const float p1 = ps * L1, p2 = (1.f - ps) * L2, D = p1 + p2 + L3;
       uint32_t ctr = 0;
@@ -1445,8 +1451,8 @@ __global__ void __launch_bounds__(256) simulate_counts_kernel(uint64_t seed, int
         for (int k = 0; k < Kc; ++k) z = fmaf(Xc[c * Kc + k], Wc[(int64_t)k * ld + g], z);
         z = fminf(fmaxf(z, -9.f), 9.f);
         const float psi = 1.f / (1.f + expf(-z));
-        float L1 = 1.f, L2 = 1.f, L3 = 0.f;
-        if (eff) { L1 = eff[g]; L2 = eff[ld + g]; L3 = eff[2 * ld + g]; }
+        float L1, L2, L3;
+        event_lengths(eff, ld, g, L1, L2, L3);
         const float p1 = psi * L1, p2 = (1.f - psi) * L2, D = p1 + p2 + L3;
         const int k1 = sim_binomial(r, n, p1 / D);
         const int k2 = sim_binomial(r, n - k1, p2 / (D - p1));

@@ -47,21 +47,14 @@ __device__ __forceinline__ void margin_element(float pm, float sig, float c1, fl
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       if (s0 + q < S) {
-        const float z = fmaf(sig, eps[q], pm);
-        const float e = expf(-fabsf(z));
-        const float lsp = fminf(z, 0.f) - log1pf(e);
-        const float inv = 1.0f / (1.0f + e);
-        const float psi = z >= 0.f ? inv : e * inv;
-        const float qq = z >= 0.f ? e * inv : inv;
-        const float D = fmaf(psi, L1, fmaf(qq, L2, L3));
-        const float l = fmaf(c1, lsp, c2 * (lsp - z)) - (eff ? n * logf(D) : 0.f);
-        const float gz = fmaf(c1, qq, -c2 * psi) - ndL * (psi * qq) / D;
-        if (l > mx) {
-          const float sc = expf(mx - l);   // 0 on the first sample
+        const SampleLL r = sample_ll(fmaf(sig, eps[q], pm), c1, c2, n, L1, L2, L3, eff);
+        const float gz = fmaf(c1, r.q, -c2 * r.psi) - ndL * (r.psi * r.q) / r.D;
+        if (r.l > mx) {
+          const float sc = expf(mx - r.l);   // 0 on the first sample
           Z *= sc; A *= sc; B *= sc;
-          mx = l;
+          mx = r.l;
         }
-        const float w = expf(l - mx);
+        const float w = expf(r.l - mx);
         Z += w;
         A = fmaf(w, gz, A);
         B = fmaf(w * gz, eps[q], B);
@@ -111,7 +104,6 @@ __global__ void __launch_bounds__(kThreads) margin_step_kernel(const MarginArgs 
 #pragma unroll
     for (int i = 0; i < kMarginMaxCell; ++i) cacc[i] = 0.f;
     const float* xrow = a.Xc + ((int64_t)m * a.Nc + row) * KC;
-    const float* wgrow = a.Wg + ((int64_t)m * a.Nc + row) * KG;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int col = j * 32 + lane;
@@ -121,15 +113,11 @@ __global__ void __launch_bounds__(kThreads) margin_step_kernel(const MarginArgs 
       const float c1 = a.c[0][off], c2 = a.c[1][off], c3 = a.c[2] ? a.c[2][off] : 0.f;
       const float n = c1 + c2 + c3;
       if (!(n > 0.f)) continue;
-      float pm = cell ? a.b[(int64_t)m * a.Nc + row] : a.b[(int64_t)m * a.ld + g];
+      const float pm = prior_mean(a, m, row, g, cell ? a.b[(int64_t)m * a.Nc + row] : a.b[(int64_t)m * a.ld + g]);
       const float tj = cell ? a.tau[(int64_t)m * a.Nc + row] : a.tau[(int64_t)m * a.ld + g];
-      for (int k = 0; k < KC; ++k) pm = fmaf(xrow[k], a.Wc[((int64_t)m * KC + k) * a.ld + g], pm);
-      for (int k = 0; k < KG; ++k) pm = fmaf(wgrow[k], a.Xg[g * KG + k], pm);
-      float L1 = 1.f, L2 = 1.f, L3 = 0.f, k0 = 0.f;
-      if (eff) {
-        L1 = a.eff[g]; L2 = a.eff[a.ld + g]; L3 = a.eff[2 * a.ld + g];
-        k0 = fmaf(c1, logf(L1), fmaf(c2, logf(L2), c3 * logf(L3)));
-      }
+      float L1, L2, L3;
+      event_lengths(a.eff, a.ld, g, L1, L2, L3);
+      const float k0 = log_length_const(eff, c1, c2, c3, L1, L2, L3);
       float lme, G, H;
       margin_element(pm, expf(tj), c1, c2, n, L1, L2, L3, eff, a.S, (uint32_t)(a.event_offset + g), (uint32_t)row,
                      a.step, stream0, a.seed, lme, G, H);
