@@ -8,7 +8,7 @@ import ctypes as C
 import os
 
 BRIE_MAX_MODELS = 32
-ABI_VERSION = 9
+ABI_VERSION = 10
 TARGETS = {"ELBO": 0, "marginLik": 1}
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbrie_b200.so")
@@ -64,6 +64,7 @@ SYMBOLS = {
     "brie_fit_run_steps": (C.c_int, [_P, C.c_int32, C.c_int32, _P]),
     "brie_fit_set_active_blocks": (C.c_int, [_P, _P, C.c_int64, C.POINTER(C.c_int32)]),
     "brie_fit_set_count_codes": (C.c_int, [_P, _P, C.c_int64, _P]),
+    "brie_fit_set_model_mask": (C.c_int, [_P, C.c_uint32]),
     "brie_fit_step_phase": (C.c_int, [_P, C.c_int32, C.c_int32, _P]),
     "brie_fit_cell_grad": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_int64)]),
     "brie_comm_nccl_version": (C.c_int, []),

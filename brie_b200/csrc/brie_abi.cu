@@ -55,6 +55,10 @@ struct brie_fit {
   float alpha = 0.f;
   int64_t launches = 0;
   bool step_open = false;    // phase 0 done, phase 1 pending
+  // bit m set iff model m still steps (brie_fit_set_model_mask).  In shared-parameter fits (cell_mode or Kg > 0) the
+  // caller clears a model's bit when it stops, so its per-cell parameters stay put; for per-event fits the kernels
+  // also consult `active` per event.
+  uint32_t model_mask = 0;
   // optional CUDA-event timing of the fused step kernel (bench.py roofline)
   std::vector<cudaEvent_t> ev0, ev1;
   int ev_used = 0;
@@ -132,6 +136,10 @@ const char* blas_status(cublasStatus_t st) {
       return brie::fail(BRIE_ERR_CUDA, "%s failed: cuBLAS %s (%s:%d)", #call, blas_status(st_), __FILE__, __LINE__); \
   } while (0)
 
+uint32_t all_models(int n_models) { return n_models >= 32 ? 0xffffffffu : ((1u << n_models) - 1u); }
+
+bool model_steps(const brie_fit* f, int m) { return ((f->model_mask >> m) & 1u) != 0; }
+
 // Wide form, before the fused kernel: PM[m] (Nc x ld, row-major) = Xc[m] (Nc x Kc) Wc[m] (Kc x ld) + Wg[m] (Nc x Kg) Xg^T
 // (Z_prior, model_TFProb.py:121-125).  Row-major arrays are handed to cuBLAS as their column-major transposes.
 int wide_prior_mean(brie_fit* f, cudaStream_t s) {
@@ -141,6 +149,7 @@ int wide_prior_mean(brie_fit* f, cudaStream_t s) {
   BRIE_BLAS(cublasSetStream(f->blas, s));
   const int64_t plane = d.n_cells * d.ld;
   for (int m = 0; m < d.n_models; ++m) {
+    if (!model_steps(f, m)) continue;
     float* PM = scratch + f->off_PM + (size_t)m * plane;
     if (d.Kc > 0)
       BRIE_BLAS(cublasSgemm(f->blas, CUBLAS_OP_N, CUBLAS_OP_N, (int)d.ld, (int)d.n_cells, d.Kc, &one,
@@ -152,7 +161,7 @@ int wide_prior_mean(brie_fit* f, cudaStream_t s) {
       BRIE_BLAS(cublasSgemm(f->blas, CUBLAS_OP_T, CUBLAS_OP_N, (int)d.n_events, (int)d.n_cells, d.Kg, &one,
                             f->buf.Xg, d.Kg, f->buf.Wg + (size_t)m * d.n_cells * d.Kg, d.Kg, &one, PM, (int)d.ld));
   }
-  f->launches += d.n_models * ((d.Kc > 0) + (d.Kg > 0));
+  f->launches += (int64_t)__builtin_popcount(f->model_mask) * ((d.Kc > 0) + (d.Kg > 0));
   return BRIE_OK;
 }
 
@@ -166,6 +175,7 @@ int wide_gradients(brie_fit* f, cudaStream_t s) {
   BRIE_BLAS(cublasSetStream(f->blas, s));
   const int64_t plane = d.n_cells * d.ld;
   for (int m = 0; m < d.n_models; ++m) {
+    if (!model_steps(f, m)) continue;   // stopped: its R is stale and nothing reads its gradients
     const float* R = scratch + f->off_R + (size_t)m * plane;
     if (d.Kc > 0)
       BRIE_BLAS(cublasSgemm(f->blas, CUBLAS_OP_N, CUBLAS_OP_T, (int)d.ld, d.Kc, (int)d.n_cells, &minus, R, (int)d.ld,
@@ -175,7 +185,7 @@ int wide_gradients(brie_fit* f, cudaStream_t s) {
       BRIE_BLAS(cublasSgemm(f->blas, CUBLAS_OP_N, CUBLAS_OP_N, d.Kg, (int)d.n_cells, (int)d.n_events, &minus, f->buf.Xg,
                             d.Kg, R, (int)d.ld, &zero, scratch + f->off_G + (size_t)m * d.n_cells * f->ncell, f->ncell));
   }
-  f->launches += d.n_models * ((d.Kc > 0) + (d.Kg > 0));
+  f->launches += (int64_t)__builtin_popcount(f->model_mask) * ((d.Kc > 0) + (d.Kg > 0));
   return BRIE_OK;
 }
 
@@ -211,13 +221,6 @@ cudaError_t dispatch_step(const StepArgs& a, bool wide, int KC, int KG, bool cel
   return cudaErrorInvalidValue;
 }
 
-// bit m set iff model m still has an active event.  In shared-parameter fits
-// (cell_mode or Kg > 0) the caller deactivates whole models; for per-event fits
-// the kernels consult `active` per event and this mask stays all-ones.
-uint32_t g_all_models(const brie_fit* f) {
-  return f->d.n_models >= 32 ? 0xffffffffu : ((1u << f->d.n_models) - 1u);
-}
-
 // The fields that StepArgs, MarginArgs, EvalArgs and TermsArgs share under the same names; the rest are zero.
 template <class A>
 A fit_args(const brie_fit* f) {
@@ -241,7 +244,7 @@ CellArgs cell_args(const brie_fit* f, int n_tiles) {
   memset(&c, 0, sizeof c);
   c.Nc = d.n_cells; c.M = d.n_models; c.KG = d.Kg; c.NCELL = f->ncell; c.n_tiles = n_tiles;
   c.cell_mode = d.cell_mode; c.train_b = d.train_intercept; c.train_tau = d.train_sigma;
-  c.model_mask = g_all_models(f); c.alpha = f->alpha;
+  c.model_mask = f->model_mask; c.alpha = f->alpha;
   c.part_cell = scratch + f->off_part_cell; c.G = scratch + f->off_G;
   c.Wg = f->buf.Wg; c.b = f->buf.intercept; c.tau = f->buf.sigma_log;
   c.mom = f->buf.adam_small + f->off_mom_cell;
@@ -258,7 +261,7 @@ int launch_margin_step(brie_fit* f, int nev, int cell_tiles, cudaStream_t s) {
   MarginArgs g = fit_args<MarginArgs>(f);
   g.active = f->buf.active;
   g.part_ev = scratch + f->off_part_ev; g.part_cell = scratch + f->off_part_cell;
-  g.step = f->global_step; g.model_mask = g_all_models(f);
+  g.step = f->global_step; g.model_mask = f->model_mask;
   g.S = d.mc_size; g.rows_per_cta = f->sz.rows_per_cta;
   g.KC = d.Kc; g.KG = d.Kg; g.cell_mode = d.cell_mode; g.NEV = nev; g.NCELL = f->ncell;
   for (int m = 0; m < d.n_models; ++m) g.model_id[m] = d.model_id[m];
@@ -281,7 +284,7 @@ int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s) {
   a.active = f->buf.active;
   a.part_ev = scratch + f->off_part_ev; a.part_cell = scratch + f->off_part_cell;
   a.alpha = f->alpha; a.inv_S = 1.0f / (float)d.mc_size;
-  a.step = f->global_step; a.model_mask = g_all_models(f);
+  a.step = f->global_step; a.model_mask = f->model_mask;
   a.S = d.mc_size; a.rows_per_cta = f->sz.rows_per_cta;
   for (int m = 0; m < d.n_models; ++m) a.model_id[m] = d.model_id[m];
   a.ev_ids = f->buf.event_ids; a.c_mstride = f->buf.counts_model_stride; a.eff_mstride = f->buf.efflen_model_stride;
@@ -391,6 +394,7 @@ int brie_fit_create(const brie_fit_desc* desc, brie_fit** out) {
   if (!f) return fail(BRIE_ERR_ARG, "out of host memory");
   f->d = d;
   f->wide = wide;
+  f->model_mask = all_models(d.n_models);
   memset(&f->buf, 0, sizeof f->buf);
   const int n_tiles = (int)ceil_div(d.ld, step_tile_cols(wide ? 0 : d.Kc, wide ? 0 : d.Kg));   // 128 events per tile, 64 when Kc = 16
   // rows per CTA: up to 256 (fewer row-chunk partials for event_update_kernel) while keeping
@@ -715,6 +719,15 @@ int brie_fit_set_active_blocks(brie_fit* f, const int32_t* blk_ids, int64_t blk_
   f->blk_ids = blk_ids;
   f->blk_stride = blk_stride;
   f->blk_tiles = tiles;
+  return BRIE_OK;
+}
+
+int brie_fit_set_model_mask(brie_fit* f, uint32_t mask) {
+  if (!f) return fail(BRIE_ERR_ARG, "null argument");
+  if (f->step_open) return fail(BRIE_ERR_ARG, "a split step is still open");
+  if ((mask & ~all_models(f->d.n_models)) != 0)
+    return fail(BRIE_ERR_ARG, "model mask 0x%x has bits beyond n_models = %d", mask, f->d.n_models);
+  f->model_mask = mask;
   return BRIE_OK;
 }
 

@@ -405,11 +405,18 @@ class FitEngine:
         """act: (M, n_groups) bool -> per-event active mask.  When some reference batches are
         frozen the step kernel is pointed at the 8-event column blocks that still hold an active
         event (brie_fit_set_active_blocks): an extension round then costs what its active events
-        cost, not what the whole shard costs.  Bit-identical to the dense walk."""
+        cost, not what the whole shard costs.  Bit-identical to the dense walk.
+
+        A model with no active batch left is also taken out of the step (brie_fit_set_model_mask): its per-cell
+        parameters (Wg, a per-cell intercept / sigma_log), which no `active` flag covers, then stay put as its
+        per-event state does.  In a sharded fit `act` comes from the all-reduced group trace, so every rank sets the
+        same mask."""
         g = (np.arange(self.Ng) + self.event_offset) // self.group_size - self.first_group
         ev = np.zeros((self.M, self.ld), np.uint8)
         ev[:, :self.Ng] = act[:, g]
         self.active.copy_(torch.from_numpy(ev).to(self.device))
+        mask = sum(1 << m for m in range(self.M) if act[m].any())
+        _lib.check(self.lib.brie_fit_set_model_mask(self.h, mask))
         if self.shared or self.target != "ELBO" or os.environ.get("BRIE_NO_COMPACT"):
             return
         blk = ev.reshape(self.M, self.ld // 8, 8).any(axis=2)

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BRIE_ABI_VERSION 9
+#define BRIE_ABI_VERSION 10
 #define BRIE_MAX_MODELS 32
 #define BRIE_MAX_KC 16   /* widest design whose covariate contraction stays in registers / shared memory */
 #define BRIE_MAX_KG 8
@@ -173,6 +173,14 @@ int brie_fit_set_count_codes(brie_fit* fit, const uint32_t* codes, int64_t codes
  * target ELBO. */
 int brie_fit_set_active_blocks(brie_fit* fit, const int32_t* blk_ids, int64_t blk_stride,
                                const int32_t* n_blk_host);
+
+/* Which models the step entry points step: bit m of `mask` set = model m steps (brie_fit_create starts with all
+ * models).  A step leaves a cleared model alone: its fused or marginLik step CTAs, wide-form GEMMs, per-cell reduce
+ * and per-cell Adam update are skipped.  A shared-parameter fit (Kg > 0 or cell_mode) clears the bit of
+ * every model whose convergence-extension rounds (model_TFProb.py:250-258) have ended: its `active` flags keep its
+ * per-event state put, but only the mask keeps Wg and a per-cell intercept / sigma_log put.  Refuses bits at or
+ * beyond n_models and an open split step. */
+int brie_fit_set_model_mask(brie_fit* fit, uint32_t mask);
 
 /* All-reduce hook for event-sharded fits with shared per-cell parameters
  * (Kg > 0 or cell_mode).  brie_fit_step_phase runs ONE step in two halves:

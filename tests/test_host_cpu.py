@@ -139,6 +139,24 @@ def test_subfit_is_refused_by_every_entry_but_the_step(lib):
     lib.brie_fit_destroy(h)
 
 
+def test_model_mask_refuses_bits_beyond_the_models(lib):
+    """brie_fit_set_model_mask: a null fit and bits at or beyond n_models are refused; any subset of the models,
+    none and all 32 included, is taken.  (The open-split-step refusal needs a launched phase 0: test_gpu_frozen_models.)"""
+    assert lib.brie_fit_set_model_mask(None, 1) == -1 and b"null" in lib.brie_last_error()
+    for n_models, ok, bad in ((1, (0, 1), (2, 0x80000000)), (3, (0, 5, 7), (8, 0xf)), (32, (0xffffffff,), ())):
+        h = C.c_void_p()
+        d = _desc(n_models=n_models)
+        for m in range(n_models):
+            d.xc_mask[m] = 1
+        assert lib.brie_fit_create(C.byref(d), C.byref(h)) == 0
+        for mask in bad:
+            assert lib.brie_fit_set_model_mask(h, mask) == -1, (n_models, mask)
+            assert b"beyond n_models" in lib.brie_last_error()
+        for mask in ok:
+            assert lib.brie_fit_set_model_mask(h, mask) == 0, (n_models, mask)
+        lib.brie_fit_destroy(h)
+
+
 def test_host_normals_match_numpy_spec(lib):
     from brie_b200 import _lib
     S, R, Cn, off = 5, 7, 19, 4000
