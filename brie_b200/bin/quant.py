@@ -37,7 +37,8 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
           intercept=None, intercept_mode='gene', nproc=1, min_counts=50,
           min_counts_uniq=10, min_cells_uniq=30, min_MIF_uniq=0.001,
           min_iter=5000, max_iter=20000, MC_size=1, batch_size=500000,
-          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0, wald=False):
+          pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0, wald=False,
+          score_file=None):
     """CLI driver (quant.py:13-130).  `nproc` is accepted for compatibility (host threads are
     not on the hot path any more); `seed` keys the counter-based noise (new, default 0).
     `out_dir` (new): directory for `.npy` memory maps of the dense (cells, events) output layers
@@ -49,7 +50,10 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     there (checkpoint / restart).  `n_perm` (new): permutation replicates per tested covariate; adds the
     pooled permutation p-values and their FDR to the container (varm) and the table (fitBRIE).  `wald`
     (new): standard errors, Wald p-values and their FDR for every cell coefficient, from the fitted
-    posterior without refits (fitBRIE); in the container (varm) and the table.
+    posterior without refits (fitBRIE); in the container (varm) and the table.  `score_file` (new): a table laid out
+    like `cell_file` (cell ids, then one candidate covariate per column) whose candidates are score-tested against
+    the fitted model without refits (fitBRIE's score_X); every fitted cell must be in it.  Results go to the
+    container (varm, uns['score_ids']) and to <out>.brie_score.tsv.
 
     Multi-GPU: launch one process per GPU (`python -m torch.distributed.run --nproc-per-node N
     -m brie_b200.bin.quant ...`); every rank reads the input, fits its own event shard
@@ -84,6 +88,17 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
         Xc_ids = tab[0, 1:]
         adata = adata[mm1, :]
 
+    score_X, score_ids = None, None
+    if score_file is not None:
+        tab = _read_table(score_file)
+        idx = match(adata.obs.index, tab[1:, 0]).astype(float)
+        if not (idx == idx).all():
+            print("[BRIE2] Error: %d of %d cells are missing from --scoreFile." % ((idx != idx).sum(), len(idx)))
+            sys.exit(1)
+        score_X = tab[idx.astype(int) + 1, 1:].astype(np.float32)
+        score_ids = tab[0, 1:]
+        print("[BRIE2] %d candidate covariates for score tests" % len(score_ids))
+
     print("layers:", layer_keys)                                 # quant.py:69-75
     import torch
     adata = filter_genes(adata, min_counts=min_counts, min_counts_uniq=min_counts_uniq,
@@ -110,11 +125,13 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
             intercept=intercept, intercept_mode=intercept_mode,
             min_iter=min_iter, max_iter=max_iter, MC_size=MC_size, batch_size=batch_size,
             pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed, n_perm=n_perm, wald=wald,
-            **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
+            score_X=score_X, **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
 
     adata.uns['brie_version'] = brie_b200.__version__
     adata.uns['Xc_ids'] = Xc_ids
     adata.uns['Xg_ids'] = Xg_ids
+    if score_ids is not None:
+        adata.uns['score_ids'] = score_ids
 
     if rank != 0:                                                # every rank holds the full result; one writes it
         return adata
@@ -127,6 +144,9 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     out_table_file = ".".join(out_file.split('.')[:-1]) + '.brie_ident.tsv'
     df = io_utils.dump_results(adata)
     df.to_csv(out_table_file, sep='\t', header=True, index=True, index_label='GeneID', float_format='%.3e')
+    if score_ids is not None:
+        io_utils.score_table(adata).to_csv(".".join(out_file.split('.')[:-1]) + '.brie_score.tsv', sep='\t',
+                                           header=True, index=True, index_label='GeneID', float_format='%.3e')
     return adata
 
 
@@ -190,6 +210,10 @@ def main():
         help="Standard errors and Wald p-values of every cell coefficient from the fitted posterior, without "
              "refits, with their FDR over all events (columns <feature>_se, <feature>_pval_wald, "
              "<feature>_FDR_wald); covers every feature, also those not in --LRTindex")
+    group4.add_option("--scoreFile", dest="score_file", default=None,
+        help="Candidate cell covariates in tsv[.gz] laid out like --cellFile (cell ids, then one candidate per "
+             "column), score-tested against the fitted model from its posterior without refits; every fitted cell "
+             "must be in it.  Writes <out>.brie_score.tsv (columns <id>_score_z, <id>_pval_score, <id>_FDR_score)")
     parser.add_option_group(group1)
     parser.add_option_group(group2)
     parser.add_option_group(group3)
@@ -224,7 +248,8 @@ def main():
           options.min_uniq_count, options.min_cell, options.min_MIF,
           options.min_iter, options.max_iter, options.MC_size,
           options.batch_size, options.pseudo_count, options.test_base, options.seed,
-          options.out_dir, options.resume, options.n_perm, options.wald)
+          options.out_dir, options.resume, options.n_perm, options.wald,
+          **({} if options.score_file is None else dict(score_file=options.score_file)))
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         if dist.is_initialized():

@@ -17,6 +17,7 @@
 #include "brie_kernels.cuh"
 #include "brie_margin.cuh"
 #include "brie_wald.cuh"
+#include "brie_score.cuh"
 
 #include "brie_host.h"
 
@@ -816,36 +817,73 @@ int brie_fit_element_terms(brie_fit* f, int32_t model, const float* c1, const fl
 
 namespace {
 
-// Geometry of the Wald information pass of model m (brie_wald.cuh): x~ width, pair block, row chunks.
-struct WaldPlan {
-  int width, has_b, kt, n_pairs, pb, n_pblk, n_tiles, n_chunks;
+// Geometry shared by the passes over model m's fitted posterior (the Wald information, the score parts): x~ width
+// and row chunks.  `what` names the pass in the refusals.
+struct PosteriorPlan {
+  int width, has_b, kt, n_tiles, n_chunks;
   int64_t rows_per_chunk;
-  size_t scratch_bytes;
 };
 
-int wald_plan(const brie_fit* f, int32_t model, WaldPlan* w) {
+int posterior_plan(const brie_fit* f, int32_t model, const char* what, PosteriorPlan* p) {
   if (!f || !f->bound) return fail(BRIE_ERR_ARG, "fit not bound");
   const brie_fit_desc& d = f->d;
   if (model < 0 || model >= d.n_models) return fail(BRIE_ERR_ARG, "model index out of range");
   if (d.target != BRIE_TARGET_ELBO)
-    return fail(BRIE_ERR_UNSUPPORTED, "Wald information needs a trained posterior (target ELBO)");
-  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "Wald information is computed on the parent fit, not on a gathered sub-fit");
-  w->width = f->wide ? d.xc_width[model] : __builtin_popcount(d.xc_mask[model]);
-  w->has_b = (!d.cell_mode && d.train_intercept) ? 1 : 0;
-  w->kt = w->width + w->has_b;
-  w->n_pairs = w->kt * (w->kt + 1) / 2;
-  w->pb = w->n_pairs <= 4 ? 4 : (w->n_pairs <= 12 ? 12 : kWaldMaxPairs);
-  w->n_pblk = (int)ceil_div(w->n_pairs, w->pb);
-  w->n_tiles = (int)ceil_div(d.n_events, kWaldCols);
+    return fail(BRIE_ERR_UNSUPPORTED, "%s needs a trained posterior (target ELBO)", what);
+  if (f->subfit) return fail(BRIE_ERR_UNSUPPORTED, "%s is computed on the parent fit, not on a gathered sub-fit", what);
+  p->width = f->wide ? d.xc_width[model] : __builtin_popcount(d.xc_mask[model]);
+  p->has_b = (!d.cell_mode && d.train_intercept) ? 1 : 0;
+  p->kt = p->width + p->has_b;
+  p->n_tiles = (int)ceil_div(d.n_events, kWaldCols);
   // Row chunks of >= kWaldMinRows cells, at most kWaldMaxChunks of them: a function of n_cells alone, so the float64
   // sums over cells associate the same way whatever the event count -- an event chunk or shard of a fit gets the
   // same bits as the whole -- and the scratch stays within kWaldMaxChunks partials per output.
-  const int64_t blocks = (int64_t)w->n_tiles * w->n_pblk;
   const int64_t n_chunks = std::min<int64_t>(ceil_div(d.n_cells, kWaldMinRows), kWaldMaxChunks);
-  w->rows_per_chunk = ceil_div(ceil_div(d.n_cells, n_chunks), kWaldBatch) * kWaldBatch;
-  w->n_chunks = (int)ceil_div(d.n_cells, w->rows_per_chunk);
+  p->rows_per_chunk = ceil_div(ceil_div(d.n_cells, n_chunks), kWaldBatch) * kWaldBatch;
+  p->n_chunks = (int)ceil_div(d.n_cells, p->rows_per_chunk);
+  return BRIE_OK;
+}
+
+// Geometry of the Wald information pass of model m (brie_wald.cuh): the posterior plan, pair block, scratch.
+struct WaldPlan : PosteriorPlan {
+  int n_pairs, pb, n_pblk;
+  size_t scratch_bytes;
+};
+
+int wald_plan(const brie_fit* f, int32_t model, WaldPlan* w) {
+  int rc = posterior_plan(f, model, "Wald information", w);
+  if (rc) return rc;
+  const brie_fit_desc& d = f->d;
+  w->n_pairs = w->kt * (w->kt + 1) / 2;
+  w->pb = w->n_pairs <= 4 ? 4 : (w->n_pairs <= 12 ? 12 : kWaldMaxPairs);
+  w->n_pblk = (int)ceil_div(w->n_pairs, w->pb);
+  const int64_t blocks = (int64_t)w->n_tiles * w->n_pblk;
   if (blocks > 0x7fffffffLL) return fail(BRIE_ERR_UNSUPPORTED, "too many event tiles x pair blocks");
   w->scratch_bytes = (size_t)w->n_chunks * w->n_pairs * d.ld * sizeof(double);
+  return BRIE_OK;
+}
+
+// Geometry of the score pass of model m over n_cand candidates (brie_score.cuh): the posterior plan, candidate and
+// x~ blocks (<16, 1> when x~ is at most the intercept, else <8, 4>), outputs per event, scratch.
+struct ScorePlan : PosteriorPlan {
+  int jb, kb, n_jblk, n_kblk;
+  int64_t n_q;
+  size_t scratch_bytes;
+};
+
+int score_plan(const brie_fit* f, int32_t model, int32_t n_cand, ScorePlan* p) {
+  int rc = posterior_plan(f, model, "the score test", p);
+  if (rc) return rc;
+  if (n_cand <= 0) return fail(BRIE_ERR_ARG, "n_cand must be >= 1");
+  const brie_fit_desc& d = f->d;
+  p->kb = p->kt <= 1 ? 1 : 4;
+  p->jb = p->kt <= 1 ? 16 : 8;
+  p->n_jblk = (int)ceil_div(n_cand, p->jb);
+  p->n_kblk = std::max(1, (int)ceil_div(p->kt, p->kb));
+  if ((int64_t)p->n_tiles * p->n_jblk * p->n_kblk > 0x7fffffffLL)
+    return fail(BRIE_ERR_UNSUPPORTED, "too many event tiles x candidate blocks");
+  p->n_q = (int64_t)n_cand * (p->kt + 2) + p->kt;
+  p->scratch_bytes = (size_t)p->n_chunks * p->n_q * d.ld * sizeof(double);
   return BRIE_OK;
 }
 
@@ -854,6 +892,14 @@ cudaError_t launch_wald(const WaldArgs& a, dim3 grid, cudaStream_t s) {
   wald_info_kernel<PB><<<grid, kWaldCols * kWaldRowGroups, 0, s>>>(a);
   return cudaGetLastError();
 }
+
+template <int JB, int KB>
+cudaError_t launch_score(const ScoreArgs& a, dim3 grid, cudaStream_t s) {
+  score_parts_kernel<JB, KB><<<grid, kScoreCols * kScoreRowGroups, 0, s>>>(a);
+  return cudaGetLastError();
+}
+
+bool aligned8(const void* p) { return p && (((uintptr_t)p) & 7u) == 0; }
 
 }  // namespace
 
@@ -899,6 +945,49 @@ int brie_fit_wald_info(brie_fit* f, int32_t model, double* info, void* scratch, 
   }
   const int64_t n_out = d.n_events * w.n_pairs;
   wald_reduce_kernel<<<(unsigned)ceil_div(n_out, 256), 256, 0, s>>>(a.part, w.n_chunks, w.n_pairs, d.ld, d.n_events, info);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 2;
+  return BRIE_OK;
+}
+
+int brie_fit_score_sizes(const brie_fit* f, int32_t model, int32_t n_cand, size_t* scratch_bytes, int32_t* k_tilde) {
+  if (!scratch_bytes || !k_tilde) return fail(BRIE_ERR_ARG, "null argument");
+  ScorePlan p;
+  int rc = score_plan(f, model, n_cand, &p);
+  if (rc) return rc;
+  *scratch_bytes = p.scratch_bytes;
+  *k_tilde = p.kt;
+  return BRIE_OK;
+}
+
+int brie_fit_score_parts(brie_fit* f, int32_t model, const float* X, int32_t n_cand, int64_t ldx, double* U, double* A,
+                         double* B, double* Utheta, void* scratch, void* stream) {
+  ScorePlan p;
+  int rc = score_plan(f, model, n_cand, &p);
+  if (rc) return rc;
+  if (!X) return fail(BRIE_ERR_ARG, "X required");
+  if (ldx < n_cand) return fail(BRIE_ERR_ARG, "ldx must be >= n_cand");
+  if (!aligned8(U) || !aligned8(A) || !aligned8(scratch) || (p.kt > 0 && (!aligned8(B) || !aligned8(Utheta))))
+    return fail(BRIE_ERR_ARG, "outputs and scratch must be non-null and 8-byte aligned");
+  const brie_fit_desc& d = f->d;
+  cudaStream_t s = (cudaStream_t)stream;
+  ScoreArgs a;
+  memset(&a, 0, sizeof a);
+  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld; a.m = model;
+  a.Xc = f->buf.Xc; a.Wc = f->buf.Wc; a.Wg = f->buf.Wg; a.Xg = f->buf.Xg; a.KC = d.Kc; a.KG = d.Kg;
+  a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log; a.b = f->buf.intercept; a.tau = f->buf.sigma_log;
+  a.cell_mode = d.cell_mode;
+  a.X = X; a.ldx = ldx; a.J = n_cand;
+  a.width = p.width; a.wide = f->wide ? 1 : 0; a.kt = p.kt; a.xc_mask = d.xc_mask[model];
+  a.rows_per_chunk = p.rows_per_chunk; a.n_jblk = p.n_jblk; a.n_kblk = p.n_kblk; a.n_q = p.n_q;
+  a.part = (double*)scratch;
+  if (d.Kc > 0 && !a.Xc) return fail(BRIE_ERR_ARG, "Xc required");
+  const dim3 grid((unsigned)((int64_t)p.n_tiles * p.n_jblk * p.n_kblk), (unsigned)p.n_chunks);
+  if (p.kb == 1) BRIE_CUDA((launch_score<16, 1>(a, grid, s)));
+  else BRIE_CUDA((launch_score<8, 4>(a, grid, s)));
+  const int64_t n_out = d.n_events * p.n_q;
+  score_reduce_kernel<<<(unsigned)ceil_div(n_out, 256), 256, 0, s>>>(a.part, p.n_chunks, p.n_q, d.ld, d.n_events, n_cand,
+                                                                     p.kt, U, A, B, Utheta);
   BRIE_CUDA(cudaGetLastError());
   f->launches += 2;
   return BRIE_OK;

@@ -1010,13 +1010,15 @@ __device__ __forceinline__ float log_length_const(bool eff, float c1, float c2, 
 }
 
 // Prior mean intercept + Xc Wc + Wg Xg^T of (row, event g) for model m (model_TFProb.py:118-126); `base` is the
-// intercept.  A is any argument struct with the fields Nc, ld, KC, KG, Xc, Wc, Wg, Xg.
-template <class A>
-__device__ __forceinline__ float prior_mean(const A& a, int m, int64_t row, int64_t g, float base) {
-  float pm = base;
+// intercept.  A is any argument struct with the fields Nc, ld, KC, KG, Xc, Wc, Wg, Xg.  T is the accumulation type:
+// float for the model terms, double for the score pass (brie_score.cuh), whose residuals Z_loc - prior mean of cells
+// without reads are far smaller than the float32 rounding of the sum.
+template <class T, class A>
+__device__ __forceinline__ T prior_mean(const A& a, int m, int64_t row, int64_t g, T base) {
+  T pm = base;
   for (int k = 0; k < a.KC; ++k)
-    pm = fmaf(a.Xc[((int64_t)m * a.Nc + row) * a.KC + k], a.Wc[((int64_t)m * a.KC + k) * a.ld + g], pm);
-  for (int k = 0; k < a.KG; ++k) pm = fmaf(a.Wg[((int64_t)m * a.Nc + row) * a.KG + k], a.Xg[g * a.KG + k], pm);
+    pm = fma((T)a.Xc[((int64_t)m * a.Nc + row) * a.KC + k], (T)a.Wc[((int64_t)m * a.KC + k) * a.ld + g], pm);
+  for (int k = 0; k < a.KG; ++k) pm = fma((T)a.Wg[((int64_t)m * a.Nc + row) * a.KG + k], (T)a.Xg[g * a.KG + k], pm);
   return pm;
 }
 

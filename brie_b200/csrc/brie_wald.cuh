@@ -44,13 +44,14 @@ struct WaldArgs {
   double* part;         // (n_chunks, n_pairs, ld)
 };
 
-// Xc column of x~ column j, or -1 for the intercept's 1
-__device__ __forceinline__ int wald_xc_col(const WaldArgs& a, int j) {
-  if (j >= a.width) return -1;
-  if (a.wide) return j;
+// Xc column of x~ column j of a model whose x~ takes `width` Xc columns (!wide: the j-th set bit of xc_mask; wide:
+// column j), or -1 for the intercept's 1.  Shared by the Wald and score passes (brie_score.cuh).
+__device__ __forceinline__ int wald_xc_col(int width, int wide, uint32_t xc_mask, int j) {
+  if (j >= width) return -1;
+  if (wide) return j;
   int seen = 0;
   for (int k = 0; k < 32; ++k)
-    if ((a.xc_mask >> k) & 1u) {
+    if ((xc_mask >> k) & 1u) {
       if (seen == j) return k;
       ++seen;
     }
@@ -80,8 +81,8 @@ __global__ void __launch_bounds__(kWaldCols * kWaldRowGroups) wald_info_kernel(c
         first += kt - k;
         ++k;
       }
-      ck = wald_xc_col(a, k);
-      cl = wald_xc_col(a, k + (p - first));
+      ck = wald_xc_col(a.width, a.wide, a.xc_mask, k);
+      cl = wald_xc_col(a.width, a.wide, a.xc_mask, k + (p - first));
     }
     s_col[0][threadIdx.x] = ck;
     s_col[1][threadIdx.x] = cl;

@@ -23,6 +23,7 @@ KG_SUPPORTED = (0, 4, 8)
 
 
 K_WIDE_MAX = 4096
+SCORE_BLOCK_BYTES = 1 << 30     # device scratch + outputs of one block of score candidates (FitEngine.score_parts)
 
 
 def _pad_to(k, allowed, what):
@@ -99,6 +100,24 @@ def unpack_pairs(packed, kt):
 WALD_RCOND = 1e-12
 
 
+def _pd_factor(info):
+    """The positive-definiteness checks of wald_from_info on a batch of informations (Ng, K, K), and the Cholesky
+    factor of the accepted ones after rescaling to a unit diagonal: (ok (Ng,) bool, d (Ng, K) = sqrt(diag(info)),
+    idx = flatnonzero(ok), L (len(idx), K, K) with L L^T = info[idx] / d d^T)."""
+    Ng, K = info.shape[:2]
+    with np.errstate(invalid='ignore'):
+        d = np.sqrt(np.diagonal(info, axis1=1, axis2=2))         # rescale to a unit diagonal first
+    ok = np.all(np.isfinite(info), axis=(1, 2)) & np.all(d > 0, axis=1)
+    dd = np.where(ok[:, None], d, 1.0)
+    with np.errstate(invalid='ignore'):
+        R = np.where(ok[:, None, None], info / dd[:, :, None] / dd[:, None, :], np.eye(K))
+    ev = np.linalg.eigvalsh(R)
+    ok &= ev[:, 0] > WALD_RCOND * ev[:, -1]
+    idx = np.flatnonzero(ok)
+    L = np.linalg.cholesky(R[idx]) if idx.size else np.zeros((0, K, K))   # batched; PD after the checks above
+    return ok, d, idx, L
+
+
 def wald_from_info(coef, info):
     """Wald standard errors and p-values of per-event coefficients `coef` (Ng, K) from their observed information
     `info` (Ng, K, K): se = sqrt(diag(info^-1)), pval = chi2.sf((coef / se)^2, 1).  An event whose information is
@@ -111,17 +130,8 @@ def wald_from_info(coef, info):
     Ng, K = coef.shape
     se = np.full((Ng, K), np.nan)
     if K > 0 and Ng > 0:
-        with np.errstate(invalid='ignore'):
-            d = np.sqrt(np.diagonal(info, axis1=1, axis2=2))         # rescale to a unit diagonal first
-        ok = np.all(np.isfinite(info), axis=(1, 2)) & np.all(d > 0, axis=1)
-        dd = np.where(ok[:, None], d, 1.0)
-        with np.errstate(invalid='ignore'):
-            R = np.where(ok[:, None, None], info / dd[:, :, None] / dd[:, None, :], np.eye(K))
-        ev = np.linalg.eigvalsh(R)
-        ok &= ev[:, 0] > WALD_RCOND * ev[:, -1]
-        idx = np.flatnonzero(ok)
+        _, d, idx, L = _pd_factor(info)
         if idx.size:
-            L = np.linalg.cholesky(R[idx])                            # batched; PD after the checks above
             Linv = np.linalg.solve(L, np.broadcast_to(np.eye(K), L.shape))
             diag_inv = (Linv ** 2).sum(axis=1)                        # diag(R^-1) = column sums of Linv^2
             se[idx] = np.sqrt(diag_inv) / d[idx]
@@ -129,6 +139,42 @@ def wald_from_info(coef, info):
         pval = chi2.sf((coef / se) ** 2, df=1)
     pval[~np.isfinite(se)] = 1.0
     return se, pval
+
+
+SCORE_VTOL = 1e-10
+
+
+def score_from_parts(parts, info):
+    """Score tests of candidates from their parts (FitEngine.score_parts: U, A (Ng, J), B (Ng, J, K~), Ut (Ng, K~))
+    and the null model's information `info` (Ng, K~, K~) (DESIGN §2.3):
+        V = A - B I^-1 B^T   (efficient information),   Ue = U - B I^-1 Ut   (efficient score),
+        score_z = Ue / sqrt(V),   pval = chi2.sf(score_z^2, 1),   effect = Ue / V   (one-step estimate, logit scale).
+    An event whose information fails wald_from_info's checks, and a candidate with A <= 0 or V <= SCORE_VTOL * A
+    (collinear with the fitted columns, or zero on every cell), get score_z and effect NaN and pval 1.0.
+    Returns (score_z, effect, pval), each (Ng, J) float64."""
+    from scipy.stats import chi2
+    U, A, B, Ut = (np.asarray(x, np.float64) for x in parts)
+    info = np.asarray(info, np.float64)
+    Ng, J = U.shape
+    K = info.shape[1] if info.ndim == 3 else 0
+    V, Ue = A.copy(), U.copy()
+    ok = np.ones(Ng, bool)
+    if K > 0 and Ng > 0:
+        ok, d, idx, L = _pd_factor(info)
+        if idx.size:                                                  # B I^-1 B^T = (L^-1 Bs^T)^T (L^-1 Bs^T), Bs = B / d
+            dd = d[idx]
+            Y = np.linalg.solve(L, np.swapaxes(B[idx] / dd[:, None, :], 1, 2))      # (n, K, J)
+            y = np.linalg.solve(L, (Ut[idx] / dd)[:, :, None])                     # (n, K, 1)
+            V[idx] -= (Y ** 2).sum(axis=1)
+            Ue[idx] -= (Y * y).sum(axis=1)
+    good = ok[:, None] & (A > 0) & (V > SCORE_VTOL * A)
+    z, eff = np.full((Ng, J), np.nan), np.full((Ng, J), np.nan)
+    with np.errstate(invalid='ignore', divide='ignore'):
+        z[good] = Ue[good] / np.sqrt(V[good])
+        eff[good] = Ue[good] / V[good]
+    pval = np.ones((Ng, J))
+    pval[good] = chi2.sf(z[good] ** 2, df=1)
+    return z, eff, pval
 
 
 class FitEngine:
@@ -553,6 +599,45 @@ class FitEngine:
             _lib.check(self.lib.brie_fit_wald_info(self.h, int(m), packed.data_ptr(), scratch.data_ptr(),
                                                    self._stream()))
         return unpack_pairs(packed.cpu().numpy(), kt)
+
+    def score_parts(self, m, X):
+        """Score-test parts of candidate cell covariates X (Nc, J) against model m as the null model, from its fitted
+        posterior (brie_fit_score_parts; DESIGN §2.3): (U, A (Ng, J), B (Ng, J, K~), Ut (Ng, K~)) float64 host arrays,
+        x~ as in wald_info.  The candidates go in blocks whose device scratch and outputs stay within
+        SCORE_BLOCK_BYTES (the scratch alone is up to 64 row chunks x J (K~ + 2) x ld doubles)."""
+        X = torch.as_tensor(np.asarray(X, np.float32) if not torch.is_tensor(X) else X)
+        X = X.to(device=self.device, dtype=torch.float32).contiguous()
+        if X.dim() != 2 or X.shape[0] != self.Nc or X.shape[1] < 1:
+            raise ValueError("brie_b200: score candidates must be (%d, J >= 1), got %s" % (self.Nc, tuple(X.shape)))
+        J = X.shape[1]
+        nbytes, c_kt = C.c_size_t(), C.c_int32()
+
+        def scratch_of(n):
+            _lib.check(self.lib.brie_fit_score_sizes(self.h, int(m), int(n), C.byref(nbytes), C.byref(c_kt)))
+            return int(nbytes.value)
+        s1 = scratch_of(1)
+        kt = c_kt.value
+        s_cand = scratch_of(2) - s1                                         # the scratch grows linearly in J
+        per_cand = s_cand + 8 * self.Ng * (kt + 2)                          # + U, A and B
+        fixed = s1 - s_cand + 8 * self.Ng * kt                              # + Ut
+        jb = int(max(1, min(J, (SCORE_BLOCK_BYTES - fixed) // per_cand)))
+        new = lambda *shape: torch.empty(shape, dtype=torch.float64, device=self.device)
+        out_U, out_A, out_B, Ut = np.empty((self.Ng, J)), np.empty((self.Ng, J)), np.empty((self.Ng, J, kt)), None
+        ptr = lambda t: t.data_ptr() if t.numel() else None
+        for j0 in range(0, J, jb):
+            n = min(jb, J - j0)
+            U, A, B, T = new(self.Ng, n), new(self.Ng, n), new(self.Ng, n, kt), new(self.Ng, kt)
+            scratch = torch.empty(max(scratch_of(n), 8), dtype=torch.uint8, device=self.device)
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.brie_fit_score_parts(self.h, int(m), X[:, j0:].data_ptr(), int(n), int(J),
+                                                         U.data_ptr(), A.data_ptr(), ptr(B), ptr(T),
+                                                         scratch.data_ptr(), self._stream()))
+            out_U[:, j0:j0 + n], out_A[:, j0:j0 + n] = U.cpu().numpy(), A.cpu().numpy()
+            out_B[:, j0:j0 + n] = B.cpu().numpy()
+            if Ut is None:
+                Ut = T.cpu().numpy()
+            del U, A, B, T, scratch
+        return out_U, out_A, out_B, Ut
 
     # ------------------------------------------------------------------ schedule
     def fit(self, min_iter=1000, max_iter=5000, add_iter=500, epsilon_conv=1e-2, n_eval=500,

@@ -7,12 +7,13 @@ model_wrap.py:156-187) run as one batched `FitEngine`, and the sequential event
 batches of `fitBRIE` (model_wrap.py:241-260) become convergence groups inside
 the same launches, so one pass over the counts serves all of them.
 """
+import hashlib
 import time
 
 import numpy as np
 from scipy.stats import chi2
 
-from ..engine import FitEngine, wald_from_info
+from ..engine import SCORE_BLOCK_BYTES, FitEngine, score_from_parts, wald_from_info
 from ..sharding import event_shards
 from ..utils.layer_store import LayerStore, BIG_KEYS
 from ..settings import verbosity
@@ -157,6 +158,43 @@ def _set_wald_outputs(res, per_model, full, base_cols, tested):
     _set_fdr_wald(res)
 
 
+SCORE_KEYS = ('score_z', 'score_effect', 'pval_score', 'fdr_score')
+
+
+def check_score_X(score_X, target, Nc):
+    """Validate `score_X` against the fit (before any device work): None, or a finite (Nc, J >= 1) matrix of
+    candidate cell covariates, returned as float32; a marginLik fit trains no posterior to score against."""
+    if score_X is None:
+        return None
+    if target == "marginLik":
+        raise ValueError("score_X needs target 'ELBO': a marginLik fit has no trained posterior")
+    X = np.asarray(score_X, np.float32)
+    if X.ndim != 2 or X.shape[0] != Nc or X.shape[1] < 1:
+        raise ValueError("score_X must be (n_cells=%d, J >= 1), got shape %s" % (Nc, np.shape(score_X)))
+    if not np.isfinite(X).all():
+        raise ValueError("score_X has non-finite values")
+    return X
+
+
+def _score_of_model(eng, j, X):
+    """(score_z, score_effect, pval_score) of candidates X against model j of a fitted engine as the null model
+    (FitEngine.score_parts with the model's information, score_from_parts)."""
+    return score_from_parts(eng.score_parts(j, X), eng.wald_info(j))
+
+
+def _set_fdr_score(res):
+    """fdr_score: BH over all events of the result, per candidate (the pooled scope of fdr_wald)."""
+    res.fdr_score = np.zeros(res.pval_score.shape)
+    for i in range(res.fdr_score.shape[1]):
+        res.fdr_score[:, i] = fdr_bh(res.pval_score[:, i])
+
+
+def _append_score(out, r):
+    """Event-axis concatenation of the score outputs of two results (fdr_score is recomputed over all events)."""
+    for k in SCORE_KEYS:
+        setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
+
+
 def _append_wald(out, r):
     """Event-axis concatenation of the Wald outputs of two results (fdr_wald is recomputed over all events)."""
     out.cell_coeff_se = np.append(out.cell_coeff_se, r.cell_coeff_se, axis=1)
@@ -222,6 +260,8 @@ class BRIE_RV():
                 setattr(self, k, np.append(getattr(self, k), getattr(new_RV, k), axis=0))
         if hasattr(new_RV, 'pval_wald'):
             _append_wald(self, new_RV)
+        if hasattr(new_RV, 'pval_score'):
+            _append_score(self, new_RV)
         if hasattr(new_RV, 'n_iter'):
             self.n_iter = np.append(self.n_iter, new_RV.n_iter, axis=1)
         if getattr(self, 'timing', None) is not None and getattr(new_RV, 'timing', None) is not None:
@@ -346,7 +386,7 @@ def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=No
 
 def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
                     intercept_mode='gene', LRT_index=None, pseudo_count=0.01,
-                    sigma=None, base_mode='full', tau_prior=[3, 27], **keyargs):
+                    sigma=None, base_mode='full', tau_prior=[3, 27], score_X=None, **keyargs):
     """Fit a BRIE model with cell and/or gene features (model_wrap.py:88-199).
 
     Extra keyword arguments consumed here (not in the reference): `seed` (noise and
@@ -371,6 +411,13 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     base_mode 'null': then the last row of each test model, from that model's own information), `intercept_se`
     (1, Ng) when the intercept is per-event and trained, `pval_wald` / `fdr_wald` (Ng, rows of cell_coeff; BH
     over all events) and `wald_columns`, the Xc column of each cell_coeff row.  Every other output is unchanged.
+
+    `score_X` (Nc, J), candidate cell covariates aligned with the cells, adds their Rao score tests against model 0
+    (the full model, or the base model with base_mode 'null') from its fitted posterior, without refits (DESIGN
+    §2.3): `score_z`, `score_effect` (one-step estimate of each candidate's coefficient, logit scale), `pval_score`
+    and `fdr_score` (BH per candidate over all events), each (Ng, J).  A candidate collinear with the fitted columns
+    or zero on every cell, and an event whose information is not positive definite, get NaN and pval 1.  Every
+    other output is unchanged.
     """
     from scipy.sparse import issparse
     seed = keyargs.pop('seed', 0)
@@ -388,6 +435,7 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     n_tests = len(LRT_index) if LRT_index is not None else (0 if Xc is None else np.shape(Xc)[1])
     n_perm = check_n_perm(keyargs.pop('n_perm', 0), n_tests)
     wald = check_wald(keyargs.pop('wald', False), target)
+    score_X = check_score_X(score_X, target, data[0].shape[0])
     for k in ('optimizer', 'learn_rate', 'verbose'):                # accepted and ignored (:214-237)
         keyargs.pop(k, None)
 
@@ -500,6 +548,8 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
             n_iter_rows[mid] = eng.n_iter[j]
             if wald and (mid == 0 or not full):
                 wald_out[mid] = _wald_of_model(eng, j)
+            if score_X is not None and mid == 0:
+                score_out = _score_of_model(eng, j, score_X)
             if mid == 0:
                 brie_results = _rv_from_engine(eng, j, Xc[:, base_cols], Xg, intercept_mode, out_sink)   # :146
             else:
@@ -515,6 +565,9 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     brie_results.timing = timing
     if wald:
         _set_wald_outputs(brie_results, wald_out, full, base_cols, LRT_index)
+    if score_X is not None:
+        brie_results.score_z, brie_results.score_effect, brie_results.pval_score = score_out
+        _set_fdr_score(brie_results)
     if T == 0:                                                      # :152-153
         return brie_results
 
@@ -570,6 +623,8 @@ def _merge_shared(parts):
                 setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
         if hasattr(r, 'pval_wald'):
             _append_wald(out, r)
+        if hasattr(r, 'pval_score'):
+            _append_score(out, r)
     out.shape = (out.Nc, out.Ng)
     if hasattr(out, 'pval'):               # one fit => one multiple-testing scope over all events
         for i in range(out.fdr.shape[1]):
@@ -601,18 +656,19 @@ def _balanced_chunk(n_events, budget, n_gene):
     return max(-(-groups // n_chunks), 1) * n_gene
 
 
-def _device_event_budget(Nc, n_models, n_layers, device=None, frac=0.7):
-    """Events per device chunk so that counts, their packed codes, (1+T) model states and outputs fit in HBM."""
+def _device_event_budget(Nc, n_models, n_layers, device=None, frac=0.7, reserve=0):
+    """Events per device chunk so that counts, their packed codes, (1+T) model states and outputs fit in HBM,
+    besides `reserve` bytes held for the whole fit (the score candidates and one block of the score pass)."""
     import torch
     free, _ = torch.cuda.mem_get_info(device)
     per_event = Nc * 4 * (n_layers + 1 + 6 * n_models + 3 + 1) * 1.05
-    return max(int(free * frac / per_event), 1)
+    return max(int(max(free - reserve, 0) * frac / per_event), 1)
 
 
 def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             LRT_index=[], layer_keys=['isoform1', 'isoform2', 'ambiguous'],
             batch_size=500000, pseudo_count=0.01, sigma=None,
-            base_mode='full', tau_prior=[3, 27], **keyargs):
+            base_mode='full', tau_prior=[3, 27], score_X=None, **keyargs):
     """Fit a BRIE model from AnnData with cell and/or gene features (model_wrap.py:202-314).
 
     `out_dir` (not in the reference): directory for `.npy` memory maps of the dense
@@ -629,6 +685,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     `wald` (not in the reference, default False): Wald tests from the fitted posterior, see fit_BRIE_matrix;
     stored as varm['cell_coeff_se', 'pval_wald', 'fdr_wald'] (and varm['intercept_se'] in gene mode) with
     uns['brie_param']['wald'] and ['wald_columns']; fdr_wald is BH over all events of the fit.
+    `score_X` (not in the reference, default None): (Nc, J) candidate cell covariates aligned with adata's cells,
+    score-tested from the fitted posterior, see fit_BRIE_matrix; stored as varm['score_z', 'score_effect',
+    'pval_score', 'fdr_score'] (Ng, J) with uns['brie_param']['score'] = J; fdr_score is BH over all events of the fit.
 
     Returns the BRIE_RV result and adds to `adata` exactly the keys the reference adds
     (obsm['Xc'], varm['cell_coeff'], varm['Xg'], obsm['gene_coeff'], varm|obsm['intercept',
@@ -649,6 +708,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     wald = check_wald(keyargs.pop('wald', False), keyargs.get('target', "ELBO"))
     if wald:                               # (likewise absent when False)
         keyargs['wald'] = True
+    score_X = check_score_X(score_X, keyargs.get('target', "ELBO"), Nc)
     out_dir = keyargs.pop('out_dir', None)
     resume = keyargs.pop('resume', False)
     out_keys = tuple(keyargs.pop('out_keys', None) or BIG_KEYS)
@@ -660,12 +720,15 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         # groups per launch as HBM holds, and give each GPU a contiguous range of groups.
         _n_gene = int(np.ceil(batch_size / Nc))
         lo, hi = event_shards(Ng, world, _n_gene)[rank]
-        chunk = _device_event_budget(Nc, n_models, len(layer_keys), keyargs.get('device'))
+        chunk = _device_event_budget(Nc, n_models, len(layer_keys), keyargs.get('device'),
+                                     **({} if score_X is None else dict(reserve=score_X.nbytes + SCORE_BLOCK_BYTES)))
         chunk = _balanced_chunk(hi - lo, chunk, _n_gene)
         # finished chunks go straight into their column range of the output arrays (RAM, or
         # .npy memory maps under out_dir shared by all ranks) instead of np.append (:55-76)
         signature = _fit_signature(Nc, Ng, Xc, LRT_index, layer_keys, _n_gene, world, intercept, intercept_mode,
                                    pseudo_count, sigma, base_mode, keyargs) if out_dir is not None else None
+        if signature is not None and score_X is not None:     # (absent without score_X)
+            signature['score_X_sha1'] = hashlib.sha1(score_X.tobytes()).hexdigest()
         store = LayerStore(Nc, Ng, out_dir, rank, world, dist, keys=out_keys, signature=signature, resume=resume)
         res_list = []
         pending = None                     # (sink, result) of the chunk whose layers are still on their way to the host
@@ -699,7 +762,8 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
                     intercept=intercept, intercept_mode=intercept_mode,
                     LRT_index=LRT_index, pseudo_count=pseudo_count, sigma=sigma,
                     base_mode=base_mode, tau_prior=tau_prior, group_size=_n_gene,
-                    event_offset=e0, n_events_total=Ng, host_side_effect=False, out_sink=_sink, **keyargs)
+                    event_offset=e0, n_events_total=Ng, host_side_effect=False, out_sink=_sink, score_X=score_X,
+                    **keyargs)
             finally:
                 _land()
             pending = (_sink, _ResVal)
@@ -732,7 +796,8 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             intercept_mode=intercept_mode, LRT_index=LRT_index,
             pseudo_count=pseudo_count, sigma=sigma, base_mode=base_mode,
             tau_prior=tau_prior, event_offset=lo, n_events_total=Ng,
-            dist_group=dist.group.WORLD, out_sink=_ChunkSink(store, lo, background=False), **keyargs)
+            dist_group=dist.group.WORLD, out_sink=_ChunkSink(store, lo, background=False), score_X=score_X,
+            **keyargs)
         store.put(lo, local, checkpoint=False)
         parts = [None] * world
         dist.all_gather_object(parts, local)
@@ -746,12 +811,14 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             _count_layers, Xc=Xc, Xg=Xg, effLen=_effLen, intercept=intercept,
             intercept_mode=intercept_mode, LRT_index=LRT_index,
             pseudo_count=pseudo_count, sigma=sigma, base_mode=base_mode,
-            tau_prior=tau_prior, **keyargs)
+            tau_prior=tau_prior, score_X=score_X, **keyargs)
 
     if n_perm > 0:                         # one pooled null over every event of the fit, the same on every rank
         _set_perm_outputs(ResVal)
     if wald:                               # one BH scope over every event of the fit
         _set_fdr_wald(ResVal)
+    if score_X is not None:                # likewise
+        _set_fdr_score(ResVal)
 
     # update adata (:271-311)
     if Xc.shape[0] > 0:
@@ -789,6 +856,9 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         adata.varm['fdr_wald'] = ResVal.fdr_wald
         if hasattr(ResVal, 'intercept_se') and ResVal.intercept_mode == 'gene':
             adata.varm['intercept_se'] = ResVal.intercept_se.T
+    if score_X is not None:
+        for k in SCORE_KEYS:
+            adata.varm[k] = getattr(ResVal, k)
 
     adata.uns['brie_param'] = {
         'LRT_index': LRT_index,
@@ -804,4 +874,6 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     if wald:
         adata.uns['brie_param']['wald'] = True
         adata.uns['brie_param']['wald_columns'] = list(ResVal.wald_columns)
+    if score_X is not None:
+        adata.uns['brie_param']['score'] = int(score_X.shape[1])
     return ResVal

@@ -97,3 +97,14 @@ def dump_results(adata):
             table[label + '_pval_wald'] = adata.varm['pval_wald'][:, j]
             table[label + '_FDR_wald'] = adata.varm['fdr_wald'][:, j]
     return table
+
+
+def score_table(adata):
+    """Per-event table of the score tests of candidate cell covariates (brie-quant --scoreFile), written as
+    <out>.brie_score.tsv: per candidate, in uns['score_ids'] order, <id>_score_z, <id>_pval_score, <id>_FDR_score."""
+    table = pd.DataFrame(index=adata.var.index)
+    for j, cid in enumerate(adata.uns['score_ids']):
+        table[str(cid) + '_score_z'] = adata.varm['score_z'][:, j]
+        table[str(cid) + '_pval_score'] = adata.varm['pval_score'][:, j]
+        table[str(cid) + '_FDR_score'] = adata.varm['fdr_score'][:, j]
+    return table

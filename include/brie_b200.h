@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BRIE_ABI_VERSION 10
+#define BRIE_ABI_VERSION 11
 #define BRIE_MAX_MODELS 32
 #define BRIE_MAX_KC 16   /* widest design whose covariate contraction stays in registers / shared memory */
 #define BRIE_MAX_KG 8
@@ -241,6 +241,26 @@ int brie_fit_posterior(brie_fit* fit, int32_t model, float* Psi, float* Psi95CI,
  *                        posterior). */
 int brie_fit_wald_sizes(const brie_fit* fit, int32_t model, size_t* scratch_bytes, int32_t* k_tilde);
 int brie_fit_wald_info(brie_fit* fit, int32_t model, double* info, void* scratch, void* stream);
+
+/* Score-test parts of n_cand candidate cell covariates against model `model` as the null model (no reference
+ * counterpart; DESIGN §2.3), from its fitted posterior with no refit.  With x~_c as above, the prior mean m_cg, sigma
+ * the event's (or, cell_mode, the cell's) and x_cj = X[c * ldx + j]:
+ *   r_cg = (Z_loc[model, c, g] - m_cg) / sigma^2,   w_cg = max(sigma^2 - s_cg^2, 0) / sigma^4   (as in the Wald pass)
+ *   U[g, j] = sum_c x_cj r_cg,   A[g, j] = sum_c w_cg x_cj^2,   B[g, j, k] = sum_c w_cg x_cj x~_ck,
+ *   Utheta[g, k] = sum_c x~_ck r_cg
+ * in float64 (the prior mean too).  With I_g of brie_fit_wald_info the efficient information of candidate j is
+ * A - B I^-1 B^T and its efficient score U - B I^-1 Utheta.
+ *  brie_fit_score_sizes : scratch bytes and K~ of `model` for n_cand candidates (the scratch grows with n_cand:
+ *                         up to 64 row chunks x n_cand (K~ + 2) x ld doubles; callers split the candidates);
+ *  brie_fit_score_parts : X (DEVICE, (n_cells, ldx) float32, ldx >= n_cand); U, A (DEVICE, (n_events, n_cand)),
+ *                         B (DEVICE, (n_events, n_cand, K~)), Utheta (DEVICE, (n_events, K~)), all float64 and
+ *                         8-byte aligned (B and Utheta may be NULL when K~ = 0).  The row chunks are the Wald pass's,
+ *                         a function of n_cells alone; no atomics: repeated calls, event chunks and shards give the
+ *                         same bits.  Works on a fit whose extension rounds ran on gathered sub-fits (not on a
+ *                         sub-fit itself).  Target ELBO only. */
+int brie_fit_score_sizes(const brie_fit* fit, int32_t model, int32_t n_cand, size_t* scratch_bytes, int32_t* k_tilde);
+int brie_fit_score_parts(brie_fit* fit, int32_t model, const float* X, int32_t n_cand, int64_t ldx, double* U,
+                         double* A, double* B, double* Utheta, void* scratch, void* stream);
 
 /* Replaces the tensors the public model API returns for one model (BRIE2.logLik_MC model_TFProb.py:130-191,
  * Z_prior :118-127, the KL of get_loss :208), as dense (Nc, ld) arrays; any output may be NULL.
