@@ -38,7 +38,7 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
           min_counts_uniq=10, min_cells_uniq=30, min_MIF_uniq=0.001,
           min_iter=5000, max_iter=20000, MC_size=1, batch_size=500000,
           pseudo_count=0.01, base_mode='full', seed=0, out_dir=None, resume=False, n_perm=0, wald=False,
-          score_file=None):
+          score_file=None, LRT_groups=None, wald_groups=None, score_groups=None):
     """CLI driver (quant.py:13-130).  `nproc` is accepted for compatibility (host threads are
     not on the hot path any more); `seed` keys the counter-based noise (new, default 0).
     `out_dir` (new): directory for `.npy` memory maps of the dense (cells, events) output layers
@@ -53,7 +53,9 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     posterior without refits (fitBRIE); in the container (varm) and the table.  `score_file` (new): a table laid out
     like `cell_file` (cell ids, then one candidate covariate per column) whose candidates are score-tested against
     the fitted model without refits (fitBRIE's score_X); every fitted cell must be in it.  Results go to the
-    container (varm, uns['score_ids']) and to <out>.brie_score.tsv.
+    container (varm, uns['score_ids']) and to <out>.brie_score.tsv.  `LRT_groups`, `wald_groups` (new): groups of
+    `cell_file` columns tested jointly by refits and from the fitted posterior; `score_groups` (new): groups of
+    `score_file` columns tested jointly (fitBRIE); results go to the container and the tables.
 
     Multi-GPU: launch one process per GPU (`python -m torch.distributed.run --nproc-per-node N
     -m brie_b200.bin.quant ...`); every rank reads the input, fits its own event shard
@@ -121,11 +123,22 @@ def quant(in_file, cell_file=None, gene_file=None, out_file=None,
     tau_prior = [1, 1] if 'unspliced' in adata.layers else [3, 27]     # quant.py:102-105 (unused downstream)
 
     from brie_b200.models import fitBRIE
+    from brie_b200.models.model_wrap import check_groups
+    n_cols = 0 if Xc is None else Xc.shape[1]
+    for flag, groups, n in (("--LRTgroups", LRT_groups, n_cols), ("--waldGroups", wald_groups, n_cols),
+                            ("--scoreGroups", score_groups, 0 if score_X is None else score_X.shape[1])):
+        try:
+            check_groups(groups, n, flag)
+        except ValueError as e:
+            print("[BRIE2] Error: %s (columns of %s)." % (e, "--scoreFile" if flag == "--scoreGroups" else "-c"))
+            sys.exit(1)
+    groups = {k: v for k, v in (('LRT_groups', LRT_groups), ('wald_groups', wald_groups),
+                                 ('score_groups', score_groups)) if v is not None}
     fitBRIE(adata, Xc=Xc, Xg=Xg, LRT_index=LRT_index, layer_keys=layer_keys,
             intercept=intercept, intercept_mode=intercept_mode,
             min_iter=min_iter, max_iter=max_iter, MC_size=MC_size, batch_size=batch_size,
             pseudo_count=pseudo_count, base_mode=base_mode, tau_prior=tau_prior, seed=seed, n_perm=n_perm, wald=wald,
-            score_X=score_X, **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
+            score_X=score_X, **groups, **(dict(out_dir=out_dir, resume=resume, out_keys=('Psi', 'Psi95CI', 'Z_std')) if out_dir is not None else {}))
 
     adata.uns['brie_version'] = brie_b200.__version__
     adata.uns['Xc_ids'] = Xc_ids
@@ -214,6 +227,16 @@ def main():
         help="Candidate cell covariates in tsv[.gz] laid out like --cellFile (cell ids, then one candidate per "
              "column), score-tested against the fitted model from its posterior without refits; every fitted cell "
              "must be in it.  Writes <out>.brie_score.tsv (columns <id>_score_z, <id>_pval_score, <id>_FDR_score)")
+    group4.add_option("--LRTgroups", dest="LRT_groups", default=None,
+        help="Groups of cell features (0-based columns of --cellFile) to test jointly with one refit per group, e.g. "
+             "the indicator columns of a categorical: ';'-separated groups of ','-separated indices, e.g. \"1,2,3;4,5\" "
+             "(columns <id>+<id>_ELBO_gain_group, _pval_group, _FDR_group)")
+    group4.add_option("--waldGroups", dest="wald_groups", default=None,
+        help="Groups of fitted cell features to test jointly with Wald tests from the fitted posterior, without "
+             "refits; same syntax as --LRTgroups (columns <id>+<id>_pval_wald_group, _FDR_wald_group)")
+    group4.add_option("--scoreGroups", dest="score_groups", default=None,
+        help="Groups of --scoreFile columns to score-test jointly; same syntax as --LRTgroups (columns "
+             "<id>+<id>_score_stat_group, _pval_score_group, _FDR_score_group in <out>.brie_score.tsv)")
     parser.add_option_group(group1)
     parser.add_option_group(group2)
     parser.add_option_group(group3)
@@ -241,6 +264,19 @@ def main():
     if options.n_perm > 0 and LRT_index is not None and len(LRT_index) == 0:
         print("[BRIE2] Error: --nPerm needs tested features (--LRTindex).")
         sys.exit(1)
+    groups = {}
+    for flag, key in (("--LRTgroups", "LRT_groups"), ("--waldGroups", "wald_groups"), ("--scoreGroups", "score_groups")):
+        text = getattr(options, key)
+        if text is not None:
+            try:
+                groups[key] = [[int(k) for k in G.split(",")] for G in text.split(";")]
+            except ValueError:
+                print("[BRIE2] Error: %s needs ';'-separated groups of ','-separated column indices, got %r."
+                      % (flag, text))
+                sys.exit(1)
+    if "score_groups" in groups and options.score_file is None:
+        print("[BRIE2] Error: --scoreGroups needs --scoreFile.")
+        sys.exit(1)
 
     quant(options.in_file, options.cell_file, options.gene_file,
           options.out_file, LRT_index, options.layers.split(','),
@@ -249,7 +285,7 @@ def main():
           options.min_iter, options.max_iter, options.MC_size,
           options.batch_size, options.pseudo_count, options.test_base, options.seed,
           options.out_dir, options.resume, options.n_perm, options.wald,
-          **({} if options.score_file is None else dict(score_file=options.score_file)))
+          **({} if options.score_file is None else dict(score_file=options.score_file)), **groups)
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         if dist.is_initialized():

@@ -887,6 +887,31 @@ int score_plan(const brie_fit* f, int32_t model, int32_t n_cand, ScorePlan* p) {
   return BRIE_OK;
 }
 
+// Geometry of the cross-term pass of model m over n_pairs candidate pairs (brie_score.cuh): the posterior plan, the
+// pair block (as the Wald pass's), and the scratch: the partials, then the device copy of the pair table.
+struct CrossPlan : PosteriorPlan {
+  int pb, n_pblk;
+  size_t part_bytes, scratch_bytes;
+};
+
+int cross_plan(const brie_fit* f, int32_t model, int32_t n_pairs, CrossPlan* p) {
+  int rc = posterior_plan(f, model, "the score test", p);
+  if (rc) return rc;
+  if (n_pairs <= 0) return fail(BRIE_ERR_ARG, "n_pairs must be >= 1");
+  p->pb = n_pairs <= 4 ? 4 : (n_pairs <= 12 ? 12 : kWaldMaxPairs);
+  p->n_pblk = (int)ceil_div(n_pairs, p->pb);
+  if ((int64_t)p->n_tiles * p->n_pblk > 0x7fffffffLL) return fail(BRIE_ERR_UNSUPPORTED, "too many event tiles x pair blocks");
+  p->part_bytes = (size_t)p->n_chunks * n_pairs * f->d.ld * sizeof(double);
+  p->scratch_bytes = p->part_bytes + (size_t)ceil_div(2 * (int64_t)n_pairs * sizeof(int32_t), 8) * 8;
+  return BRIE_OK;
+}
+
+template <int PB>
+cudaError_t launch_cross(const CrossArgs& a, dim3 grid, cudaStream_t s) {
+  score_cross_kernel<PB><<<grid, kWaldCols * kWaldRowGroups, 0, s>>>(a);
+  return cudaGetLastError();
+}
+
 template <int PB>
 cudaError_t launch_wald(const WaldArgs& a, dim3 grid, cudaStream_t s) {
   wald_info_kernel<PB><<<grid, kWaldCols * kWaldRowGroups, 0, s>>>(a);
@@ -988,6 +1013,53 @@ int brie_fit_score_parts(brie_fit* f, int32_t model, const float* X, int32_t n_c
   const int64_t n_out = d.n_events * p.n_q;
   score_reduce_kernel<<<(unsigned)ceil_div(n_out, 256), 256, 0, s>>>(a.part, p.n_chunks, p.n_q, d.ld, d.n_events, n_cand,
                                                                      p.kt, U, A, B, Utheta);
+  BRIE_CUDA(cudaGetLastError());
+  f->launches += 2;
+  return BRIE_OK;
+}
+
+int brie_fit_score_cross_sizes(const brie_fit* f, int32_t model, int32_t n_pairs, size_t* scratch_bytes) {
+  if (!scratch_bytes) return fail(BRIE_ERR_ARG, "null argument");
+  CrossPlan p;
+  int rc = cross_plan(f, model, n_pairs, &p);
+  if (rc) return rc;
+  *scratch_bytes = p.scratch_bytes;
+  return BRIE_OK;
+}
+
+int brie_fit_score_cross(brie_fit* f, int32_t model, const float* X, int64_t ldx, const int32_t* pairs, int32_t n_pairs,
+                         double* out, void* scratch, void* stream) {
+  CrossPlan p;
+  int rc = cross_plan(f, model, n_pairs, &p);
+  if (rc) return rc;
+  if (!X || !pairs) return fail(BRIE_ERR_ARG, "X and pairs required");
+  if (ldx < 1) return fail(BRIE_ERR_ARG, "ldx must be >= 1");
+  for (int32_t i = 0; i < n_pairs; ++i)
+    if (pairs[2 * i] < 0 || pairs[2 * i] >= pairs[2 * i + 1] || pairs[2 * i + 1] >= ldx)
+      return fail(BRIE_ERR_ARG, "pair %d = (%d, %d) is not 0 <= j < j' < ldx = %lld", i, pairs[2 * i], pairs[2 * i + 1],
+                  (long long)ldx);
+  if (!aligned8(out) || !aligned8(scratch)) return fail(BRIE_ERR_ARG, "out and scratch must be non-null and 8-byte aligned");
+  const brie_fit_desc& d = f->d;
+  cudaStream_t s = (cudaStream_t)stream;
+  int32_t* table = (int32_t*)((char*)scratch + p.part_bytes);
+  BRIE_CUDA(cudaMemcpyAsync(table, pairs, 2 * (size_t)n_pairs * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  CrossArgs a;
+  memset(&a, 0, sizeof a);
+  a.Nc = d.n_cells; a.Ng = d.n_events; a.ld = d.ld;
+  a.Zs = f->buf.Z_std_log + model * d.n_cells * d.ld;
+  a.tau = f->buf.sigma_log + (int64_t)model * (d.cell_mode ? d.n_cells : d.ld);
+  a.cell_tau = d.cell_mode;
+  a.X = X; a.ldx = ldx; a.pairs = table; a.n_pairs = n_pairs;
+  a.rows_per_chunk = p.rows_per_chunk; a.n_tiles = p.n_tiles;
+  a.part = (double*)scratch;
+  const dim3 grid((unsigned)((int64_t)p.n_tiles * p.n_pblk), (unsigned)p.n_chunks);
+  switch (p.pb) {
+    case 4: BRIE_CUDA(launch_cross<4>(a, grid, s)); break;
+    case 12: BRIE_CUDA(launch_cross<12>(a, grid, s)); break;
+    default: BRIE_CUDA(launch_cross<kWaldMaxPairs>(a, grid, s)); break;
+  }
+  const int64_t n_out = d.n_events * n_pairs;
+  wald_reduce_kernel<<<(unsigned)ceil_div(n_out, 256), 256, 0, s>>>(a.part, p.n_chunks, n_pairs, d.ld, d.n_events, out);
   BRIE_CUDA(cudaGetLastError());
   f->launches += 2;
   return BRIE_OK;

@@ -197,4 +197,109 @@ __global__ void __launch_bounds__(256) score_reduce_kernel(const double* __restr
   else Ut[g * kt + q - 2 * J - nb] = s;
 }
 
+// Cross terms of the joint score test of a group of candidates (DESIGN §2.4): for a table of candidate pairs (j, j'),
+//   A_gjj' = sum_c w_cg x_cj x_cj'
+// with w_cg the Louis weight above.  The diagonal (j = j') is score_parts_kernel's A.
+//
+// score_cross_kernel: CTA = 32 events (one per lane) x one block of PB pairs x one chunk of cell rows (the Wald pass's
+// chunks).  Each staged batch of kWaldBatch rows has its pair products x_cj x_cj' in shared memory (float64, exact for
+// float32 inputs); warp r takes rows r, r + 8, ... of a batch, computes w_cg once per (row, event) and accumulates
+// in float64 registers.  The 8 warps' sums are added in warp order and the CTA writes one partial per (chunk, pair,
+// event); wald_reduce_kernel adds the chunks in chunk order.  No atomics: repeated calls, pair blocks, event chunks
+// and shards give the same bits.
+struct CrossArgs {
+  int64_t Nc, Ng, ld;
+  const float* Zs;      // (Nc, ld) Z_std_log of the model
+  const float* tau;     // sigma_log of the model: (ld) per event, or (Nc) per cell (cell_tau)
+  int cell_tau;
+  const float* X;       // (Nc, ldx) candidates
+  int64_t ldx;
+  const int32_t* pairs; // (n_pairs, 2) candidate columns, device
+  int n_pairs;
+  int64_t rows_per_chunk;
+  int n_tiles;
+  double* part;         // (n_chunks, n_pairs, ld)
+};
+
+template <int PB>
+__global__ void __launch_bounds__(kWaldCols * kWaldRowGroups) score_cross_kernel(const CrossArgs a) {
+  static_assert(PB % kWaldRedPairs == 0 && PB <= kWaldMaxPairs, "pair block");
+  __shared__ double s_buf[kWaldBatch * kWaldMaxPairs];   // staged pair products, then the reduction
+  __shared__ int s_col[2][PB];                            // candidate columns of the block's pairs (-1: none)
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int tile = blockIdx.x % a.n_tiles, pblk = blockIdx.x / a.n_tiles;
+  const int p0 = pblk * PB;
+  const int64_t g = (int64_t)tile * kWaldCols + lane;
+  const bool ev_ok = g < a.Ng;
+  const int64_t c0 = (int64_t)blockIdx.y * a.rows_per_chunk;
+  const int64_t c1 = min(c0 + a.rows_per_chunk, a.Nc);
+
+  if (threadIdx.x < PB) {
+    const int p = p0 + threadIdx.x;
+    s_col[0][threadIdx.x] = p < a.n_pairs ? a.pairs[2 * p] : -1;
+    s_col[1][threadIdx.x] = p < a.n_pairs ? a.pairs[2 * p + 1] : -1;
+  }
+
+  double tau_w = 0.0, scale_w = 0.0;   // per-event sigma: tau and exp(-2 tau) once
+  if (!a.cell_tau && ev_ok) {
+    tau_w = (double)a.tau[g];
+    scale_w = exp(-2.0 * tau_w);
+  }
+  double acc[PB];
+#pragma unroll
+  for (int p = 0; p < PB; ++p) acc[p] = 0.0;
+
+  for (int64_t r0 = c0; r0 < c1; r0 += kWaldBatch) {
+    __syncthreads();   // the previous batch is consumed (and s_col is written, first time round)
+    for (int i = threadIdx.x; i < kWaldBatch * PB; i += blockDim.x) {
+      const int r = i / PB, q = i % PB;
+      const int64_t c = r0 + r;
+      const int j = s_col[0][q], k = s_col[1][q];
+      double v = 0.0;
+      if (c < c1 && j >= 0) {
+        const float* x = a.X + c * a.ldx;
+        v = (double)x[j] * (double)x[k];
+      }
+      s_buf[r * PB + q] = v;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int jj = 0; jj < kWaldBatch / kWaldRowGroups; ++jj) {
+      const int r = warp + jj * kWaldRowGroups;
+      const int64_t c = r0 + r;
+      double w = 0.0;
+      if (c < c1 && ev_ok) {
+        const double lam = (double)a.Zs[c * a.ld + g];
+        double tau = tau_w, scale = scale_w;
+        if (a.cell_tau) {
+          tau = (double)a.tau[c];
+          scale = exp(-2.0 * tau);
+        }
+        w = fmax(-expm1(2.0 * (lam - tau)), 0.0) * scale;
+      }
+#pragma unroll
+      for (int p = 0; p < PB; ++p) acc[p] = fma(w, s_buf[r * PB + p], acc[p]);
+    }
+  }
+
+  // warps 0..7 added in order; kWaldRedPairs pairs per round
+  const int64_t plane = (int64_t)a.n_pairs * a.ld;
+  double* out = a.part + (int64_t)blockIdx.y * plane;
+#pragma unroll
+  for (int q0 = 0; q0 < PB; q0 += kWaldRedPairs) {
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < kWaldRedPairs; ++i) s_buf[(warp * kWaldRedPairs + i) * kWaldCols + lane] = acc[q0 + i];
+    __syncthreads();
+    if (threadIdx.x < kWaldRedPairs * kWaldCols) {
+      const int i = threadIdx.x / kWaldCols, e = threadIdx.x % kWaldCols;
+      const int p = p0 + q0 + i;
+      const int64_t ge = (int64_t)tile * kWaldCols + e;
+      double s = 0.0;
+      for (int wp = 0; wp < kWaldRowGroups; ++wp) s += s_buf[(wp * kWaldRedPairs + i) * kWaldCols + e];
+      if (p < a.n_pairs && ge < a.Ng) out[(int64_t)p * a.ld + ge] = s;
+    }
+  }
+}
+
 }  // namespace brie

@@ -177,6 +177,106 @@ def score_from_parts(parts, info):
     return z, eff, pval
 
 
+def _quad_form(M, v, tol):
+    """v^T M^-1 v per event for a batch of symmetric k x k matrices M (n, k, k) and vectors v (n, k), or NaN where M
+    is not positive definite after rescaling to a unit diagonal with reciprocal condition number above `tol`."""
+    n, k = v.shape
+    out = np.full(n, np.nan)
+    with np.errstate(invalid='ignore'):
+        d = np.sqrt(np.diagonal(M, axis1=1, axis2=2))
+    ok = np.all(np.isfinite(M), axis=(1, 2)) & np.all(d > 0, axis=1) & np.all(np.isfinite(v), axis=1)
+    idx = np.flatnonzero(ok)
+    if idx.size:
+        dd = d[idx]
+        R = M[idx] / dd[:, :, None] / dd[:, None, :]
+        ev = np.linalg.eigvalsh(R)
+        good = ev[:, 0] > tol * ev[:, -1]
+        idx, R, dd = idx[good], R[good], dd[good]
+        if idx.size:
+            y = np.linalg.solve(np.linalg.cholesky(R), (v[idx] / dd)[:, :, None])[:, :, 0]
+            out[idx] = (y ** 2).sum(axis=1)
+    return out
+
+
+def wald_groups_from_info(coef, info, groups):
+    """Joint Wald tests that all coefficients of a group are 0 (DESIGN §2.4): per event and group G of columns of
+    `coef` (Ng, K), stat = beta_G^T ((I^-1)_GG)^-1 beta_G with `info` (Ng, K, K), df = |G|.  An event whose
+    information fails wald_from_info's checks gets stat NaN and pval 1.  Returns (stat, pval), each (Ng, H) float64."""
+    from scipy.stats import chi2
+    coef = np.asarray(coef, np.float64)
+    info = np.asarray(info, np.float64)
+    Ng, K = coef.shape
+    stat, pval = np.full((Ng, len(groups)), np.nan), np.ones((Ng, len(groups)))
+    if Ng == 0 or K == 0:
+        return stat, pval
+    _, d, idx, L = _pd_factor(info)
+    if idx.size:
+        Linv = np.linalg.solve(L, np.broadcast_to(np.eye(K), L.shape))   # R^-1 = Linv^T Linv, R = info / d d^T
+        for h, G in enumerate(groups):
+            G = list(G)
+            S = np.einsum('nki,nkj->nij', Linv[:, :, G], Linv[:, :, G])   # (R^-1)_GG
+            stat[idx, h] = _quad_form(S, coef[idx][:, G] * d[idx][:, G], 0.0)
+    for h, G in enumerate(groups):
+        ok = np.isfinite(stat[:, h])
+        pval[ok, h] = chi2.sf(stat[ok, h], df=len(G))
+    return stat, pval
+
+
+def group_pairs(groups):
+    """(n_pairs, 2) int32 table of the distinct off-diagonal candidate pairs (j < j') of the groups, sorted: the pairs
+    whose cross terms FitEngine.score_cross computes."""
+    pairs = sorted({(min(a, b), max(a, b)) for G in groups for i, a in enumerate(G) for b in G[i + 1:]})
+    return np.array(pairs, np.int32).reshape(-1, 2)
+
+
+def score_groups_from_parts(parts, cross, pairs, info, groups):
+    """Joint score tests of groups of candidates (DESIGN §2.4) from their parts (FitEngine.score_parts: U, A, B, Ut),
+    the cross terms `cross` (Ng, n_pairs) of the pairs `pairs` (FitEngine.score_cross, group_pairs) and the null
+    model's information `info`: per group G of k candidates
+        V_GG = A_GG - B_G I^-1 B_G^T,   Ue_G = U_G - B_G I^-1 Ut,   stat = Ue_G^T V_GG^-1 Ue_G,   df = k.
+    An event whose information fails wald_from_info's checks, a member that fails score_from_parts' rule (A <= 0 or
+    V <= SCORE_VTOL * A: collinear with the fitted columns, or zero on every cell), and a V_GG whose unit-diagonal
+    rescaling has reciprocal condition number <= SCORE_VTOL (members collinear with each other) give stat NaN and
+    pval 1.  Returns (stat, pval), each (Ng, H) float64."""
+    from scipy.stats import chi2
+    U, A, B, Ut = (np.asarray(x, np.float64) for x in parts)
+    cross = np.asarray(cross, np.float64)
+    info = np.asarray(info, np.float64)
+    Ng = U.shape[0]
+    K = info.shape[1] if info.ndim == 3 else 0
+    col = {(int(a), int(b)): p for p, (a, b) in enumerate(np.asarray(pairs).reshape(-1, 2))}
+    ok = np.ones(Ng, bool)
+    Y = y = None
+    if K > 0 and Ng > 0:
+        ok, d, idx, L = _pd_factor(info)
+        dfull = np.where(ok[:, None], d, 1.0)
+        Lfull = np.broadcast_to(np.eye(K), (Ng, K, K)).copy()
+        Lfull[idx] = L
+        Y = np.linalg.solve(Lfull, np.swapaxes(B / dfull[:, None, :], 1, 2))    # (Ng, K, J): L^-1 (B / d)^T
+        y = np.linalg.solve(Lfull, (Ut / dfull)[:, :, None])[:, :, 0]           # (Ng, K)
+    stat, pval = np.full((Ng, len(groups)), np.nan), np.ones((Ng, len(groups)))
+    for h, G in enumerate(groups):
+        G = [int(j) for j in G]
+        k = len(G)
+        V = np.empty((Ng, k, k))
+        for a, ja in enumerate(G):
+            V[:, a, a] = A[:, ja]
+            for b in range(a + 1, k):
+                V[:, a, b] = V[:, b, a] = cross[:, col[(min(ja, G[b]), max(ja, G[b]))]]
+        Ue = U[:, G].copy()
+        if Y is not None:
+            V -= np.einsum('nki,nkj->nij', Y[:, :, G], Y[:, :, G])
+            Ue -= np.einsum('nki,nk->ni', Y[:, :, G], y)
+        Ad, Vd = A[:, G], np.diagonal(V, axis1=1, axis2=2)
+        good = ok & np.all((Ad > 0) & (Vd > SCORE_VTOL * Ad), axis=1)
+        s = np.full(Ng, np.nan)
+        s[good] = _quad_form(V[good], Ue[good], SCORE_VTOL)
+        stat[:, h] = s
+        fin = np.isfinite(s)
+        pval[fin, h] = chi2.sf(s[fin], df=k)
+    return stat, pval
+
+
 class FitEngine:
     """Device-resident batched fit.
 
@@ -605,10 +705,7 @@ class FitEngine:
         posterior (brie_fit_score_parts; DESIGN §2.3): (U, A (Ng, J), B (Ng, J, K~), Ut (Ng, K~)) float64 host arrays,
         x~ as in wald_info.  The candidates go in blocks whose device scratch and outputs stay within
         SCORE_BLOCK_BYTES (the scratch alone is up to 64 row chunks x J (K~ + 2) x ld doubles)."""
-        X = torch.as_tensor(np.asarray(X, np.float32) if not torch.is_tensor(X) else X)
-        X = X.to(device=self.device, dtype=torch.float32).contiguous()
-        if X.dim() != 2 or X.shape[0] != self.Nc or X.shape[1] < 1:
-            raise ValueError("brie_b200: score candidates must be (%d, J >= 1), got %s" % (self.Nc, tuple(X.shape)))
+        X = self._device_candidates(X)
         J = X.shape[1]
         nbytes, c_kt = C.c_size_t(), C.c_int32()
 
@@ -638,6 +735,44 @@ class FitEngine:
                 Ut = T.cpu().numpy()
             del U, A, B, T, scratch
         return out_U, out_A, out_B, Ut
+
+    def _device_candidates(self, X):
+        X = torch.as_tensor(np.asarray(X, np.float32) if not torch.is_tensor(X) else X)
+        X = X.to(device=self.device, dtype=torch.float32).contiguous()
+        if X.dim() != 2 or X.shape[0] != self.Nc or X.shape[1] < 1:
+            raise ValueError("brie_b200: score candidates must be (%d, J >= 1), got %s" % (self.Nc, tuple(X.shape)))
+        return X
+
+    def score_cross(self, m, X, pairs):
+        """Cross terms sum_c w_cg x_cj x_cj' of candidate pairs `pairs` ((n_pairs, 2), j < j' < J) of X (Nc, J)
+        against model m's fitted posterior (brie_fit_score_cross; DESIGN §2.4): (Ng, n_pairs) float64 host array.
+        X may be the device tensor score_parts read (nothing is uploaded again).  The pairs go in blocks whose device
+        scratch and output stay within SCORE_BLOCK_BYTES."""
+        X = self._device_candidates(X)
+        pairs = np.ascontiguousarray(np.asarray(pairs, np.int32).reshape(-1, 2))
+        P = pairs.shape[0]
+        out = np.empty((self.Ng, P))
+        if P == 0:
+            return out
+        nbytes = C.c_size_t()
+
+        def scratch_of(n):
+            _lib.check(self.lib.brie_fit_score_cross_sizes(self.h, int(m), int(n), C.byref(nbytes)))
+            return int(nbytes.value)
+        per_pair = scratch_of(2) - scratch_of(1) + 8 * self.Ng           # the scratch grows linearly in n_pairs
+        pb = int(max(1, min(P, SCORE_BLOCK_BYTES // per_pair)))
+        for p0 in range(0, P, pb):
+            n = min(pb, P - p0)
+            res = torch.empty((self.Ng, n), dtype=torch.float64, device=self.device)
+            scratch = torch.empty(scratch_of(n), dtype=torch.uint8, device=self.device)
+            blk = pairs[p0:p0 + n]
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.brie_fit_score_cross(self.h, int(m), X.data_ptr(), int(X.shape[1]),
+                                                         blk.ctypes.data, int(n), res.data_ptr(), scratch.data_ptr(),
+                                                         self._stream()))
+            out[:, p0:p0 + n] = res.cpu().numpy()
+            del res, scratch
+        return out
 
     # ------------------------------------------------------------------ schedule
     def fit(self, min_iter=1000, max_iter=5000, add_iter=500, epsilon_conv=1e-2, n_eval=500,

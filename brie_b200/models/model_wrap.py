@@ -13,7 +13,8 @@ import time
 import numpy as np
 from scipy.stats import chi2
 
-from ..engine import SCORE_BLOCK_BYTES, FitEngine, score_from_parts, wald_from_info
+from ..engine import (SCORE_BLOCK_BYTES, FitEngine, group_pairs, score_from_parts, score_groups_from_parts,
+                      wald_from_info, wald_groups_from_info)
 from ..sharding import event_shards
 from ..utils.layer_store import LayerStore, BIG_KEYS
 from ..settings import verbosity
@@ -88,6 +89,113 @@ def check_n_perm(n_perm, n_tests):
     return n_perm
 
 
+def check_groups(groups, n_cols, name):
+    """Validate `groups` (before any device work): None, or a non-empty list of groups, each a non-empty list of
+    distinct integer column indices in [0, n_cols).  Returned as lists of int."""
+    if groups is None:
+        return None
+    try:
+        groups = [list(G) for G in groups]
+    except TypeError:
+        raise ValueError("%s must be a list of groups of column indices, got %r" % (name, groups)) from None
+    if not groups:
+        raise ValueError("%s must hold at least one group" % name)
+    for G in groups:
+        if not G:
+            raise ValueError("%s: a group is empty" % name)
+        for k in G:
+            if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)):
+                raise ValueError("%s: column index %r is not an integer" % (name, k))
+            if not 0 <= k < n_cols:
+                raise ValueError("%s: column index %d is out of range for %d columns" % (name, k, n_cols))
+        if len(set(int(k) for k in G)) != len(G):
+            raise ValueError("%s: group %r repeats a column index" % (name, [int(k) for k in G]))
+    return [[int(k) for k in G] for G in groups]
+
+
+def _base_columns(Kc, LRT_index, full):
+    """Columns of model 0 (model_wrap.py:130-136): all of Xc in base_mode 'full', else those not tested."""
+    if full:
+        return list(range(Kc))
+    if LRT_index is not None and len(LRT_index) < Kc:
+        return [k for k in range(Kc) if k not in set(int(i) for i in LRT_index)]
+    return []
+
+
+def group_model_id(i, n_tests, n_perm):
+    """RNG model word of the refit of LRT group i: after the base model, the LRT refits and the permuted models."""
+    return 1 + n_tests * (1 + n_perm) + i
+
+
+def check_LRT_groups(groups, Kc, base_cols, full, n_tests, n_perm):
+    """Validate `LRT_groups` (before any device work): groups of Xc columns; with base_mode 'null' a group is added to
+    the base model and must not overlap its columns; every group model needs a model id of the noise stream."""
+    groups = check_groups(groups, Kc, "LRT_groups")
+    if groups is None:
+        return None
+    if not full:
+        for G in groups:
+            if set(G) & set(base_cols):
+                raise ValueError("LRT_groups: group %r overlaps the base model's columns %r (base_mode 'null' adds "
+                                 "the group to the base model)" % (G, base_cols))
+    n_ids = group_model_id(len(groups), n_tests, n_perm)
+    if n_ids > MAX_MODEL_IDS:
+        raise ValueError("LRT_groups: %d groups with %d tested covariates and n_perm = %d need %d model ids; the noise "
+                         "stream has %d" % (len(groups), n_tests, n_perm, n_ids, MAX_MODEL_IDS))
+    return groups
+
+
+def check_wald_groups(groups, Kc, base_cols, target):
+    """Validate `wald_groups` (before any device work): groups of the columns model 0 fits (any Xc column in
+    base_mode 'full', the base columns in 'null'); a marginLik fit trains no posterior."""
+    if groups is None:
+        return None
+    if target == "marginLik":
+        raise ValueError("wald_groups needs target 'ELBO': a marginLik fit has no trained posterior")
+    groups = check_groups(groups, Kc, "wald_groups")
+    for G in groups:
+        if not set(G) <= set(base_cols):
+            raise ValueError("wald_groups: group %r has columns model 0 does not fit (its columns: %r)" % (G, base_cols))
+    return groups
+
+
+def check_score_groups(groups, score_X, target):
+    """Validate `score_groups` (before any device work): groups of columns of the (validated) score_X."""
+    if groups is None:
+        return None
+    if target == "marginLik":
+        raise ValueError("score_groups needs target 'ELBO': a marginLik fit has no trained posterior")
+    if score_X is None:
+        raise ValueError("score_groups needs score_X: a group is a group of score_X columns")
+    return check_groups(groups, score_X.shape[1], "score_groups")
+
+
+# (statistic or gain, p-value, FDR) of each kind of joint test of a group, each (Ng, groups)
+GROUP_KEYS = (('ELBO_gain_group', 'pval_group', 'fdr_group'),
+              ('wald_stat_group', 'pval_wald_group', 'fdr_wald_group'),
+              ('score_stat_group', 'pval_score_group', 'fdr_score_group'))
+
+
+def _set_fdr_groups(res):
+    """fdr_group / fdr_wald_group / fdr_score_group: BH over all events of the result, per group (the pooled scope
+    of fdr_wald), for each kind of group test the result holds."""
+    for _, pk, fk in GROUP_KEYS:
+        if hasattr(res, pk):
+            p = getattr(res, pk)
+            fdr = np.zeros(p.shape)
+            for i in range(p.shape[1]):
+                fdr[:, i] = fdr_bh(p[:, i])
+            setattr(res, fk, fdr)
+
+
+def _append_groups(out, r):
+    """Event-axis concatenation of the group-test outputs of two results (the FDRs are recomputed over all events)."""
+    for keys in GROUP_KEYS:
+        if hasattr(r, keys[1]):
+            for k in keys:
+                setattr(out, k, np.append(getattr(out, k), getattr(r, k), axis=0))
+
+
 def perm_pvalue(gain, gain_perm):
     """Pooled empirical p-values (Ng, T) of the observed gains `gain` (Ng, T) against the permutation null
     `gain_perm` (Ng, T, B) of every event: (1 + #{(g', b) : gain_perm[g', t, b] >= gain[g, t]}) / (1 + Ng * B).
@@ -121,16 +229,22 @@ def check_wald(wald, target):
     return wald
 
 
-def _wald_of_model(eng, j):
-    """(se, pval, width) of model j of a fitted engine: Wald statistics of its Wc rows, then of its intercept when
-    that is per-event and trained, from the observed information of its posterior (FitEngine.wald_info)."""
+def _coef_and_info(eng, j):
+    """(coef (Ng, K~), info (Ng, K~, K~)) of model j of a fitted engine: its Wc rows, then its intercept when that is
+    per-event and trained, and their observed information from its posterior (FitEngine.wald_info)."""
     import torch
     w = len(eng.masks[j])
     coef = [eng.Wc[j, :w, :eng.Ng].T.double()]
     if not eng.cell_mode and eng.intercept_const is None:
         coef.append(eng.intercept[j, :eng.Ng, None].double())
-    se, pval = wald_from_info(torch.cat(coef, dim=1).cpu().numpy(), eng.wald_info(j))
-    return se, pval, w
+    return torch.cat(coef, dim=1).cpu().numpy(), eng.wald_info(j)
+
+
+def _wald_of_model(eng, j):
+    """(se, pval, width) of model j of a fitted engine: Wald statistics of its Wc rows, then of its intercept when
+    that is per-event and trained (_coef_and_info)."""
+    se, pval = wald_from_info(*_coef_and_info(eng, j))
+    return se, pval, len(eng.masks[j])
 
 
 def _set_fdr_wald(res):
@@ -176,10 +290,19 @@ def check_score_X(score_X, target, Nc):
     return X
 
 
-def _score_of_model(eng, j, X):
-    """(score_z, score_effect, pval_score) of candidates X against model j of a fitted engine as the null model
-    (FitEngine.score_parts with the model's information, score_from_parts)."""
-    return score_from_parts(eng.score_parts(j, X), eng.wald_info(j))
+def _score_of_model(eng, j, X, groups=None):
+    """((score_z, score_effect, pval_score), group tests) of candidates X against model j of a fitted engine as the
+    null model (FitEngine.score_parts with the model's information, score_from_parts).  With `groups`, the group
+    tests are the joint tests (score_stat_group, pval_score_group) of those groups of candidates
+    (FitEngine.score_cross, score_groups_from_parts), else None.  X goes to the device once for both passes."""
+    import torch
+    X = torch.from_numpy(np.ascontiguousarray(X, np.float32)).to(eng.device)
+    parts, info = eng.score_parts(j, X), eng.wald_info(j)
+    single = score_from_parts(parts, info)
+    if groups is None:
+        return single, None
+    pairs = group_pairs(groups)
+    return single, score_groups_from_parts(parts, eng.score_cross(j, X, pairs), pairs, info, groups)
 
 
 def _set_fdr_score(res):
@@ -262,6 +385,7 @@ class BRIE_RV():
             _append_wald(self, new_RV)
         if hasattr(new_RV, 'pval_score'):
             _append_score(self, new_RV)
+        _append_groups(self, new_RV)
         if hasattr(new_RV, 'n_iter'):
             self.n_iter = np.append(self.n_iter, new_RV.n_iter, axis=1)
         if getattr(self, 'timing', None) is not None and getattr(new_RV, 'timing', None) is not None:
@@ -347,7 +471,7 @@ def _host_pseudo_count_inplace(data, pseudo_count):
 
 
 def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=None, n_perm=0, tested=(),
-                 n_cols=0, full=True):
+                 n_cols=0, full=True, group_masks=()):
     """[(column masks, model ids, intercept mode)] per FitEngine: the base model (id 0) with as many LRT refits
     (ids 1..T) as one launch batches, the remaining refits in further engines of at most `max_models` models; a
     cell-mode base model sits alone, because the reference's refits always use the per-event layout
@@ -359,7 +483,11 @@ def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=No
     of fitBRIE holds).  Model (t, b) is the observed alternative of test t -- the full model (base_mode
     'full', base layout) or test model t (base_mode 'null', per-event layout) -- with column tested[t] replaced
     in place by column n_cols + j of the engine's design, j its position in the engine; its id is
-    perm_model_id(t, b, T, B)."""
+    perm_model_id(t, b, T, B).
+
+    The refits of LRT groups (`group_masks`, one column mask per group) follow the permuted models in further
+    engines under the same size rule, in the per-event layout of the LRT refits; group i has id
+    group_model_id(i, T, B)."""
     if max_models is None:
         from .._lib import BRIE_MAX_MODELS as max_models
     T = len(test_masks)
@@ -373,20 +501,25 @@ def _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, max_models=No
     for t0 in range(first_tests, T, max_models):
         t1 = min(t0 + max_models, T)
         plan.append((test_masks[t0:t1], list(range(1 + t0, 1 + t1)), 'gene'))
+    size = min(max(len(ids) for _, ids, _ in plan), max_models)
     if n_perm > 0:
-        size = min(max(len(ids) for _, ids, _ in plan), max_models)
         perm = [(t, b) for t in range(T) for b in range(n_perm)]
         for p0 in range(0, len(perm), size):
             part = perm[p0:p0 + size]
             masks = [[n_cols + j if k == tested[t] else k for k in (base_cols if full else test_masks[t])]
                      for j, (t, b) in enumerate(part)]
             plan.append((masks, [perm_model_id(t, b, T, n_perm) for t, b in part], intercept_mode if full else 'gene'))
+    for g0 in range(0, len(group_masks), size):
+        g1 = min(g0 + size, len(group_masks))
+        plan.append(([list(m) for m in group_masks[g0:g1]], [group_model_id(i, T, n_perm) for i in range(g0, g1)],
+                     'gene'))
     return plan
 
 
 def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
                     intercept_mode='gene', LRT_index=None, pseudo_count=0.01,
-                    sigma=None, base_mode='full', tau_prior=[3, 27], score_X=None, **keyargs):
+                    sigma=None, base_mode='full', tau_prior=[3, 27], score_X=None, LRT_groups=None,
+                    wald_groups=None, score_groups=None, **keyargs):
     """Fit a BRIE model with cell and/or gene features (model_wrap.py:88-199).
 
     Extra keyword arguments consumed here (not in the reference): `seed` (noise and
@@ -418,6 +551,17 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     and `fdr_score` (BH per candidate over all events), each (Ng, J).  A candidate collinear with the fitted columns
     or zero on every cell, and an event whose information is not positive definite, get NaN and pval 1.  Every
     other output is unchanged.
+
+    Joint tests of groups of columns (DESIGN §2.4; a group is a list of distinct 0-based column indices, each input a
+    list of groups; at None nothing changes):
+    `LRT_groups` refits, per group, the full model without the group's columns (base_mode 'null': the base model plus
+    the group's columns, which must not overlap it), in the per-event layout of the LRT refits, and returns
+    `ELBO_gain_group` (Ng, G), `pval_group` = chi2.sf(2 gain, df=len(group)) and `fdr_group` (BH over all events).
+    Group refits only evaluate `loss_gene`.
+    `wald_groups`, groups of model 0's columns, returns the joint Wald statistic beta_G^T ((I^-1)_GG)^-1 beta_G from
+    model 0's information (no refit; also without `wald`): `wald_stat_group`, `pval_wald_group`, `fdr_wald_group`.
+    `score_groups`, groups of score_X columns, returns their joint score statistics against model 0:
+    `score_stat_group`, `pval_score_group`, `fdr_score_group`.  An undefined statistic is NaN with p-value 1.
     """
     from scipy.sparse import issparse
     seed = keyargs.pop('seed', 0)
@@ -436,6 +580,12 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     n_perm = check_n_perm(keyargs.pop('n_perm', 0), n_tests)
     wald = check_wald(keyargs.pop('wald', False), target)
     score_X = check_score_X(score_X, target, data[0].shape[0])
+    full = base_mode.upper() == 'FULL'
+    Kc = 0 if Xc is None else np.shape(Xc)[1]
+    base_cols = _base_columns(Kc, LRT_index, full)
+    LRT_groups = check_LRT_groups(LRT_groups, Kc, base_cols, full, n_tests, n_perm)
+    wald_groups = check_wald_groups(wald_groups, Kc, base_cols, target)
+    score_groups = check_score_groups(score_groups, score_X, target)
     for k in ('optimizer', 'learn_rate', 'verbose'):                # accepted and ignored (:214-237)
         keyargs.pop(k, None)
 
@@ -479,15 +629,6 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
         Xg = np.ones((Ng, 0), np.float32)
     Xc = np.asarray(Xc, np.float32)
     Xg = np.asarray(Xg, np.float32)
-    Kc = Xc.shape[1]
-
-    full = base_mode.upper() == 'FULL'
-    if full:                                                        # :130-136
-        base_cols = list(range(Kc))
-    elif LRT_index is not None and len(LRT_index) < Kc:
-        base_cols = [k for k in range(Kc) if k not in set(int(i) for i in LRT_index)]
-    else:
-        base_cols = []
     if LRT_index is None:                                           # :149-150
         LRT_index = np.arange(Kc)
     LRT_index = [int(i) for i in LRT_index]
@@ -517,22 +658,25 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     # that runs the remaining refits in further engines, one after the other, over the same device tiles.
     # NB the reference builds the refits WITHOUT intercept_mode (model_wrap.py:174-178), so they always use
     # the default per-event ('gene') intercept/sigma layout: a cell-mode base model gets an engine of its own.
+    group_masks = [[k for k in range(Kc) if k not in G] if full else base_cols + G for G in (LRT_groups or [])]
+    first_group = group_model_id(0, T, n_perm)
     plan = _engine_plan(base_cols, test_masks, cell_mode, intercept_mode, n_perm=n_perm, tested=LRT_index,
-                        n_cols=Kc, full=full)
+                        n_cols=Kc, full=full, group_masks=group_masks)
     t_ph = _tick("engine_setup", t_ph)
 
     brie_results = None
     n_iter_rows, lg_tests, wc_last, launches = [None] * (T + 1), [None] * T, [None] * T, 0
     lg_perm = {}                                                    # (t, b) -> loss_gene of permuted model (t, b)
+    lg_group = {}                                                   # i -> loss_gene of the refit of LRT group i
     wald_out = {}                                                   # model id -> _wald_of_model (base, null-mode tests)
     codes = None                                                    # the chunk's packed count codes, encoded once
     for masks_e, ids_e, mode_e in plan:
         io, kw_e = None, common
-        if ids_e[0] > T:                                            # permuted models: their columns appended to Xc
+        if T < ids_e[0] < first_group:                              # permuted models: their columns appended to Xc
             tb = [divmod(mid - 1 - T, n_perm) for mid in ids_e]
             cols = [Xc[perm_indices(seed, t, b, Nc), LRT_index[t]] for t, b in tb]
             kw_e = dict(common, Xc=np.concatenate([Xc, np.stack(cols, axis=1)], axis=1))
-        elif init_objs is not None:
+        elif init_objs is not None and ids_e[0] < first_group:
             io = [init_objs[i] for i in ids_e]
         eng = FitEngine(data, masks=masks_e, model_ids=ids_e, intercept_mode=mode_e, count_codes=codes, **kw_e)
         codes = eng.count_codes
@@ -542,14 +686,20 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
             for k, v in eng.phase_s.items():
                 timing[k] = timing.get(k, 0.0) + v
         for j, mid in enumerate(ids_e):
+            if mid >= first_group:
+                lg_group[mid - first_group] = eng.loss_gene[j].cpu().numpy()
+                continue
             if mid > T:
                 lg_perm[divmod(mid - 1 - T, n_perm)] = eng.loss_gene[j].cpu().numpy()
                 continue
             n_iter_rows[mid] = eng.n_iter[j]
             if wald and (mid == 0 or not full):
                 wald_out[mid] = _wald_of_model(eng, j)
+            if wald_groups is not None and mid == 0:            # positions of the groups' columns in model 0
+                wald_group_out = wald_groups_from_info(*_coef_and_info(eng, j),
+                                                       [[base_cols.index(k) for k in G] for G in wald_groups])
             if score_X is not None and mid == 0:
-                score_out = _score_of_model(eng, j, score_X)
+                score_out, score_group_out = _score_of_model(eng, j, score_X, score_groups)
             if mid == 0:
                 brie_results = _rv_from_engine(eng, j, Xc[:, base_cols], Xg, intercept_mode, out_sink)   # :146
             else:
@@ -568,6 +718,18 @@ def fit_BRIE_matrix(data, Xc=None, Xg=None, effLen=None, intercept=None,
     if score_X is not None:
         brie_results.score_z, brie_results.score_effect, brie_results.pval_score = score_out
         _set_fdr_score(brie_results)
+    if LRT_groups is not None:
+        gain = np.zeros((Ng, len(LRT_groups)), dtype=np.float32)
+        pval = np.zeros((Ng, len(LRT_groups)))
+        for i, G in enumerate(LRT_groups):
+            gain[:, i] = lg_group[i] - brie_results.loss_gene if full else brie_results.loss_gene - lg_group[i]
+            pval[:, i] = chi2.sf(2 * gain[:, i], df=len(G))
+        brie_results.ELBO_gain_group, brie_results.pval_group = gain, pval
+    if wald_groups is not None:
+        brie_results.wald_stat_group, brie_results.pval_wald_group = wald_group_out
+    if score_groups is not None:
+        brie_results.score_stat_group, brie_results.pval_score_group = score_group_out
+    _set_fdr_groups(brie_results)
     if T == 0:                                                      # :152-153
         return brie_results
 
@@ -625,6 +787,7 @@ def _merge_shared(parts):
             _append_wald(out, r)
         if hasattr(r, 'pval_score'):
             _append_score(out, r)
+        _append_groups(out, r)
     out.shape = (out.Nc, out.Ng)
     if hasattr(out, 'pval'):               # one fit => one multiple-testing scope over all events
         for i in range(out.fdr.shape[1]):
@@ -668,7 +831,8 @@ def _device_event_budget(Nc, n_models, n_layers, device=None, frac=0.7, reserve=
 def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             LRT_index=[], layer_keys=['isoform1', 'isoform2', 'ambiguous'],
             batch_size=500000, pseudo_count=0.01, sigma=None,
-            base_mode='full', tau_prior=[3, 27], score_X=None, **keyargs):
+            base_mode='full', tau_prior=[3, 27], score_X=None, LRT_groups=None, wald_groups=None,
+            score_groups=None, **keyargs):
     """Fit a BRIE model from AnnData with cell and/or gene features (model_wrap.py:202-314).
 
     `out_dir` (not in the reference): directory for `.npy` memory maps of the dense
@@ -688,6 +852,11 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     `score_X` (not in the reference, default None): (Nc, J) candidate cell covariates aligned with adata's cells,
     score-tested from the fitted posterior, see fit_BRIE_matrix; stored as varm['score_z', 'score_effect',
     'pval_score', 'fdr_score'] (Ng, J) with uns['brie_param']['score'] = J; fdr_score is BH over all events of the fit.
+    `LRT_groups`, `wald_groups`, `score_groups` (not in the reference, default None): joint tests of groups of
+    columns, see fit_BRIE_matrix; stored as varm['ELBO_gain_group', 'pval_group', 'fdr_group'],
+    varm['wald_stat_group', 'pval_wald_group', 'fdr_wald_group'] and varm['score_stat_group', 'pval_score_group',
+    'fdr_score_group'] with the groups in uns['brie_param']['LRT_groups' / 'wald_groups' / 'score_groups']; each FDR
+    is BH over all events of the fit.
 
     Returns the BRIE_RV result and adds to `adata` exactly the keys the reference adds
     (obsm['Xc'], varm['cell_coeff'], varm['Xg'], obsm['gene_coeff'], varm|obsm['intercept',
@@ -709,6 +878,12 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     if wald:                               # (likewise absent when False)
         keyargs['wald'] = True
     score_X = check_score_X(score_X, keyargs.get('target', "ELBO"), Nc)
+    full = base_mode.upper() == 'FULL'
+    base_cols = _base_columns(Xc.shape[1], LRT_index, full)
+    LRT_groups = check_LRT_groups(LRT_groups, Xc.shape[1], base_cols, full, len(LRT_index), n_perm)
+    wald_groups = check_wald_groups(wald_groups, Xc.shape[1], base_cols, keyargs.get('target', "ELBO"))
+    score_groups = check_score_groups(score_groups, score_X, keyargs.get('target', "ELBO"))
+    groups = dict(LRT_groups=LRT_groups, wald_groups=wald_groups, score_groups=score_groups)
     out_dir = keyargs.pop('out_dir', None)
     resume = keyargs.pop('resume', False)
     out_keys = tuple(keyargs.pop('out_keys', None) or BIG_KEYS)
@@ -729,6 +904,8 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
                                    pseudo_count, sigma, base_mode, keyargs) if out_dir is not None else None
         if signature is not None and score_X is not None:     # (absent without score_X)
             signature['score_X_sha1'] = hashlib.sha1(score_X.tobytes()).hexdigest()
+        if signature is not None:                             # (each absent when None)
+            signature.update({k: v for k, v in groups.items() if v is not None})
         store = LayerStore(Nc, Ng, out_dir, rank, world, dist, keys=out_keys, signature=signature, resume=resume)
         res_list = []
         pending = None                     # (sink, result) of the chunk whose layers are still on their way to the host
@@ -763,7 +940,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
                     LRT_index=LRT_index, pseudo_count=pseudo_count, sigma=sigma,
                     base_mode=base_mode, tau_prior=tau_prior, group_size=_n_gene,
                     event_offset=e0, n_events_total=Ng, host_side_effect=False, out_sink=_sink, score_X=score_X,
-                    **keyargs)
+                    **groups, **keyargs)
             finally:
                 _land()
             pending = (_sink, _ResVal)
@@ -797,7 +974,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             pseudo_count=pseudo_count, sigma=sigma, base_mode=base_mode,
             tau_prior=tau_prior, event_offset=lo, n_events_total=Ng,
             dist_group=dist.group.WORLD, out_sink=_ChunkSink(store, lo, background=False), score_X=score_X,
-            **keyargs)
+            **groups, **keyargs)
         store.put(lo, local, checkpoint=False)
         parts = [None] * world
         dist.all_gather_object(parts, local)
@@ -811,7 +988,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
             _count_layers, Xc=Xc, Xg=Xg, effLen=_effLen, intercept=intercept,
             intercept_mode=intercept_mode, LRT_index=LRT_index,
             pseudo_count=pseudo_count, sigma=sigma, base_mode=base_mode,
-            tau_prior=tau_prior, score_X=score_X, **keyargs)
+            tau_prior=tau_prior, score_X=score_X, **groups, **keyargs)
 
     if n_perm > 0:                         # one pooled null over every event of the fit, the same on every rank
         _set_perm_outputs(ResVal)
@@ -819,6 +996,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         _set_fdr_wald(ResVal)
     if score_X is not None:                # likewise
         _set_fdr_score(ResVal)
+    _set_fdr_groups(ResVal)                # likewise, for each kind of group test
 
     # update adata (:271-311)
     if Xc.shape[0] > 0:
@@ -859,6 +1037,10 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
     if score_X is not None:
         for k in SCORE_KEYS:
             adata.varm[k] = getattr(ResVal, k)
+    for (name, g), keys in zip(groups.items(), GROUP_KEYS):
+        if g is not None:
+            for k in keys:
+                adata.varm[k] = getattr(ResVal, k)
 
     adata.uns['brie_param'] = {
         'LRT_index': LRT_index,
@@ -876,4 +1058,7 @@ def fitBRIE(adata, Xc=None, Xg=None, intercept=None, intercept_mode='gene',
         adata.uns['brie_param']['wald_columns'] = list(ResVal.wald_columns)
     if score_X is not None:
         adata.uns['brie_param']['score'] = int(score_X.shape[1])
+    for name, g in groups.items():
+        if g is not None:
+            adata.uns['brie_param'][name] = g
     return ResVal

@@ -96,15 +96,33 @@ def dump_results(adata):
             table[label + '_se'] = adata.varm['cell_coeff_se'][:, j]
             table[label + '_pval_wald'] = adata.varm['pval_wald'][:, j]
             table[label + '_FDR_wald'] = adata.varm['fdr_wald'][:, j]
+    param = adata.uns['brie_param'] if 'brie_param' in adata.uns else {}
+    label = lambda G: '+'.join(str(names[k]) if names is not None else 'X%d' % k for k in G)
+    if 'LRT_groups' in param:              # joint tests of groups of covariates, labelled <id>+<id>+..., after all others
+        for i, G in enumerate(param['LRT_groups']):
+            table[label(G) + '_ELBO_gain_group'] = adata.varm['ELBO_gain_group'][:, i]
+            table[label(G) + '_pval_group'] = adata.varm['pval_group'][:, i]
+            table[label(G) + '_FDR_group'] = adata.varm['fdr_group'][:, i]
+    if 'wald_groups' in param:
+        for i, G in enumerate(param['wald_groups']):
+            table[label(G) + '_pval_wald_group'] = adata.varm['pval_wald_group'][:, i]
+            table[label(G) + '_FDR_wald_group'] = adata.varm['fdr_wald_group'][:, i]
     return table
 
 
 def score_table(adata):
     """Per-event table of the score tests of candidate cell covariates (brie-quant --scoreFile), written as
-    <out>.brie_score.tsv: per candidate, in uns['score_ids'] order, <id>_score_z, <id>_pval_score, <id>_FDR_score."""
+    <out>.brie_score.tsv: per candidate, in uns['score_ids'] order, <id>_score_z, <id>_pval_score, <id>_FDR_score;
+    then per group of candidates (--scoreGroups) <id>+<id>..._score_stat_group, _pval_score_group, _FDR_score_group."""
     table = pd.DataFrame(index=adata.var.index)
     for j, cid in enumerate(adata.uns['score_ids']):
         table[str(cid) + '_score_z'] = adata.varm['score_z'][:, j]
         table[str(cid) + '_pval_score'] = adata.varm['pval_score'][:, j]
         table[str(cid) + '_FDR_score'] = adata.varm['fdr_score'][:, j]
+    ids = adata.uns['score_ids']
+    for i, G in enumerate(adata.uns['brie_param'].get('score_groups', [])):    # then per group of candidates
+        label = '+'.join(str(ids[j]) for j in G)
+        table[label + '_score_stat_group'] = adata.varm['score_stat_group'][:, i]
+        table[label + '_pval_score_group'] = adata.varm['pval_score_group'][:, i]
+        table[label + '_FDR_score_group'] = adata.varm['fdr_score_group'][:, i]
     return table

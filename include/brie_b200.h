@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define BRIE_ABI_VERSION 11
+#define BRIE_ABI_VERSION 12
 #define BRIE_MAX_MODELS 32
 #define BRIE_MAX_KC 16   /* widest design whose covariate contraction stays in registers / shared memory */
 #define BRIE_MAX_KG 8
@@ -261,6 +261,23 @@ int brie_fit_wald_info(brie_fit* fit, int32_t model, double* info, void* scratch
 int brie_fit_score_sizes(const brie_fit* fit, int32_t model, int32_t n_cand, size_t* scratch_bytes, int32_t* k_tilde);
 int brie_fit_score_parts(brie_fit* fit, int32_t model, const float* X, int32_t n_cand, int64_t ldx, double* U,
                          double* A, double* B, double* Utheta, void* scratch, void* stream);
+
+/* Cross terms of the joint score test of groups of candidates (DESIGN §2.4), from model `model`'s fitted posterior:
+ *   out[g, p] = sum_c w_cg x_c,j x_c,j'   for pair p = (j, j') = (pairs[2 p], pairs[2 p + 1])
+ * with w_cg the Louis weight of brie_fit_wald_info, in float64.  The pairs j = j' are brie_fit_score_parts' A; the
+ * joint efficient information of a group G is V_GG = A_GG - B_G I^-1 B_G^T.
+ *  brie_fit_score_cross_sizes : scratch bytes of `model` for n_pairs pairs (up to 64 row chunks x n_pairs x ld
+ *                               doubles, plus the pair table; callers split the pairs);
+ *  brie_fit_score_cross       : X (DEVICE, (n_cells, ldx) float32), pairs (HOST, (n_pairs, 2) int32, each
+ *                               0 <= j < j' < ldx, copied into the scratch with cudaMemcpyAsync on `stream`), out
+ *                               (DEVICE, (n_events, n_pairs) float64).  out and scratch 8-byte aligned.  The row chunks
+ *                               are the Wald pass's, a function of n_cells alone; no atomics: repeated calls, pair
+ *                               blocks, event chunks and shards give the same bits.
+ * Both refuse what brie_fit_score_parts refuses (a null or unbound fit, a model out of range, a gathered sub-fit,
+ * target marginLik) and n_pairs <= 0; brie_fit_score_cross also refuses pairs out of range, before any launch. */
+int brie_fit_score_cross_sizes(const brie_fit* fit, int32_t model, int32_t n_pairs, size_t* scratch_bytes);
+int brie_fit_score_cross(brie_fit* fit, int32_t model, const float* X, int64_t ldx, const int32_t* pairs,
+                         int32_t n_pairs, double* out, void* scratch, void* stream);
 
 /* Replaces the tensors the public model API returns for one model (BRIE2.logLik_MC model_TFProb.py:130-191,
  * Z_prior :118-127, the KL of get_loss :208), as dense (Nc, ld) arrays; any output may be NULL.
