@@ -48,6 +48,9 @@ struct brie_fit {
   bool subfit = false;       // bound as a gathered sub-fit (event_ids or a per-model count / length stride)
   int nev_max = 0, ncell = 0;
   size_t off_part_ev = 0, off_part_cell = 0, off_G = 0;  // scratch carve-up (float offsets)
+  // two-step passes (brie_fit_run_steps): statistic partials, the first step's parameters, float64 Gram sums
+  bool pairs = false;
+  size_t off_part_st = 0, off_prev = 0, off_gram = 0;
   size_t off_mom_cell = 0;   // adam_small: per-event moments (2, M, Kc + 2, ld) first, per-cell (2, M, Nc, Kg + 2) here
   bool stage_open = false;   // begin_stage has set the learning rate and cleared the Adam moments
   float lr = 0.f;
@@ -102,19 +105,20 @@ cudaError_t opt_in_smem(int bytes) {
   return e;
 }
 
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool CODE8>
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool CODE8, bool PAIR = false>
 cudaError_t launch_step(const StepArgs& a, dim3 grid, cudaStream_t s) {
-  constexpr int smem = step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8);
-  cudaError_t e = opt_in_smem<elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8>>(smem);
+  constexpr int smem = step_smem_bytes(KC, KG, CELL, LOSS, EXT, CODE8, PAIR);
+  cudaError_t e = opt_in_smem<elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8, PAIR>>(smem);
   if (e != cudaSuccess) return e;
-  elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8><<<grid, kThreads, smem, s>>>(a);
+  elbo_step_kernel<KC, KG, CELL, LOSS, EXT, CODE8, PAIR><<<grid, kThreads, smem, s>>>(a);
   return cudaGetLastError();
 }
 
 // the count form (f32 tiles or packed codes) is the innermost choice
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT>
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT, bool PAIR = false>
 cudaError_t launch_step_fmt(const StepArgs& a, dim3 grid, cudaStream_t s) {
-  return a.codes ? launch_step<KC, KG, CELL, LOSS, EXT, true>(a, grid, s) : launch_step<KC, KG, CELL, LOSS, EXT, false>(a, grid, s);
+  return a.codes ? launch_step<KC, KG, CELL, LOSS, EXT, true, PAIR>(a, grid, s)
+                 : launch_step<KC, KG, CELL, LOSS, EXT, false, PAIR>(a, grid, s);
 }
 
 const char* blas_status(cublasStatus_t st) {
@@ -136,6 +140,11 @@ const char* blas_status(cublasStatus_t st) {
     if (st_ != CUBLAS_STATUS_SUCCESS)                                                                 \
       return brie::fail(BRIE_ERR_CUDA, "%s failed: cuBLAS %s (%s:%d)", #call, blas_status(st_), __FILE__, __LINE__); \
   } while (0)
+
+// keras Adam's bias-corrected step size of Adam step t
+float adam_alpha(const brie_fit* f, int64_t t) {
+  return (float)((double)f->lr * sqrt(1.0 - pow(0.999, (double)t)) / (1.0 - pow(0.9, (double)t)));
+}
 
 uint32_t all_models(int n_models) { return n_models >= 32 ? 0xffffffffu : ((1u << n_models) - 1u); }
 
@@ -199,7 +208,12 @@ cudaError_t dispatch_step2(const StepArgs& a, bool cell, bool loss, dim3 grid, c
 }
 
 template <int KC>
-cudaError_t dispatch_step1(const StepArgs& a, int KG, bool cell, bool loss, dim3 grid, cudaStream_t s) {
+cudaError_t dispatch_step1(const StepArgs& a, int KG, bool cell, bool loss, bool pair, dim3 grid, cudaStream_t s) {
+  if constexpr (KC <= kMaxPairKc) {
+    if (pair)   // gene mode, Kg = 0 (brie_fit.pairs)
+      return loss ? launch_step_fmt<KC, 0, false, true, false, true>(a, grid, s)
+                  : launch_step_fmt<KC, 0, false, false, false, true>(a, grid, s);
+  }
   switch (KG) {
     case 0: return dispatch_step2<KC, 0>(a, cell, loss, grid, s);
     case 4: return dispatch_step2<KC, 4>(a, cell, loss, grid, s);
@@ -208,18 +222,32 @@ cudaError_t dispatch_step1(const StepArgs& a, int KG, bool cell, bool loss, dim3
   return cudaErrorInvalidValue;
 }
 
-cudaError_t dispatch_step(const StepArgs& a, bool wide, int KC, int KG, bool cell, bool loss, dim3 grid,
+cudaError_t dispatch_step(const StepArgs& a, bool wide, int KC, int KG, bool cell, bool loss, bool pair, dim3 grid,
                           cudaStream_t s) {
   if (wide) return dispatch_step2<0, 0, true>(a, cell, loss, grid, s);
   switch (KC) {
-    case 0: return dispatch_step1<0>(a, KG, cell, loss, grid, s);
-    case 1: return dispatch_step1<1>(a, KG, cell, loss, grid, s);
-    case 2: return dispatch_step1<2>(a, KG, cell, loss, grid, s);
-    case 4: return dispatch_step1<4>(a, KG, cell, loss, grid, s);
-    case 8: return dispatch_step1<8>(a, KG, cell, loss, grid, s);
-    case 16: return dispatch_step1<16>(a, KG, cell, loss, grid, s);   // 2 events per lane, 64-event tiles
+    case 0: return dispatch_step1<0>(a, KG, cell, loss, pair, grid, s);
+    case 1: return dispatch_step1<1>(a, KG, cell, loss, pair, grid, s);
+    case 2: return dispatch_step1<2>(a, KG, cell, loss, pair, grid, s);
+    case 4: return dispatch_step1<4>(a, KG, cell, loss, pair, grid, s);
+    case 8: return dispatch_step1<8>(a, KG, cell, loss, pair, grid, s);
+    case 16: return dispatch_step1<16>(a, KG, cell, loss, pair, grid, s);   // 2 events per lane, 64-event tiles
   }
   return cudaErrorInvalidValue;
+}
+
+// the pre-pass of a run of two-step passes, one instantiation per covariate width
+cudaError_t dispatch_kl_sums(const StepArgs& a, int KC, int n_rows_chunks, cudaStream_t s) {
+  const unsigned tiles = (unsigned)ceil_div(a.ld, step_tile_cols(KC));
+  const dim3 grid(a.M, tiles, n_rows_chunks);
+  switch (KC) {
+    case 0: kl_sums_kernel<0><<<grid, kThreads, 0, s>>>(a); break;
+    case 1: kl_sums_kernel<1><<<grid, kThreads, 0, s>>>(a); break;
+    case 2: kl_sums_kernel<2><<<grid, kThreads, 0, s>>>(a); break;
+    case 4: kl_sums_kernel<4><<<grid, kThreads, 0, s>>>(a); break;
+    default: return cudaErrorInvalidValue;
+  }
+  return cudaGetLastError();
 }
 
 // The fields that StepArgs, MarginArgs, EvalArgs and TermsArgs share under the same names; the rest are zero.
@@ -277,10 +305,14 @@ int launch_margin_step(brie_fit* f, int nev, int cell_tiles, cudaStream_t s) {
 
 // target ELBO: the fused step kernel, between the wide form's prior-mean and gradient GEMMs.  The timing events
 // (brie_fit_kernel_timing) bracket the fused kernel alone.
-int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s) {
+// pair: a two-step pass, steps global_step and global_step + 1 with alpha and alpha2 (brie_fit_run_steps).
+int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s, bool pair = false, float alpha2 = 0.f) {
   const brie_fit_desc& d = f->d;
   float* scratch = (float*)f->buf.scratch;
   StepArgs a = fit_args<StepArgs>(f);
+  if (pair) {
+    a.alpha2 = alpha2; a.prev = scratch + f->off_prev; a.part_st = scratch + f->off_part_st;
+  }
   a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log; a.aZ = f->buf.adam_Z;
   a.active = f->buf.active;
   a.part_ev = scratch + f->off_part_ev; a.part_cell = scratch + f->off_part_cell;
@@ -303,7 +335,7 @@ int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s) {
   }
   const bool timed = f->ev_used < (int)f->ev0.size();
   if (timed) BRIE_CUDA(cudaEventRecord(f->ev0[f->ev_used], s));
-  BRIE_CUDA(dispatch_step(a, f->wide, d.Kc, d.Kg, d.cell_mode != 0, loss, grid, s));
+  BRIE_CUDA(dispatch_step(a, f->wide, d.Kc, d.Kg, d.cell_mode != 0, loss, pair, grid, s));
   if (timed) BRIE_CUDA(cudaEventRecord(f->ev1[f->ev_used++], s));
   f->launches += 1;
   return f->wide ? wide_gradients(f, s) : BRIE_OK;
@@ -311,7 +343,10 @@ int launch_fused_step(brie_fit* f, bool loss, cudaStream_t s) {
 
 // Per-event reduce of the row-chunk partials (nev rows, the loss last if loss_row), Adam on Wc and the per-event
 // intercept / sigma_log, and the loss trace if trace_slot >= 0.  The wide form's d/dWc comes from wide_gradients.
-int launch_event_update(brie_fit* f, int nev, bool loss_row, int32_t trace_slot, cudaStream_t s) {
+// Two-step passes: pair_loss (the second loss row), prev (save the parameters the next pass starts from) and
+// look_ahead (a second update with alpha2 from the statistics), see EventArgs.
+int launch_event_update(brie_fit* f, int nev, bool loss_row, int32_t trace_slot, cudaStream_t s, bool pair_loss = false,
+                        bool prev = false, bool look_ahead = false, float alpha2 = 0.f) {
   const brie_fit_desc& d = f->d;
   if (nev == 0 && !(f->wide && d.Kc > 0)) return BRIE_OK;
   float* scratch = (float*)f->buf.scratch;
@@ -321,6 +356,11 @@ int launch_event_update(brie_fit* f, int nev, bool loss_row, int32_t trace_slot,
   e.ld = d.ld; e.Ng = d.n_events; e.M = d.n_models; e.KC = d.Kc; e.NEV = nev; e.n_chunks = f->sz.n_row_chunks;
   e.idx_gb = d.cell_mode ? -1 : kc_kernel; e.idx_gt = d.cell_mode ? -1 : kc_kernel + 1;
   e.idx_loss = loss_row ? kc_kernel + (d.cell_mode ? 0 : 2) : -1;
+  e.idx_loss2 = pair_loss ? e.idx_loss + 1 : -1;
+  e.prev = prev || look_ahead ? scratch + f->off_prev : nullptr;
+  e.part_st = look_ahead ? scratch + f->off_part_st : nullptr;
+  e.gram = (const double*)(scratch + f->off_gram);
+  e.Nc = d.n_cells; e.alpha2 = alpha2;
   e.wc_grad = f->wide ? scratch + f->off_gWc : nullptr;
   e.train_b = d.train_intercept; e.train_tau = d.train_sigma;
   e.trace_slot = trace_slot; e.trace_cap = d.trace_cap;
@@ -423,7 +463,10 @@ int brie_fit_create(const brie_fit_desc* desc, brie_fit** out) {
     return fail(BRIE_ERR_UNSUPPORTED, "grid too large (%lld row chunks, %d column tiles)", (long long)n_chunks,
                 n_tiles);
   }
-  f->nev_max = (wide ? 0 : d.Kc) + 2 + 1;
+  // Fits whose per-event parameters are the only ones (gene mode, Kg = 0, Kc <= 4, target ELBO) step in two-step
+  // passes (brie_fit_run_steps): two loss rows, and the statistic partials, first-step parameters and Gram sums.
+  f->pairs = !d.cell_mode && d.Kg == 0 && !wide && d.Kc <= kMaxPairKc && d.target == BRIE_TARGET_ELBO;
+  f->nev_max = (wide ? 0 : d.Kc) + 2 + (f->pairs ? 2 : 1);
   f->ncell = d.Kg + (d.cell_mode ? 2 : 0);
   const int ncell_part = wide ? (d.cell_mode ? 2 : 0) : f->ncell;   // what the fused kernel leaves per cell and tile
   f->sz.rows_per_cta = rows;
@@ -438,6 +481,16 @@ int brie_fit_create(const brie_fit_desc* desc, brie_fit** out) {
   f->off_G = off;
   off += (size_t)d.n_models * d.n_cells * f->ncell;
   off = (off + 3) / 4 * 4;                     // 16-byte alignment of what follows
+  if (f->pairs) {
+    f->off_part_st = off;
+    off += (size_t)n_chunks * d.n_models * pair_stat_rows(d.Kc) * d.ld;
+    f->off_prev = off;
+    off += (size_t)d.n_models * (d.Kc + 2) * d.ld;
+    off = (off + 3) / 4 * 4;
+    f->off_gram = off;
+    off += (size_t)2 * d.n_models * (d.Kc * d.Kc + d.Kc + 1);   // float64
+    off = (off + 3) / 4 * 4;
+  }
   if (wide) {
     f->off_PM = off;
     off += (size_t)d.n_models * d.n_cells * d.ld;
@@ -644,8 +697,7 @@ int brie_fit_step_phase(brie_fit* f, int32_t phase, int32_t trace_slot, void* st
     if (!f->codes && !f->buf.counts[0]) return fail(BRIE_ERR_ARG, "neither count tiles nor count codes bound");
     // checked: a refused call leaves the Adam step as it was
     f->t += 1;
-    const double t = (double)f->t;
-    f->alpha = (float)((double)f->lr * sqrt(1.0 - pow(0.999, t)) / (1.0 - pow(0.9, t)));
+    f->alpha = adam_alpha(f, f->t);
     // per-event partials: the covariates the step kernel contracts itself, intercept and sigma (gene mode), then the
     // loss, which the marginLik kernel always sums; marginLik tiles its columns its own way
     const bool loss_row = loss || margin;
@@ -672,13 +724,58 @@ int brie_fit_step_phase(brie_fit* f, int32_t phase, int32_t trace_slot, void* st
 int brie_fit_run_steps(brie_fit* f, int32_t n_steps, int32_t trace_slot0, void* stream) {
   if (!f || !f->bound) return fail(BRIE_ERR_ARG, "fit not bound");
   if (n_steps < 0) return fail(BRIE_ERR_ARG, "n_steps must be >= 0");
-  const int64_t n_G = (int64_t)f->d.n_models * f->d.n_cells * f->ncell;
-  for (int i = 0; i < n_steps; ++i) {
+  cudaStream_t s = (cudaStream_t)stream;
+  const brie_fit_desc& d = f->d;
+  const int64_t n_G = (int64_t)d.n_models * d.n_cells * f->ncell;
+  int i = 0;
+  // Per-event-only fits take their steps two per pass over the state (elbo_step_kernel PAIR): the state is read and
+  // written once for both.  A pass starts from the parameters of its two steps, which a sums-only pre-pass provides
+  // for the first; every pass but the last also takes the next pass' parameters from its statistics.  An odd last
+  // step runs alone.  The call ends at the state, parameters, Adam step and RNG step word of n_steps single steps.
+  if (f->pairs && !f->comm && n_steps >= 2) {
+    if (f->step_open) return fail(BRIE_ERR_ARG, "a split step is still open");
+    if (!f->stage_open) return fail(BRIE_ERR_ARG, "brie_fit_begin_stage must be called before the first step");
+    if (!f->codes && !f->buf.counts[0]) return fail(BRIE_ERR_ARG, "neither count tiles nor count codes bound");
+    if (trace_slot0 >= 0 && trace_slot0 + n_steps > d.trace_cap)
+      return fail(BRIE_ERR_ARG, "trace slots %d..%d exceed trace_cap %d", trace_slot0, trace_slot0 + n_steps - 1,
+                  d.trace_cap);
+    float* scratch = (float*)f->buf.scratch;
+    if (d.Kc > 0) {
+      gram_kernel<<<dim3(d.Kc * d.Kc + d.Kc, d.n_models), 256, 0, s>>>(f->buf.Xc, d.n_cells, d.Kc,
+                                                                     (double*)(scratch + f->off_gram));
+      BRIE_CUDA(cudaGetLastError());
+      f->launches += 1;
+    }
+    StepArgs a = fit_args<StepArgs>(f);
+    a.Zl = f->buf.Z_loc; a.Zs = f->buf.Z_std_log;
+    a.active = f->buf.active; a.part_ev = scratch + f->off_part_ev;
+    a.model_mask = f->model_mask; a.rows_per_cta = f->sz.rows_per_cta;
+    BRIE_CUDA(dispatch_kl_sums(a, d.Kc, f->sz.n_row_chunks, s));
+    f->launches += 1;
+    f->alpha = adam_alpha(f, f->t + 1);
+    int rc = launch_event_update(f, d.Kc + 2, false, -1, s, false, true);
+    if (rc) return rc;
+    for (; i + 2 <= n_steps; i += 2) {
+      const bool loss = trace_slot0 >= 0;
+      const bool look_ahead = i + 4 <= n_steps;
+      const int nev = d.Kc + 2 + (loss ? 2 : 0);
+      f->alpha = adam_alpha(f, f->t + 1);
+      const float alpha2 = adam_alpha(f, f->t + 2);
+      rc = launch_fused_step(f, loss, s, true, alpha2);
+      f->alpha = alpha2;
+      if (!rc) rc = launch_event_update(f, nev, loss, loss ? trace_slot0 + i : -1, s, loss, false, look_ahead,
+                                        adam_alpha(f, f->t + 3));
+      if (rc) return rc;
+      f->t += 2;
+      f->global_step += 2;
+    }
+  }
+  for (; i < n_steps; ++i) {
     const int slot = trace_slot0 >= 0 ? trace_slot0 + i : -1;
     int rc = brie_fit_step_phase(f, 0, slot, stream);
     if (rc) return rc;
     if (f->comm && n_G > 0) {   // the path's one exchange step, in stream order between the two halves
-      rc = comm_allreduce_sum_f32(f->comm, (float*)f->buf.scratch + f->off_G, n_G, (cudaStream_t)stream);
+      rc = comm_allreduce_sum_f32(f->comm, (float*)f->buf.scratch + f->off_G, n_G, s);
       if (rc) return rc;
     }
     rc = brie_fit_step_phase(f, 1, slot, stream);

@@ -58,6 +58,13 @@ struct StepArgs {
   float alpha;
   float inv_S;
   uint32_t step;
+  // Two-step passes (PAIR instantiations, gene mode with per-event parameters only): the pass takes step `step` with
+  // the parameters in `prev` ((M, KC + 2, ld): Wc rows, intercept, sigma_log) and `alpha`, then step `step` + 1 with
+  // Wc / b / tau and `alpha2`, and leaves in part_st the statistics of the state it writes around Wc / b / tau
+  // (pair_stat_rows, brie_fit_run_steps).
+  float alpha2;
+  const float* prev;
+  float* part_st;    // (n_row_chunks, M, KC + 3, ld)
   uint32_t model_mask;  // bit m: model m has any active event
   int32_t M, S, rows_per_cta;
   int32_t model_id[kMaxModels];
@@ -261,12 +268,12 @@ __device__ __forceinline__ void mc_samples(float mu, float s, float c1, float c2
   }
 }
 
-template <int KC, int KG, bool CELL, bool LOSS>
+template <int KC, int KG, bool CELL, bool LOSS, bool PAIR = false>
 struct StepTraits {
   static constexpr int kGB = KC;                       // index of d/d intercept (gene mode)
   static constexpr int kGT = KC + 1;                   // index of d/d sigma_log (gene mode)
-  static constexpr int kLoss = KC + (CELL ? 0 : 2);    // sum over cells of KL - loglik
-  static constexpr int NEV = KC + (CELL ? 0 : 2) + (LOSS ? 1 : 0);
+  static constexpr int kLoss = KC + (CELL ? 0 : 2);    // sum over cells of KL - loglik (PAIR: of each step in turn)
+  static constexpr int NEV = KC + (CELL ? 0 : 2) + (LOSS ? (PAIR ? 2 : 1) : 0);
   static constexpr int NCELL = KG + (CELL ? 2 : 0);
 };
 
@@ -351,37 +358,56 @@ __host__ __device__ constexpr int step_rpi(int KC, int KG = 0) {
 // (profiles/r1_ab_smem_consts.md, r1_ab_row_consts.md): C3 with loss trace +11 %, C4 +10 % / +23 %,
 // Kc 15 +9 %; C3 without the loss trace runs 1 % slower from shared memory but spills from registers.
 __host__ __device__ constexpr bool step_consts_in_smem(int KC, int KG) { return KC + KG >= 3; }
-__host__ __device__ constexpr int step_n_consts(int KC, int KG, bool CELL) {
-  return step_consts_in_smem(KC, KG) ? KC + KG + (CELL ? 0 : 3) : 0;
+// Two-step passes keep both steps' constants in shared memory, whatever the width.
+__host__ __device__ constexpr int step_n_consts(int KC, int KG, bool CELL, bool PAIR = false) {
+  return PAIR ? 2 * (KC + 3) : (step_consts_in_smem(KC, KG) ? KC + KG + (CELL ? 0 : 3) : 0);
 }
+// Widest design stepped in two-step passes: above it the two steps' per-event sums and statistics no longer fit the
+// register budget of two CTAs per SM (the Kc = 8 and 16 forms spill hundreds of bytes to local memory).
+constexpr int kMaxPairKc = 4;
+// Per-event statistics a two-step pass leaves per row chunk: R_k = sum_c x_ck d_c, R_0 = sum_c d_c, Q = sum_c d_c^2 and
+// E = sum_c exp(2 (lam_c - tau)), d_c = mu_c - prior mean, of the state it writes, around the second step's parameters.
+__host__ __device__ constexpr int pair_stat_rows(int KC) { return KC + 3; }
 constexpr int kRowConstSlots = 32;   // per warp and ring stage: Xc[c, :], Wg[c, :], per-cell intercept / sigma_log of the row
-// CODE8: per warp and row of an iteration, the Monte-Carlo sums d/dZ_loc, d/dZ_std_log and (LOSS) the log-likelihood
+// CODE8 or PAIR: per warp and row of an iteration, the Monte-Carlo sums d/dZ_loc, d/dZ_std_log and (LOSS) the
+// log-likelihood (a two-step pass keeps the counts in the ring for its second step)
 __host__ __device__ constexpr int step_n_scratch(bool LOSS) { return LOSS ? 3 : 2; }
 __host__ __device__ constexpr int step_smem_bytes(int KC, int KG, bool CELL, bool LOSS, bool EXT = false,
-                                                  bool CODE8 = false) {
+                                                  bool CODE8 = false, bool PAIR = false) {
   return ((kWarps * kRingStages * ((CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0)) +
-           kWarps * kQueueFields + (CODE8 ? kWarps * step_n_scratch(LOSS) : 0)) *
+           kWarps * kQueueFields + (CODE8 || PAIR ? kWarps * step_n_scratch(LOSS) : 0)) *
               step_rpi(KC, KG) +
-          7 + step_n_consts(KC, KG, CELL)) *
+          7 + step_n_consts(KC, KG, CELL, PAIR)) *
              step_tile_cols(KC, KG) * 4 +
          kWarps * kRingStages * step_rpi(KC, KG) * kRowConstSlots * 4 + (CODE8 ? 3 * kDictSize * 4 : 0);
 }
 
-template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false, bool CODE8 = false>
+// PAIR (two steps per pass, gene mode with per-event parameters only): after phase C of the first step the updated
+// Z_loc, Z_std_log and moments go back into the row's ring slot instead of HBM, and phases A-C run again with the
+// second step's constants, RNG step word and alpha; the Monte-Carlo queue is built once (it depends on the counts
+// only).  The per-event gradient sums are those of the second step (the first step's came from the previous pass'
+// statistics, or the sums-only pre-pass, kl_sums_kernel), and the state written is also summed into the statistics
+// of pair_stat_rows around the second step's parameters, from which event_update_kernel forms the next step's sums.
+template <int KC, int KG, bool CELL, bool LOSS, bool EXT = false, bool CODE8 = false, bool PAIR = false>
 __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const StepArgs a) {
   static_assert(!EXT || (KC == 0 && KG == 0), "the wide-design form takes all covariates through PM / R");
+  static_assert(!PAIR || (!CELL && KG == 0 && !EXT), "two-step passes need per-event parameters only");
+  constexpr int NSTEP = PAIR ? 2 : 1;
+  constexpr bool SCR = CODE8 || PAIR;                // Monte-Carlo sums go to the per-warp scratch, not the count slots
+  constexpr int NK = KC + KG + (CELL ? 0 : 3);       // per-event constant rows of one step (kSm)
+  constexpr int NST = PAIR ? pair_stat_rows(KC) : 0;
   // ring arrays per row slot (EXT: + the prior-mean tile) and the slots of the Adam moments / prior-mean tile in it
   constexpr int NRA = (CODE8 ? kRingArraysCode8 : kRingArrays) + (EXT ? 1 : 0);
   constexpr int IA = CODE8 ? 3 : 5;                  // m_loc, v_loc, m_std, v_std at IA .. IA + 3
   constexpr int IPM = IA + 4;
   constexpr int NSCR = step_n_scratch(LOSS);
   constexpr int RPI = step_rpi(KC, KG);              // rows per loop iteration = row slots per ring stage
-  using T = StepTraits<KC, KG, CELL, LOSS>;
+  using T = StepTraits<KC, KG, CELL, LOSS, PAIR>;
   constexpr int NEV = T::NEV;
   constexpr int NCELL = T::NCELL;
   constexpr int EPL = step_epl(KC, KG);
   constexpr int TC = 32 * EPL;              // events per warp row segment (column tile)
-  constexpr bool kSm = step_consts_in_smem(KC, KG);
+  constexpr bool kSm = step_consts_in_smem(KC, KG) || PAIR;
   using Vec = typename LaneVec<EPL>::type;
   const int m = blockIdx.x;
   if (!((a.model_mask >> m) & 1u)) return;
@@ -421,7 +447,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
   float(*s_L)[TC] = reinterpret_cast<float(*)[TC]>(smem + kWarps * kRingStages * RPI * SLOT +
                                                    kWarps * kQueueFields * RPI * TC);
   uint32_t* s_ev = reinterpret_cast<uint32_t*>(s_L + 6);   // global event id of each tile column (RNG counter word)
-  float(*s_k)[TC] = s_L + 7;                // kSm: rows Wc[0..KC), Xg[0..KG), then (gene mode) b, tau, 1/sigma^2
+  float(*s_k)[TC] = s_L + 7;                // kSm: rows Wc[0..KC), Xg[0..KG), then (gene mode) b, tau, 1/sigma^2 (PAIR: per step)
   // Gene-feature slots are stored XOR-permuted per lane (slot i of lane L holds feature i ^ pk(L), pk = the top
   // log2(KG) lane bits reversed into a feature index) so that the per-cell reduction over the 32 lanes of
   // d loss / d Wg[c, :] is a halving butterfly without selects (see the end of the row loop).
@@ -433,9 +459,9 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
   constexpr int NRC = KC + KG + (CELL ? 2 : 0);   // per-row (cell) constants: Xc[c, :], Wg[c, :], b[c], tau[c]
   static_assert(NRC <= kRowConstSlots, "row constants must fit one slot per lane");
   constexpr int kRcBase = ((kWarps * kRingStages * NRA + kWarps * kQueueFields) * RPI + 7 +
-                           step_n_consts(KC, KG, CELL)) * TC;
+                           step_n_consts(KC, KG, CELL, PAIR)) * TC;
   float* s_rc = smem + kRcBase + warp * (kRingStages * RPI * kRowConstSlots);
-  // CODE8: this warp's Monte-Carlo sums (row r, sum k at (r * NSCR + k) * TC) and the count dictionary
+  // CODE8 or PAIR: this warp's Monte-Carlo sums (row r, sum k at (r * NSCR + k) * TC); CODE8: the count dictionary
   constexpr int kScrBase = kRcBase + kWarps * kRingStages * RPI * kRowConstSlots;
   float* const s_scr = smem + kScrBase + warp * (NSCR * RPI * TC);
   float* const s_dict = smem + kScrBase + kWarps * NSCR * RPI * TC;
@@ -460,16 +486,24 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
       s_L[5][threadIdx.x] = a.eff ? logf(l3) : 0.f;
     }
     if (kSm) {
-      const bool okc = g < a.ld;
 #pragma unroll
-      for (int k = 0; k < KC; ++k) s_k[k][threadIdx.x] = okc ? a.Wc[((int64_t)m * KC + k) * a.ld + g] : 0.f;
+      for (int h = 0; h < NSTEP; ++h) {
+        // PAIR: the first step's parameters of the real events come from `prev`
+        const bool okc = g < a.ld, from_prev = PAIR && h == 0 && g < a.Ng;
+        const float* wsrc = from_prev ? a.prev + (int64_t)m * (KC + 2) * a.ld : a.Wc + (int64_t)m * KC * a.ld;
+        const float* bsrc = from_prev ? a.prev + ((int64_t)m * (KC + 2) + KC) * a.ld : a.b + (int64_t)m * a.ld;
+        const float* tsrc = from_prev ? a.prev + ((int64_t)m * (KC + 2) + KC + 1) * a.ld : a.tau + (int64_t)m * a.ld;
+        float(*sk)[TC] = s_k + h * NK;
 #pragma unroll
-      for (int k = 0; k < KG; ++k) s_k[KC + k][threadIdx.x] = g < a.Ng ? a.Xg[g * KG + k] : 0.f;
-      if (!CELL) {
-        const float t = okc ? a.tau[(int64_t)m * a.ld + g] : 0.f;
-        s_k[KC + KG][threadIdx.x] = okc ? a.b[(int64_t)m * a.ld + g] : 0.f;
-        s_k[KC + KG + 1][threadIdx.x] = t;
-        s_k[KC + KG + 2][threadIdx.x] = fast_exp(-2.0f * t);
+        for (int k = 0; k < KC; ++k) sk[k][threadIdx.x] = okc ? wsrc[k * a.ld + g] : 0.f;
+#pragma unroll
+        for (int k = 0; k < KG; ++k) sk[KC + k][threadIdx.x] = g < a.Ng ? a.Xg[g * KG + k] : 0.f;
+        if (!CELL) {
+          const float t = okc ? tsrc[g] : 0.f;
+          sk[KC + KG][threadIdx.x] = okc ? bsrc[g] : 0.f;
+          sk[KC + KG + 1][threadIdx.x] = t;
+          sk[KC + KG + 2][threadIdx.x] = fast_exp(-2.0f * t);
+        }
       }
     }
   }
@@ -585,6 +619,11 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
   for (int i = 0; i < (NEV > 0 ? NEV : 1); ++i)
 #pragma unroll
     for (int j = 0; j < EPL; ++j) acc[i][j] = 0.f;
+  float stat[NST > 0 ? NST : 1][EPL];       // PAIR: R_k (k < KC), R_0, Q, E of the lane's events
+#pragma unroll
+  for (int i = 0; i < (NST > 0 ? NST : 1); ++i)
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) stat[i][j] = 0.f;
 
   const uint32_t stream0 = brie_stream_word(BRIE_PHASE_TRAIN, (uint32_t)a.model_id[m], 0u);
   const uint32_t lt_mask = (1u << lane) - 1u;
@@ -623,9 +662,17 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
     cp_async_wait<1>();                   // this iteration's group has landed
     __syncwarp();                         // other lanes read this lane's copies (row constants, Monte-Carlo items)
     float* const rs0 = s_ring + stage * (RPI * SLOT);                 // row slot r of this stage: rs0 + r * SLOT
+    uint32_t nz = 0;                      // bit r * EPL + j: element j of row r has reads
+    uint32_t bal[RPI * EPL];
+    int n_items = 0;
+#pragma unroll
+    for (int h = 0; h < NSTEP; ++h) {     // PAIR: step `step` + h of the pass
+    const float(*sk)[TC] = s_k + h * NK;
+    const float alpha = h == 0 ? a.alpha : a.alpha2;
+    // PAIR: the first step leaves nothing in the per-event gradient sums (only its loss)
+    const bool grad_sums = !PAIR || h == NSTEP - 1;
     float mu[RPI][EPL], lam[RPI][EPL], gmu[RPI][EPL], glam[RPI][EPL];
     float cacc1[NCELL > 0 ? NCELL : 1];   // RPI == 1: kept until after phase C (as tuned for the gene-feature kernels)
-    uint32_t nz = 0;                      // bit r * EPL + j: element j of row r has reads
 
     // ---- phase A: KL terms, shared-parameter accumulators, non-zero detection ----
 #pragma unroll
@@ -671,14 +718,14 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
       for (int i = 0; i < (NCELL > 0 ? NCELL : 1); ++i) cacc[i] = 0.f;
       if (kSm) {  // this row's copy of the tile constants (dead again before the Monte-Carlo phase)
 #pragma unroll
-        for (int k = 0; k < KC; ++k) vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[k][lane * EPL]), wc[k]);
+        for (int k = 0; k < KC; ++k) vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[k][lane * EPL]), wc[k]);
 #pragma unroll
         for (int k = 0; k < KG; ++k)
-          vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[KC + (k ^ pk)][lane * EPL]), xg[k]);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC + (k ^ pk)][lane * EPL]), xg[k]);
         if (!CELL) {
-          vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[KC + KG][lane * EPL]), bb);
-          vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[KC + KG + 1][lane * EPL]), tau);
-          vec_get<EPL>(*reinterpret_cast<const Vec*>(&s_k[KC + KG + 2][lane * EPL]), is2);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC + KG][lane * EPL]), bb);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC + KG + 1][lane * EPL]), tau);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC + KG + 2][lane * EPL]), is2);
         }
       }
       static_assert(EPL % 2 == 0, "packed pairs need an even number of events per lane");
@@ -706,16 +753,20 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
         const float2 e2m1 = f2_add(e2, f2_splat(-1.0f));
         gmu[r][j0] = rr.x; gmu[r][j1] = rr.y;
         glam[r][j0] = e2m1.x; glam[r][j1] = e2m1.y;
-        if (has_reads(j0)) nz |= 1u << (r * EPL + j0);
-        if (has_reads(j1)) nz |= 1u << (r * EPL + j1);
+        if (h == 0) {
+          if (has_reads(j0)) nz |= 1u << (r * EPL + j0);
+          if (has_reads(j1)) nz |= 1u << (r * EPL + j1);
+        }
         const float2 gt = f2_sub(f2_sub(f2_splat(1.0f), q2), e2);            // d loss / d sigma_log
+        if (grad_sums) {
 #pragma unroll
-        for (int k = 0; k < KC; ++k) {
-          const float2 t = f2_fma(f2_splat(xc[k]), nr, make_float2(acc[k][j0], acc[k][j1]));
-          acc[k][j0] = t.x; acc[k][j1] = t.y;
+          for (int k = 0; k < KC; ++k) {
+            const float2 t = f2_fma(f2_splat(xc[k]), nr, make_float2(acc[k][j0], acc[k][j1]));
+            acc[k][j0] = t.x; acc[k][j1] = t.y;
+          }
         }
         const float2 rrs = real_row ? rr : f2_splat(0.f), gts = real_row ? gt : f2_splat(0.f);
-        if (!CELL) {
+        if (!CELL && grad_sums) {
           const float2 t = f2_sub(make_float2(acc[T::kGB][j0], acc[T::kGB][j1]), rrs);
           acc[T::kGB][j0] = t.x; acc[T::kGB][j1] = t.y;
           const float2 u = f2_add(make_float2(acc[T::kGT][j0], acc[T::kGT][j1]), gts);
@@ -724,8 +775,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
         if (LOSS) {                                                          // TFP _kl_normal_normal
           float2 kl = f2_sub(f2_fma(f2_splat(0.5f), q2, f2_mul(f2_splat(0.5f), e2m1)), d);
           if (!real_row) kl = f2_splat(0.f);
-          const float2 t = f2_add(make_float2(acc[T::kLoss][j0], acc[T::kLoss][j1]), kl);
-          acc[T::kLoss][j0] = t.x; acc[T::kLoss][j1] = t.y;
+          const float2 t = f2_add(make_float2(acc[T::kLoss + h][j0], acc[T::kLoss + h][j1]), kl);
+          acc[T::kLoss + h][j0] = t.x; acc[T::kLoss + h][j1] = t.y;
         }
         if (NCELL > 0) {
           const float2 nrm = make_float2((g0 + j0) < a.Ng ? nr.x : 0.f, (g0 + j1) < a.Ng ? nr.y : 0.f);
@@ -748,25 +799,28 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
     if (RPI > 1 && NRC > 0) __syncwarp(); // all lanes have read the row constants before the next prefetch of these slots
 
     // ---- phase B: compacted Monte-Carlo work (the items of all RPI rows share the passes) ----
-    uint32_t bal[RPI * EPL];
-    int base = 0;
-    int n_items = 0;
+    if (h == 0) {
 #pragma unroll
-    for (int j = 0; j < RPI * EPL; ++j) {
-      bal[j] = __ballot_sync(0xffffffffu, nz & (1u << j));
-      n_items += __popc(bal[j]);
+      for (int j = 0; j < RPI * EPL; ++j) {
+        bal[j] = __ballot_sync(0xffffffffu, nz & (1u << j));
+        n_items += __popc(bal[j]);
+      }
     }
     if (n_items > 0) {
-#pragma unroll
-      for (int j = 0; j < RPI * EPL; ++j) base += __popc(bal[j] & lt_mask);
       // The queue holds (row slot, tile column) only.  The rows' Z_loc, Z_std_log and counts are still in this stage
       // of the ring, so whichever lane takes an item reads them from there and leaves the Monte-Carlo sums in the
       // element's own count slots; an element without reads has zeros in those slots (counts are >= 0), so the
-      // owners subtract their slots unconditionally afterwards.
+      // owners subtract their slots unconditionally afterwards.  (PAIR: the queue of the first step serves both; the
+      // barrier below also publishes the first step's updated Z_loc / Z_std_log in the ring.)
+      if (h == 0) {
+        int base = 0;
 #pragma unroll
-      for (int j = 0; j < RPI * EPL; ++j)
-        if ((nz >> j) & 1u)
-          q[base + __popc(nz & ((1u << j) - 1u))] = (uint32_t)((j / EPL) * TC + lane * EPL + (j % EPL));
+        for (int j = 0; j < RPI * EPL; ++j) base += __popc(bal[j] & lt_mask);
+#pragma unroll
+        for (int j = 0; j < RPI * EPL; ++j)
+          if ((nz >> j) & 1u)
+            q[base + __popc(nz & ((1u << j) - 1u))] = (uint32_t)((j / EPL) * TC + lane * EPL + (j % EPL));
+      }
       __syncwarp();
       for (int k = lane; k < n_items; k += 32) {
         const int item = (int)q[k];
@@ -786,8 +840,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
         const float l1 = s_L[0][col], l2 = s_L[1][col], l3 = s_L[2][col];
         float gs, ge, ls;
         mc_samples<LOSS>(imu, is, ic1, ic2, in, l1, l2, l3, l1 - l2, a.S, s_ev[col], (uint32_t)(row_begin + lrb + r),
-                         a.step, stream0, a.seed, gs, ge, ls);
-        float* const out = CODE8 ? s_scr + r * (NSCR * TC) : rs + 2 * TC;
+                         a.step + (uint32_t)h, stream0, a.seed, gs, ge, ls);
+        float* const out = SCR ? s_scr + r * (NSCR * TC) : rs + 2 * TC;
         out[col] = gs * a.inv_S;
         out[TC + col] = ge * is * a.inv_S;
         if (LOSS)
@@ -796,14 +850,14 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
       __syncwarp();
 #pragma unroll
       for (int r = 0; r < RPI; ++r) {
-        // CODE8: the scratch holds sums only where this row had items, stale values elsewhere -- an element without
+        // SCR: the scratch holds sums only where this row had items, stale values elsewhere -- an element without
         // reads subtracts 0, as it subtracts its zero counts in the f32 form
-        const Vec* st = CODE8 ? reinterpret_cast<const Vec*>(s_scr + r * (NSCR * TC)) + lane
-                              : reinterpret_cast<const Vec*>(rs0 + r * SLOT + 2 * TC) + lane;
+        const Vec* st = SCR ? reinterpret_cast<const Vec*>(s_scr + r * (NSCR * TC)) + lane
+                            : reinterpret_cast<const Vec*>(rs0 + r * SLOT + 2 * TC) + lane;
         float r1[EPL], r2[EPL];
         vec_get<EPL>(st[0 * 32], r1);
         vec_get<EPL>(st[1 * 32], r2);
-        if (CODE8) {
+        if (SCR) {
 #pragma unroll
           for (int j = 0; j < EPL; ++j) {
             const bool hit = (nz >> (r * EPL + j)) & 1u;
@@ -820,12 +874,12 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
           float r3[EPL];
           vec_get<EPL>(st[2 * 32], r3);
 #pragma unroll
-          for (int j = 0; j < EPL; ++j) acc[T::kLoss][j] -= CODE8 && !((nz >> (r * EPL + j)) & 1u) ? 0.f : r3[j];
+          for (int j = 0; j < EPL; ++j) acc[T::kLoss + h][j] -= SCR && !((nz >> (r * EPL + j)) & 1u) ? 0.f : r3[j];
         }
       }
     }
 
-    // ---- phase C: Adam on Z_loc / Z_std_log, clip, store ----
+    // ---- phase C: Adam on Z_loc / Z_std_log, clip, store (PAIR, first step: back into the ring slot) ----
 #pragma unroll
     for (int r = 0; r < RPI; ++r) {
       const int lr = lrb + r;
@@ -840,8 +894,8 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
 #pragma unroll
           for (int p = 0; p < EPL / 2; ++p) {
             const int j0 = 2 * p, j1 = 2 * p + 1;
-            adam_update2(mu[r][j0], mu[r][j1], m1[j0], m1[j1], v1[j0], v1[j1], gmu[r][j0], gmu[r][j1], a.alpha);
-            adam_update2(lam[r][j0], lam[r][j1], m2[j0], m2[j1], v2[j0], v2[j1], glam[r][j0], glam[r][j1], a.alpha);
+            adam_update2(mu[r][j0], mu[r][j1], m1[j0], m1[j1], v1[j0], v1[j1], gmu[r][j0], gmu[r][j1], alpha);
+            adam_update2(lam[r][j0], lam[r][j1], m2[j0], m2[j1], v2[j0], v2[j1], glam[r][j0], glam[r][j1], alpha);
             mu[r][j0] = clip9(mu[r][j0]);  // Variable constraint (model_TFProb.py:80-81)
             mu[r][j1] = clip9(mu[r][j1]);
           }
@@ -849,22 +903,58 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
 #pragma unroll
           for (int j = 0; j < EPL; ++j) {
             if ((act >> j) & 1u) {
-              adam_update(mu[r][j], m1[j], v1[j], gmu[r][j], a.alpha);
-              adam_update(lam[r][j], m2[j], v2[j], glam[r][j], a.alpha);
+              adam_update(mu[r][j], m1[j], v1[j], gmu[r][j], alpha);
+              adam_update(lam[r][j], m2[j], v2[j], glam[r][j], alpha);
               mu[r][j] = clip9(mu[r][j]);
             }
           }
         }
-        const uint32_t rel = (uint32_t)lr * ld32 + col32;
-        __stcs(reinterpret_cast<Vec*>(bZl + rel), vec_make<EPL>(mu[r]));
-        __stcs(reinterpret_cast<Vec*>(bZs + rel), vec_make<EPL>(lam[r]));
-        __stcs(reinterpret_cast<Vec*>(bA0 + rel), vec_make<EPL>(m1));
-        __stcs(reinterpret_cast<Vec*>(bA1 + rel), vec_make<EPL>(v1));
-        __stcs(reinterpret_cast<Vec*>(bA2 + rel), vec_make<EPL>(m2));
-        __stcs(reinterpret_cast<Vec*>(bA3 + rel), vec_make<EPL>(v2));
+        if (h < NSTEP - 1) {
+          Vec* sw = reinterpret_cast<Vec*>(rs0 + r * SLOT) + lane;
+          sw[0 * 32] = vec_make<EPL>(mu[r]);
+          sw[1 * 32] = vec_make<EPL>(lam[r]);
+          sw[(IA + 0) * 32] = vec_make<EPL>(m1);
+          sw[(IA + 1) * 32] = vec_make<EPL>(v1);
+          sw[(IA + 2) * 32] = vec_make<EPL>(m2);
+          sw[(IA + 3) * 32] = vec_make<EPL>(v2);
+        } else {
+          const uint32_t rel = (uint32_t)lr * ld32 + col32;
+          __stcs(reinterpret_cast<Vec*>(bZl + rel), vec_make<EPL>(mu[r]));
+          __stcs(reinterpret_cast<Vec*>(bZs + rel), vec_make<EPL>(lam[r]));
+          __stcs(reinterpret_cast<Vec*>(bA0 + rel), vec_make<EPL>(m1));
+          __stcs(reinterpret_cast<Vec*>(bA1 + rel), vec_make<EPL>(v1));
+          __stcs(reinterpret_cast<Vec*>(bA2 + rel), vec_make<EPL>(m2));
+          __stcs(reinterpret_cast<Vec*>(bA3 + rel), vec_make<EPL>(v2));
+        }
+        if (PAIR && h == NSTEP - 1) {
+          // statistics of the state just written around this step's parameters, centred there: the zero-count
+          // elements' Z_loc sit close to the prior mean, so sums taken around 0 would cancel
+          const float* rc = s_rc + (stage * RPI + r) * kRowConstSlots;
+          float xs[KC > 0 ? KC : 1];
+#pragma unroll
+          for (int k = 0; k < KC; ++k) xs[k] = rc[k];
+#pragma unroll
+          for (int k = 0; k < KC; ++k) vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[k][lane * EPL]), wc[k]);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC][lane * EPL]), bb);
+          vec_get<EPL>(*reinterpret_cast<const Vec*>(&sk[KC + 1][lane * EPL]), tau);
+#pragma unroll
+          for (int j = 0; j < EPL; ++j) {
+            float pm = bb[j];
+#pragma unroll
+            for (int k = 0; k < KC; ++k) pm = fmaf(xs[k], wc[k][j], pm);
+            const float dv = mu[r][j] - pm;
+#pragma unroll
+            for (int k = 0; k < KC; ++k) stat[k][j] = fmaf(xs[k], dv, stat[k][j]);
+            stat[KC][j] += dv;
+            stat[KC + 1][j] = fmaf(dv, dv, stat[KC + 1][j]);
+            stat[KC + 2][j] += ex2_approx((lam[r][j] - tau[j]) * (2.0f * kLog2e));
+          }
+        }
       }
     }
     if (RPI == 1 && NCELL > 0) cell_reduce_store(cacc1, row_begin + lrb);
+    }
+    if (PAIR) __syncwarp();   // all lanes have read this stage's row constants and ring slots before the next prefetch
   }
   cp_async_wait<0>();
 
@@ -881,6 +971,18 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) elbo_step_kernel(const Ste
 #pragma unroll
         for (int w = 0; w < kWarps; ++w) s += red[w][threadIdx.x];
         a.part_ev[(((int64_t)chunk * a.M + m) * NEV + i) * a.ld + gcol] = s;
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < NST; ++i) {
+      *reinterpret_cast<Vec*>(&red[warp][lane * EPL]) = vec_make<EPL>(stat[i]);
+      __syncthreads();
+      if (threadIdx.x < TC && gcol < a.ld) {
+        float s = 0.f;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) s += red[w][threadIdx.x];
+        a.part_st[(((int64_t)chunk * a.M + m) * NST + i) * a.ld + gcol] = s;
       }
       __syncthreads();
     }
@@ -905,9 +1007,21 @@ struct EventArgs {
   // wide designs: d loss / d Wc comes from a GEMM as a dense (M, KC, ld) array, rows [0, xc_width[m]) in use
   const float* wc_grad;
   int32_t xc_width[kMaxModels];
+  // Two-step passes (brie_fit_run_steps).  idx_loss2 >= 0: the row of the pass' second loss, for trace_slot + 1.
+  // prev (M, KC + 2, ld), if set, receives the parameters the next pass takes its first step with: those before this
+  // update, or with part_st those after the first of two updates.  part_st, if set: the pass' statistics
+  // (pair_stat_rows), from which the look-ahead update with alpha2 takes its sums; gram (M, KC * KC + KC) holds
+  // sum_c x_c x_c^T and sum_c x_c in float64, and Nc is the number of cells.
+  int32_t idx_loss2;
+  float* prev;
+  const float* part_st;
+  const double* gram;
+  int64_t Nc;
+  float alpha2;
 };
 
-constexpr int kMaxNEV = 19;  // BRIE_MAX_KC + 2 + 1
+constexpr int kMaxNEV = 20;  // BRIE_MAX_KC + 2 + 2 (two loss rows of a two-step pass)
+constexpr int kMaxNST = 7;   // pair_stat_rows(kMaxPairKc)
 
 // block = 8 warps x 32 events: warp w sums row chunks w, w+8, ... (coalesced 128-byte rows of the
 // partial buffer), warp 0 combines the 8 sub-sums in fixed order (f64) and applies the updates.
@@ -915,17 +1029,43 @@ __global__ void __launch_bounds__(256) event_update_kernel(const EventArgs a) {
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t g = (int64_t)blockIdx.x * 32 + lane;
   const int m = blockIdx.y;
-  __shared__ float s_part[8][kMaxNEV][32];
+  __shared__ float s_part[8][kMaxNEV + kMaxNST][32];
   const bool ok = g < a.Ng && a.active[(int64_t)m * a.ld + g] != 0;
+  const int nst = a.part_st && a.KC <= kMaxPairKc ? pair_stat_rows(a.KC) : 0;
   if (ok) {
-    for (int i = 0; i < a.NEV; ++i) {
+    for (int i = 0; i < a.NEV + nst; ++i) {
+      const float* src = i < a.NEV ? a.part_ev + (int64_t)i * a.ld : a.part_st + (int64_t)(i - a.NEV) * a.ld;
+      const int n = i < a.NEV ? a.NEV : nst;
       float s = 0.f;
-      for (int c = w; c < a.n_chunks; c += 8) s += a.part_ev[(((int64_t)c * a.M + m) * a.NEV + i) * a.ld + g];
+      for (int c = w; c < a.n_chunks; c += 8) s += src[(((int64_t)c * a.M + m) * n) * a.ld + g];
       s_part[w][i][lane] = s;
     }
   }
   __syncthreads();
-  if (w != 0 || !ok) return;
+  if (w != 0 || g >= a.Ng) return;
+  float* const wc = a.Wc + (int64_t)m * a.KC * a.ld + g;   // row k at wc[k * ld]
+  float* const bp = a.b + (int64_t)m * a.ld + g;
+  float* const tp = a.tau + (int64_t)m * a.ld + g;
+  auto save_prev = [&]() {
+    float* p = a.prev + (int64_t)m * (a.KC + 2) * a.ld + g;
+    for (int k = 0; k < a.KC; ++k) p[k * a.ld] = wc[k * a.ld];
+    p[a.KC * a.ld] = *bp;
+    p[(a.KC + 1) * a.ld] = *tp;
+  };
+  // frozen events keep their parameters; the next pass still reads them
+  if (!ok) { if (a.prev) save_prev(); return; }
+  if (a.prev && !a.part_st) save_prev();
+  // look-ahead (part_st set only for KC <= kMaxPairKc, brie_fit_create): the parameters before the update are its
+  // reference point (w', b', tau'); fixed-size, fully unrolled, so they stay in registers
+  const bool look_ahead = a.part_st != nullptr && a.KC <= kMaxPairKc;
+  float w0[kMaxPairKc] = {};
+  float b0 = 0.f, t0 = 0.f;
+  if (look_ahead) {
+#pragma unroll
+    for (int k = 0; k < kMaxPairKc; ++k)
+      if (k < a.KC) w0[k] = wc[k * a.ld];
+    b0 = *bp; t0 = *tp;
+  }
   auto red = [&](int i) {
     double s = 0.0;
 #pragma unroll
@@ -933,20 +1073,158 @@ __global__ void __launch_bounds__(256) event_update_kernel(const EventArgs a) {
     return s;
   };
   const int64_t mstride = (int64_t)a.M * (a.KC + 2) * a.ld;
-  auto adam_slot = [&](float* x, int slot, float grad, bool clip) {
+  auto adam_slot = [&](float* x, int slot, float grad, bool clip, float alpha) {
     const int64_t qi = ((int64_t)m * (a.KC + 2) + slot) * a.ld + g;
-    adam_at(x, a.mom + qi, a.mom + mstride + qi, grad, a.alpha, clip);
+    adam_at(x, a.mom + qi, a.mom + mstride + qi, grad, alpha, clip);
   };
+  auto trained = [&](int k) { return a.wc_grad ? k < a.xc_width[m] : ((a.xc_mask[m] >> k) & 1u) != 0; };
   for (int k = 0; k < a.KC; ++k) {
-    if (a.wc_grad ? k >= a.xc_width[m] : !((a.xc_mask[m] >> k) & 1u)) continue;
+    if (!trained(k)) continue;
     const float grad = a.wc_grad ? a.wc_grad[((int64_t)m * a.KC + k) * a.ld + g] : (float)red(k);
-    adam_slot(a.Wc + ((int64_t)m * a.KC + k) * a.ld + g, k, grad, false);
+    adam_slot(wc + k * a.ld, k, grad, false, a.alpha);
   }
-  if (a.idx_gb >= 0 && a.train_b) adam_slot(a.b + (int64_t)m * a.ld + g, a.KC, (float)red(a.idx_gb), true);
-  if (a.idx_gt >= 0 && a.train_tau) adam_slot(a.tau + (int64_t)m * a.ld + g, a.KC + 1, (float)red(a.idx_gt), false);
+  if (a.idx_gb >= 0 && a.train_b) adam_slot(bp, a.KC, (float)red(a.idx_gb), true, a.alpha);
+  if (a.idx_gt >= 0 && a.train_tau) adam_slot(tp, a.KC + 1, (float)red(a.idx_gt), false, a.alpha);
   if (a.idx_loss >= 0 && a.trace_slot >= 0)
     a.trace[((int64_t)m * a.trace_cap + a.trace_slot) * a.ld + g] = (float)red(a.idx_loss);
+  if (a.idx_loss2 >= 0 && a.trace_slot >= 0)
+    a.trace[((int64_t)m * a.trace_cap + a.trace_slot + 1) * a.ld + g] = (float)red(a.idx_loss2);
+  if (!look_ahead) return;
+
+  // Look-ahead update.  The statistics R_k = sum_c x_ck d_c, R_0 = sum_c d_c, Q = sum_c d_c^2, E = sum_c exp(2 (lam_c
+  // - tau')) with d_c = mu_c - p'_c were taken around the parameters (w', b', tau') the pass stepped with, which the
+  // updates above moved by (dw, db, dtau).  Around the new ones, p_c = p'_c + x_c . dw + db, so
+  //   sum_c x_ck (mu_c - p_c) = R_k - (G dw)_k - s_k db,   sum_c (mu_c - p_c) = R_0 - s . dw - n db,
+  //   sum_c (mu_c - p_c)^2 = Q - 2 (dw . R + db R_0) + dw^T G dw + 2 db s . dw + n db^2,
+  //   sum_c exp(2 (lam_c - tau)) = E exp(-2 dtau)
+  // (G = sum_c x_c x_c^T, s = sum_c x_c, n cells), and the KL gradients of the next step follow exactly.
+  save_prev();
+  const int K = a.KC, i0 = a.NEV;      // statistic rows follow the a.NEV gradient / loss rows in s_part
+  const double* G = a.gram + (int64_t)m * (K * K + K);
+  const double* sv = G + K * K;
+  const double n = (double)a.Nc;
+  double dw[kMaxPairKc], Gdw[kMaxPairKc];
+#pragma unroll
+  for (int k = 0; k < kMaxPairKc; ++k) dw[k] = k < K ? (double)wc[k * a.ld] - (double)w0[k] : 0.0;   // 0 untrained
+  const double db = (double)*bp - (double)b0, dt = (double)*tp - (double)t0;
+  const double R0 = red(i0 + K), Q = red(i0 + K + 1), E = red(i0 + K + 2);
+  double sdw = 0.0, wR = 0.0, wGw = 0.0;
+#pragma unroll
+  for (int k = 0; k < kMaxPairKc; ++k) {
+    Gdw[k] = 0.0;
+    if (k >= K) continue;
+#pragma unroll
+    for (int l = 0; l < kMaxPairKc; ++l)
+      if (l < K) Gdw[k] += G[k * K + l] * dw[l];
+    sdw += sv[k] * dw[k];
+    wR += dw[k] * red(i0 + k);
+    wGw += dw[k] * Gdw[k];
+  }
+  const double kappa = exp(-2.0 * (double)*tp);
+#pragma unroll
+  for (int k = 0; k < kMaxPairKc; ++k) {
+    if (k >= K || !trained(k)) continue;
+    adam_slot(wc + k * a.ld, k, (float)(-kappa * (red(i0 + k) - Gdw[k] - sv[k] * db)), false, a.alpha2);
+  }
+  const double S0 = R0 - sdw - n * db;
+  const double S2 = Q - 2.0 * (wR + db * R0) + wGw + 2.0 * db * sdw + n * db * db;
+  if (a.train_b) adam_slot(bp, K, (float)(-kappa * S0), true, a.alpha2);
+  if (a.train_tau) adam_slot(tp, K + 1, (float)(n - kappa * S2 - E * exp(-2.0 * dt)), false, a.alpha2);
 }
+
+// Sums-only pre-pass of a run of two-step passes: the per-event gradient sums of one step (the KL terms, the only
+// source of the per-event parameters' gradients in gene mode with Kg = 0) from Z_loc and Z_std_log, in
+// elbo_step_kernel's row-chunk partial layout (KC + 2 rows), for event_update_kernel.  Lanes whose events are all
+// frozen read nothing.
+template <int KC>
+__global__ void __launch_bounds__(kThreads) kl_sums_kernel(const StepArgs a) {
+  constexpr int EPL = step_epl(KC), TC = 32 * EPL, NEV = KC + 2;
+  using Vec = typename LaneVec<EPL>::type;
+  const int m = blockIdx.x, tile = blockIdx.y, chunk = blockIdx.z;
+  if (!((a.model_mask >> m) & 1u)) return;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t g0 = (int64_t)tile * TC + lane * EPL;
+  bool act = false;
+  if (g0 < a.ld) {
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) act |= a.active[(int64_t)m * a.ld + g0 + j] != 0;
+  }
+  if (!__syncthreads_or(act)) return;
+  float wc[KC > 0 ? KC : 1][EPL], bb[EPL], tau[EPL], is2[EPL], acc[NEV][EPL];
+#pragma unroll
+  for (int j = 0; j < EPL; ++j) {
+    bb[j] = 0.f; tau[j] = 0.f;
+#pragma unroll
+    for (int k = 0; k < (KC > 0 ? KC : 1); ++k) wc[k][j] = 0.f;
+#pragma unroll
+    for (int i = 0; i < NEV; ++i) acc[i][j] = 0.f;
+  }
+  if (act) {
+#pragma unroll
+    for (int k = 0; k < KC; ++k) vec_get<EPL>(*reinterpret_cast<const Vec*>(a.Wc + ((int64_t)m * KC + k) * a.ld + g0), wc[k]);
+    vec_get<EPL>(*reinterpret_cast<const Vec*>(a.b + (int64_t)m * a.ld + g0), bb);
+    vec_get<EPL>(*reinterpret_cast<const Vec*>(a.tau + (int64_t)m * a.ld + g0), tau);
+  }
+#pragma unroll
+  for (int j = 0; j < EPL; ++j) is2[j] = fast_exp(-2.0f * tau[j]);
+  const int64_t row_begin = (int64_t)chunk * a.rows_per_cta;
+  const int64_t row_end = min(row_begin + (int64_t)a.rows_per_cta, a.Nc);
+  const int64_t plane = a.Nc * a.ld;
+  for (int64_t row = row_begin + warp; act && row < row_end; row += kWarps) {
+    float mu[EPL], lam[EPL], xc[KC > 0 ? KC : 1];
+    const int64_t off = (int64_t)m * plane + row * a.ld + g0;
+    vec_get<EPL>(__ldcs(reinterpret_cast<const Vec*>(a.Zl + off)), mu);
+    vec_get<EPL>(__ldcs(reinterpret_cast<const Vec*>(a.Zs + off)), lam);
+#pragma unroll
+    for (int k = 0; k < KC; ++k) xc[k] = a.Xc[((int64_t)m * a.Nc + row) * KC + k];
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) {
+      float pm = bb[j];
+#pragma unroll
+      for (int k = 0; k < KC; ++k) pm = fmaf(xc[k], wc[k][j], pm);
+      const float diff = mu[j] - pm, rr = diff * is2[j];
+      const float e2 = ex2_approx((lam[j] - tau[j]) * (2.0f * kLog2e));
+#pragma unroll
+      for (int k = 0; k < KC; ++k) acc[k][j] = fmaf(xc[k], -rr, acc[k][j]);
+      acc[KC][j] -= rr;
+      acc[KC + 1][j] += (1.0f - diff * rr) - e2;
+    }
+  }
+  __shared__ float red[kWarps][TC];
+#pragma unroll
+  for (int i = 0; i < NEV; ++i) {
+    *reinterpret_cast<Vec*>(&red[warp][lane * EPL]) = vec_make<EPL>(acc[i]);
+    __syncthreads();
+    const int64_t g = (int64_t)tile * TC + threadIdx.x;
+    if (threadIdx.x < TC && g < a.ld) {
+      float s = 0.f;
+#pragma unroll
+      for (int w = 0; w < kWarps; ++w) s += red[w][threadIdx.x];
+      a.part_ev[(((int64_t)chunk * a.M + m) * NEV + i) * a.ld + g] = s;
+    }
+    __syncthreads();
+  }
+}
+
+// gram[m] = (sum_c x_c x_c^T (K x K), sum_c x_c (K)) of model m's design rows, in float64 and a fixed order: one block
+// per entry and model.
+__global__ void __launch_bounds__(256) gram_kernel(const float* Xc, int64_t Nc, int K, double* gram) {
+  const int e = blockIdx.x, m = blockIdx.y;
+  const int i = e < K * K ? e / K : e - K * K, j = e < K * K ? e % K : -1;
+  const float* X = Xc + (int64_t)m * Nc * K;
+  double s = 0.0;
+  for (int64_t c = threadIdx.x; c < Nc; c += blockDim.x)
+    s += (double)X[c * K + i] * (j >= 0 ? (double)X[c * K + j] : 1.0);
+  __shared__ double red[256];
+  red[threadIdx.x] = s;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) gram[(int64_t)m * (K * K + K) + e] = red[0];
+}
+
 
 // Per-cell gradient reduce over column tiles: G[m, c, i] = sum_tiles part_cell.
 struct CellArgs {

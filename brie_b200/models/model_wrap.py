@@ -824,7 +824,11 @@ def _device_event_budget(Nc, n_models, n_layers, device=None, frac=0.7, reserve=
     besides `reserve` bytes held for the whole fit (the score candidates and one block of the score pass)."""
     import torch
     free, _ = torch.cuda.mem_get_info(device)
-    per_event = Nc * 4 * (n_layers + 1 + 6 * n_models + 3 + 1) * 1.05
+    # + the step kernel's per-event scratch of two-step fits, approximated: statistic partials and a second loss row
+    # (Kc <= 4: at most 8 floats per model and row chunk) at 256 cells per row chunk, the chunk size brie_fit_create
+    # picks for fits large enough to be cut into device chunks; the first-step parameters (Kc + 2 floats per model
+    # and event, not per cell) are left out
+    per_event = Nc * 4 * (n_layers + 1 + 6 * n_models + 3 + 1 + n_models * 8 / 256) * 1.05
     return max(int(max(free - reserve, 0) * frac / per_event), 1)
 
 
